@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (oracle port) on host cores
     python bench.py --config celebahq|div2k                  # BASELINE configs 4 / 5 (one GPU, reported lines)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's loss + parameters (.npy)
 
 Workload (BASELINE.json configs[1]): configs/cifar10/ddm_uncond_const_uncond_unet.yaml UNet (216.1 M parameters),
 batch 128 per GPU, bf16 compute with fp32 master weights, one micro-batch forward + backward + clip + AdamW per step,
@@ -44,6 +45,24 @@ LATENT_CONFIGS = {
 # (profiles/r05_conv_ncu_full.txt, final build: 27.91 MB read + 0.34 MB written): the 25 MB input is read once, weights
 # 2.6 MB, the output is still in L2 when the kernel ends.
 CONV_DRAM_TRAFFIC_BYTES = 28.25e6
+# --dump-outputs: fp32 parameter values written (32 MiB); the CIFAR UNet has 216.1 M, far more than a comparison needs
+DUMP_PARAM_SAMPLE = 1 << 23
+
+
+def dump_outputs(out_dir, loss, net):
+    """What the timed training step hands its caller after the last timed step: the loss (loss.npy) and the parameters
+    it updated (params.npy: all of them in named_parameters order, the reference's state_dict layout, or, for a larger
+    model, DUMP_PARAM_SAMPLE of them at sorted positions drawn with seed 0).  The inputs are seeded, so two builds run
+    with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    flat = torch.cat([p.detach().reshape(-1).float() for p in net.parameters()])
+    if flat.numel() > DUMP_PARAM_SAMPLE:
+        idx = torch.randint(flat.numel(), (DUMP_PARAM_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+        flat = flat[idx.to(flat.device)]
+    np.save(os.path.join(out_dir, "params.npy"), flat.cpu().numpy())
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().reshape(1).cpu().numpy())
 
 
 def peaks():
@@ -389,6 +408,8 @@ def run_latent(args):
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
         ms = float(tms.item())
     launches = (lib.adm_launch_count() - l0) // args.steps + graph_launches
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, ldm.model)
     ldm.eval()
     with torch.no_grad():
         kw = {"cond": batch["cond"]} if "cond" in batch else {"batch_size": B}
@@ -501,6 +522,8 @@ def run_ours(args):
     ms = e0.elapsed_time(e1) / args.steps
     launches = step.launches_per_step if use_graph else (lib.adm_launch_count() - l0) // args.steps
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, dpm.model)
     # ---- end to end through the public API: pinned host batch -> device each step, loss read back each step
     barrier()
     e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -595,7 +618,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--config", default="cifar", choices=["cifar"] + sorted(LATENT_CONFIGS),
                     help="cifar = the headline (BASELINE configs 2 and 3); celebahq / div2k = configs 4 / 5 (celebahq also data parallel under torchrun; div2k one GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss and (a seeded sample of) the updated "
+                         "parameters as DIR/loss.npy and DIR/params.npy (float32, under 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -274,7 +274,8 @@ def relation_layer_golden():
     tail is run on the same inputs for comparison."""
     import torch
     import adm_b200.unet.cond_unet as CU
-    g = torch.load(os.path.join(ROOT, "tests", "golden", "relation_layer.pt"))
+    from tests.golden.make_golden_relation import load
+    g = load(os.path.join(ROOT, "tests", "golden"))
     ok = True
     try:
         for name, rec in g.items():

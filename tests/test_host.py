@@ -9,7 +9,7 @@ import torch
 from oracle import ddm_oracle as O
 from tests.golden.make_golden import CIFAR, TINY
 
-REF = "/root/reference"
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _net(cfg):
@@ -56,12 +56,15 @@ def test_construct_by_reference_class_names():
         construct_class_by_name(model=unet, cfg=model_cfg, **{**model_cfg, "start_dist": "laplace"})
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 def test_reference_yaml_builds_our_classes():
+    """The CIFAR-10 model section (configs/cifar10/... keeps the reference's hyper-parameters) under the reference's own
+    dotted class names builds this package's classes at the reference's size."""
     import yaml
     from adm_b200.ddm.utils import construct_class_by_name
-    cfg = yaml.load(open(os.path.join(REF, "configs/cifar10/ddm_uncond_const_uncond_unet.yaml")), Loader=yaml.FullLoader)
+    cfg = yaml.load(open(os.path.join(ROOT, "configs/cifar10/ddm_uncond_const_uncond_unet.yaml")), Loader=yaml.FullLoader)
     model_cfg = cfg["model"]
+    model_cfg["class_name"] = "ddm.ddm_const.DDPM"
+    model_cfg["unet"]["class_name"] = "unet.uncond_unet.EDMPrecond"
     model_cfg["use_augment"] = False  # AugmentPipe is host-side data glue (SURVEY 8 f-4)
     unet = construct_class_by_name(**model_cfg["unet"])
     dpm = construct_class_by_name(model=unet, cfg=model_cfg, **model_cfg)

@@ -166,7 +166,8 @@ from oracle import relation_oracle as R  # noqa: E402
 
 
 def _relation_golden(golden_dir):
-    return torch.load(os.path.join(golden_dir, "relation_layer.pt"))
+    from tests.golden.make_golden_relation import load
+    return load(golden_dir)
 
 
 @pytest.mark.parametrize("commute", [False, True])
