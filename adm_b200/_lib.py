@@ -49,13 +49,6 @@ SIGNATURES = {
     "adm_unet_output_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
     "adm_conv_fprop": (c_i, [c_p, c_i, c_ll, c_p, c_i, c_ll, c_i, c_i, c_i, c_p, c_i, c_i, c_p, c_i, c_ll, c_p, c_p,
                              c_ll, c_f, c_p]),
-    "adm_conv_fprop_stats": (c_i, [c_p, c_i, c_ll, c_p, c_i, c_ll, c_i, c_i, c_i, c_p, c_i, c_i, c_p, c_i, c_ll, c_p, c_p,
-                                   c_ll, c_f, c_p, c_p]),
-    "adm_conv_stats_slots": (c_i, [c_i, c_i]),
-    "adm_conv_fprop_gn": (c_i, [c_p, c_i, c_ll, c_p, c_i, c_ll, c_i, c_i, c_i, c_p, c_i, c_p, c_ll, c_p, c_p, c_ll, c_p, c_i,
-                                c_f, c_ull, c_p, c_p, c_ll, c_p]),
-    "adm_conv_gn_ok": (c_i, [c_i, c_i]),
-    "adm_gn_finalize": (c_i, [c_p, c_i, c_i, c_p, c_i, c_i, c_i, c_i, c_i, c_f, c_p, c_p, c_p, c_ll, c_p, c_p]),
     "adm_conv_dgrad": (c_i, [c_p, c_i, c_ll, c_i, c_i, c_i, c_p, c_i, c_i, c_p, c_i, c_ll, c_p, c_ll, c_f, c_p]),
     "adm_conv_wgrad": (c_i, [c_p, c_i, c_ll, c_p, c_i, c_ll, c_p, c_i, c_ll, c_i, c_i, c_i, c_i, c_p, c_p]),
     "adm_gemm_batched": (c_i, [C.POINTER(GemmDesc), c_p]),

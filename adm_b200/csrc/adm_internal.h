@@ -9,18 +9,9 @@ void set_error(const char* fmt, ...);
 const char* get_error();
 int num_sms();
 void count_launch();
-bool pdl_enabled();  // ADM_PDL=1: programmatic dependent launch of the hot kernels (off by default, see tc_gemm.cu)
 
 #ifdef __CUDACC__
-// Programmatic dependent launch (sm_90+).  A kernel launched with the attribute may be scheduled while its predecessor in
-// the stream is still draining: it runs its prologue (barrier init, TMEM allocation, index math) on the SMs that are
-// already free and blocks in pdl_wait() until the predecessor grid has completed and its memory is visible.  Every kernel
-// calls pdl_trigger() first thing, which lets ITS successor be scheduled as soon as all of its own CTAs have started.
-// Without the launch attribute both instructions are no-ops.
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-// <<<>>> replacement for the hot kernels: optional thread-block cluster + the PDL attribute.
+// <<<>>> replacement for the hot kernels: optional thread-block cluster.
 template <typename... KArgs, typename... Args>
 static inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s,
                                    int cluster_x, Args... args) {
@@ -29,22 +20,15 @@ static inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = s;
-    cudaLaunchAttribute at[2];
-    int na = 0;
+    cudaLaunchAttribute at[1];
     if (cluster_x > 0) {
-        at[na].id = cudaLaunchAttributeClusterDimension;
-        at[na].val.clusterDim.x = cluster_x;
-        at[na].val.clusterDim.y = 1;
-        at[na].val.clusterDim.z = 1;
-        ++na;
+        at[0].id = cudaLaunchAttributeClusterDimension;
+        at[0].val.clusterDim.x = cluster_x;
+        at[0].val.clusterDim.y = 1;
+        at[0].val.clusterDim.z = 1;
+        cfg.attrs = at;
+        cfg.numAttrs = 1;
     }
-    if (pdl_enabled()) {
-        at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
-    cfg.attrs = at;
-    cfg.numAttrs = na;
     return cudaLaunchKernelEx(&cfg, kern, args...);
 }
 #endif

@@ -94,7 +94,6 @@ __device__ __forceinline__ void attn_unit(const AttnParams& p, int u, int& b0, i
 // ------------------------------------------------------------------------------------------------ forward
 __global__ void __launch_bounds__(AT_THREADS, 1)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ AttnParams p) {
-    pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint64_t* full = reinterpret_cast<uint64_t*>(smem + AT_RING);
@@ -126,7 +125,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
-    pdl_wait();
 
     if (warp == 0) {
         // =========================================================== TMA producer
@@ -303,7 +301,6 @@ constexpr int BW_DK = 256, BW_DV = 320, BW_DQ = 384;
 __global__ void __launch_bounds__(AT_THREADS, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmDO,
                 const __grid_constant__ AttnParams p) {
-    pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint64_t* full = reinterpret_cast<uint64_t*>(smem + AT_RING);
@@ -342,7 +339,6 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
-    pdl_wait();
 
     if (warp == 0) {
         // =========================================================== TMA producer

@@ -124,57 +124,6 @@ __device__ __forceinline__ void gn_finish_coef(const float* __restrict__ sums, c
     }
 }
 
-// Coefficient table from producer-emitted partial statistics (conv epilogue): one CTA per sample.
-__global__ void __launch_bounds__(256) gn_finalize_kernel(const float* __restrict__ st1, int slots1, int c1,
-                                                          const float* __restrict__ st2, int slots2, int c2, int hw,
-                                                          int G, float eps, const float* __restrict__ gamma,
-                                                          const float* __restrict__ beta,
-                                                          const float* __restrict__ params, long long ldp,
-                                                          float4* __restrict__ coef) {
-    extern __shared__ float fsum[];  // [C][2]
-    const int n = blockIdx.x, C = c1 + c2;
-    for (int c = threadIdx.x; c < C; c += blockDim.x) {
-        const bool first = c < c1;
-        const int cc = first ? c : c - c1, cs = first ? c1 : c2, slots = first ? slots1 : slots2;
-        const float2* src = reinterpret_cast<const float2*>(first ? st1 : st2) + (1LL * n * slots) * cs + cc;
-        float s = 0.f, q = 0.f;
-        int k = 0;
-        for (; k + 8 <= slots; k += 8) {  // eight independent loads in flight, summed in a fixed order (deterministic)
-            float2 t[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) t[u] = __ldcg(src + 1LL * (k + u) * cs);
-#pragma unroll
-            for (int u = 0; u < 8; ++u) { s += t[u].x; q += t[u].y; }
-        }
-        for (; k < slots; ++k) {
-            const float2 t = __ldcg(src + 1LL * k * cs);
-            s += t.x;
-            q += t.y;
-        }
-        fsum[2 * c] = s;
-        fsum[2 * c + 1] = q;
-    }
-    __syncthreads();
-    const int cpg = C / G;
-    const float inv_cnt = 1.f / (static_cast<float>(cpg) * static_cast<float>(hw));
-    for (int c = threadIdx.x; c < C; c += blockDim.x) {
-        const int g0 = (c / cpg) * cpg;
-        float s = 0.f, q = 0.f;
-        for (int j = 0; j < cpg; ++j) { s += fsum[2 * (g0 + j)]; q += fsum[2 * (g0 + j) + 1]; }
-        const float mean = s * inv_cnt;
-        const float var = fmaxf(q * inv_cnt - mean * mean, 0.f);
-        const float rstd = rsqrtf(var + eps);
-        const float ga = gamma[c], be = beta[c];
-        float a = rstd * ga, b = be - mean * rstd * ga;
-        if (params != nullptr) {
-            const float sc = 1.f + params[n * ldp + c], sh = params[n * ldp + C + c];
-            a *= sc;
-            b = b * sc + sh;
-        }
-        coef[1LL * n * C + c] = make_float4(a, b, mean, rstd);
-    }
-}
-
 __global__ void __launch_bounds__(256) gn_stats_kernel(const __nv_bfloat16* __restrict__ x1, int c1, long long ld1,
                                                        const __nv_bfloat16* __restrict__ x2, int c2, long long ld2,
                                                        int hw, float* __restrict__ sums, unsigned int* __restrict__ tickets,
@@ -568,8 +517,6 @@ __global__ void __launch_bounds__(256, 3) gn_bwd_apply_kernel(const __nv_bfloat1
 __global__ void __launch_bounds__(256) col_sums_kernel(const __nv_bfloat16* __restrict__ x, long long ld,
                                                        long long rows, int C_total, float* __restrict__ out,
                                                        const int* __restrict__ out_map) {
-    pdl_trigger();
-    pdl_wait();
     extern __shared__ float sm[];  // [blockDim][8]
     const int col0 = blockIdx.y * 2048;
     const int C = min(2048, C_total - col0);
@@ -619,8 +566,6 @@ __global__ void __launch_bounds__(256) add_bf16_kernel(const __nv_bfloat16* __re
                                                        const __nv_bfloat16* __restrict__ c, long long ldc,
                                                        __nv_bfloat16* __restrict__ out, long long ldo, long long rows,
                                                        int C) {
-    pdl_trigger();
-    pdl_wait();
     const int V = C >> 3;
     const unsigned total = static_cast<unsigned>(rows * V);  // < 2^31 vectors (checked by the launcher): 32-bit divisions
     for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
@@ -720,8 +665,6 @@ __global__ void __launch_bounds__(512, 1) gn_fwd_fused_kernel(
     const float* __restrict__ params, long long ldp, float4* __restrict__ coef, int act, float drop_p,
     unsigned long long seed, int resample, __nv_bfloat16* __restrict__ out, long long ldo,
     const unsigned long long* __restrict__ seed_dev) {
-    pdl_trigger();
-    pdl_wait();
     cg::cluster_group cluster = cg::this_cluster();
     const int K = static_cast<int>(cluster.num_blocks()), r = static_cast<int>(cluster.block_rank());
     if (seed_dev != nullptr) seed += *seed_dev * 0x9E3779B97F4A7C15ull;
@@ -835,7 +778,7 @@ __global__ void __launch_bounds__(512, 1) gn_fwd_fused_kernel(
         }
     }
     __syncthreads();
-    if (!active || out == nullptr) return;
+    if (!active) return;
     // ---- pass 2: y = act(x*A + B) (+ dropout) (+ resample on the store); second read of x hits L2
     float a[8], b[8];
 #pragma unroll
@@ -962,8 +905,6 @@ __global__ void __launch_bounds__(512, 1) gn_bwd_fused_kernel(
     const __nv_bfloat16* __restrict__ add, long long ldadd, int add_mode, __nv_bfloat16* __restrict__ dx1,
     long long ldx1, __nv_bfloat16* __restrict__ dx2, long long ldx2, float* __restrict__ dbias1,
     float* __restrict__ dbias1b, const unsigned long long* __restrict__ seed_dev, int dy_scratch) {
-    pdl_trigger();
-    pdl_wait();
     cg::cluster_group cluster = cg::this_cluster();
     const int K = static_cast<int>(cluster.num_blocks()), r = static_cast<int>(cluster.block_rank());
     if (seed_dev != nullptr) seed += *seed_dev * 0x9E3779B97F4A7C15ull;
@@ -1342,19 +1283,13 @@ static cudaError_t launch_cluster(void (*kern)(KArgs...), int grid, int block, s
     cfg.blockDim = dim3(block);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = s;
-    cudaLaunchAttribute at[2];
+    cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = k;
     at[0].val.clusterDim.y = 1;
     at[0].val.clusterDim.z = 1;
-    int na = 1;
-    if (pdl_enabled()) {
-        at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
     cfg.attrs = at;
-    cfg.numAttrs = na;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, args...);
 }
 
@@ -1394,20 +1329,6 @@ int adm_gn_stats(const void* x1, int c1, long long ld1, const void* x2, int c2, 
     return 0;
 }
 
-int adm_gn_finalize(const float* st1, int slots1, int c1, const float* st2, int slots2, int c2, int n, int hw,
-                    int groups, float eps, const float* gamma, const float* beta, const float* params,
-                    long long ld_params, float* coef, void* stream) {
-    const int C = c1 + c2;
-    ADM_REQUIRE(st1 != nullptr && c1 > 0 && (st2 != nullptr || c2 == 0) && C % groups == 0 && slots1 > 0,
-                "gn_finalize: bad arguments");
-    ADM_REQUIRE(C <= 4096, "gn_finalize: C too large");
-    gn_finalize_kernel<<<n, 256, 2 * C * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
-        st1, slots1, c1, st2, slots2, c2, hw, groups, eps, gamma, beta, params, ld_params,
-        reinterpret_cast<float4*>(coef));
-    ADM_CHECK_LAUNCH("gn_finalize");
-    return 0;
-}
-
 int adm_gn_apply(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h, int w,
                  const float* coef, int act, float drop_p, unsigned long long seed,
                  const unsigned long long* seed_counter, int resample, void* out, long long ldo, void* stream) {
@@ -1442,11 +1363,12 @@ int adm_gn_forward(const void* x1, int c1, long long ld1, const void* x2, int c2
                 "gn_forward: channels must be multiples of 8 and divisible by groups");
     ADM_REQUIRE(C <= 2048, "gn_forward: C too large");
     ADM_REQUIRE(resample == 0 || (resample == 1 && h % 2 == 0 && w % 2 == 0) || resample == 2, "gn_forward: bad resample");
+    ADM_REQUIRE(out != nullptr, "gn_forward: out is required");
     const int k = gn_cluster_size(n);
     if (k == 0) {
         int rc = adm_gn_stats(x1, c1, ld1, x2, c2, ld2, n, h * w, groups, eps, gamma, beta, params, ld_params, work, coef,
                               stream);
-        if (rc != 0 || out == nullptr) return rc;
+        if (rc != 0) return rc;
         return adm_gn_apply(x1, c1, ld1, x2, c2, ld2, n, h, w, coef, act, drop_p, seed, seed_counter, resample, out, ldo,
                             stream);
     }

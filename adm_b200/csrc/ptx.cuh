@@ -170,13 +170,7 @@ __device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, u
         : "memory");
 }
 
-// ---------------------------------------------------------------- CTA pairs (cta_group::2)
-// Two CTAs of a cluster on the same TPC execute ONE 256-row MMA: each holds its 128 rows of A and half the rows of B in
-// its own shared memory, the leader (cluster rank 0) issues the instruction, and both get 128 accumulator rows in
-// their own TMEM.  In the shared::cluster window bit 24 of an address selects the CTA inside the pair; clearing it
-// redirects an mbarrier operand to the leader's copy.
-constexpr uint32_t PAIR_LEADER_MASK = 0xFEFFFFFFu;
-
+// ---------------------------------------------------------------- thread-block clusters
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -185,53 +179,6 @@ __device__ __forceinline__ uint32_t cluster_ctarank() {
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
     asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// TMA loads into this CTA's shared memory whose completion bytes are credited to the LEADER's mbarrier.
-__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], "
-        "[%2];" ::"r"(smem_u32(dst)),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & PAIR_LEADER_MASK), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_pair(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2,
-                                                 int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, "
-        "%5, %6}], [%2];" ::"r"(smem_u32(dst)),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & PAIR_LEADER_MASK), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t* dst_smem, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)),
-                 "r"(ncols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                               uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// Arrive (once all previously issued MMAs completed) on the barrier at this offset in BOTH CTAs of the pair.
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
-    asm volatile(
-        "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-            smem_u32(bar)),
-        "h"(static_cast<uint16_t>(3))
-        : "memory");
-}
-// Arrive on the LEADER's copy of a barrier (from either CTA of the pair).
-__device__ __forceinline__ void mbar_arrive_leader(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & PAIR_LEADER_MASK)
-                 : "memory");
 }
 
 // Shared-memory matrix descriptor (sm_100 "version 1"), SWIZZLE_128B.

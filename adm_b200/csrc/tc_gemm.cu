@@ -22,17 +22,6 @@ void set_error(const char* fmt, ...) {
 }
 const char* get_error() { return g_err; }
 
-bool pdl_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        // off by default: measured on B200 inside the captured step it changes nothing (46.2 ms without, 47.0 ms with;
-        // sampler identical) — the step's kernels are long enough that launch latency is already hidden by the graph
-        const char* e = getenv("ADM_PDL");
-        v = (e != nullptr && e[0] == '1') ? 1 : 0;
-    }
-    return v == 1;
-}
-
 int num_sms() {
     if (g_num_sms == 0) {
         int dev = 0;
@@ -125,50 +114,12 @@ static int launch(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap
     return 0;
 }
 
-// CTA-pair conv launch: cluster (2,1,1), an even grid of at most num_sms CTAs.
-static int launch_pair(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const GemmParams& p,
+// Halo conv launch (tc_conv_halo_kernel): plain persistent grid.
+static int launch_halo(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const GemmParams& p,
                        cudaStream_t stream) {
     static bool attr_set = false;
     if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(tc_conv_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             GEMM_SMEM_TOTAL);
-        if (e != cudaSuccess) {
-            set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            return ADM_ERR_CUDA;
-        }
-        attr_set = true;
-    }
-    const long long pair_tiles = 1LL * ((p.m_tiles + 1) / 2) * p.n_tiles;
-    const int max_pairs = num_sms() / 2;
-    const int pairs = static_cast<int>(pair_tiles < max_pairs ? pair_tiles : max_pairs);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * pairs);
-    cfg.blockDim = dim3(PAIR_THREADS);
-    cfg.dynamicSmemBytes = GEMM_SMEM_TOTAL;
-    cfg.stream = stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, tc_conv_pair_kernel, a, a2, b, p);
-    if (e != cudaSuccess) {
-        set_error("tc_conv_pair launch: %s", cudaGetErrorString(e));
-        return ADM_ERR_CUDA;
-    }
-    count_launch();
-    return 0;
-}
-
-// Halo conv launch (tc_conv_halo_kernel): plain persistent grid.  PRO = with the GroupNorm + SiLU prologue warps.
-template <bool PRO>
-static int launch_halo_t(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const GemmParams& p,
-                         cudaStream_t stream) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(tc_conv_halo_kernel<PRO>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        cudaError_t e = cudaFuncSetAttribute(tc_conv_halo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              GEMM_SMEM_TOTAL);
         if (e != cudaSuccess) {
             set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e));
@@ -186,8 +137,7 @@ static int launch_halo_t(const CUtensorMap& a, const CUtensorMap& a2, const CUte
     if (dbg < 0) { const char* e = getenv("ADM_GEMM_DEBUG"); dbg = e ? atoi(e) : 0; }
     GemmParams pd = p;
     pd.debug = dbg;
-    cudaError_t e = launch_k(tc_conv_halo_kernel<PRO>, dim3(grid), dim3(PRO ? GEMM_PRO_THREADS : GEMM_THREADS),
-                             GEMM_SMEM_TOTAL, stream, 0, a, a2, b, pd);
+    cudaError_t e = launch_k(tc_conv_halo_kernel, dim3(grid), dim3(GEMM_THREADS), GEMM_SMEM_TOTAL, stream, 0, a, a2, b, pd);
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess) {
         set_error("tc_conv_halo launch: %s", cudaGetErrorString(e));
@@ -195,11 +145,6 @@ static int launch_halo_t(const CUtensorMap& a, const CUtensorMap& a2, const CUte
     }
     count_launch();
     return 0;
-}
-
-static int launch_halo(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const GemmParams& p,
-                       cudaStream_t stream) {
-    return p.pro_coef != nullptr ? launch_halo_t<true>(a, a2, b, p, stream) : launch_halo_t<false>(a, a2, b, p, stream);
 }
 
 // Cluster split-K conv launch (tc_conv_splitk_kernel): one tile per CTA, clusters of p.ksplit CTAs along K.
@@ -330,18 +275,6 @@ static bool halo_ok(int ntaps, int h, int w) {
     return v == 1 && ntaps == 9 && w % 8 == 0 && h % 16 == 0;
 }
 
-// ADM_GEMM_PAIR=1 enables the cta_group::2 conv path.  It is OFF by default: measured on B200 it is ~6 % slower than the
-// single-CTA kernel on the CIFAR shapes (tools/bench_gemm_variants.py: 960 vs 1022 TF/s at 384->384 @16x16) although it
-// moves 30 % fewer bytes — these convs are not bound by L2 / shared-memory operand traffic (DESIGN.md section 4).
-static bool pair_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("ADM_GEMM_PAIR");
-        v = (e != nullptr && e[0] == '1') ? 1 : 0;
-    }
-    return v == 1;
-}
-
 // Largest multiple of 16 that is <= cap and divides ceil16(n); falls back to the smallest cover.
 static int pick_bn(int n, int cap, int multiple) {
     const int n16 = (n + multiple - 1) / multiple * multiple;
@@ -419,67 +352,11 @@ static int nhwc_map(CUtensorMap* m, const void* ptr, int c, long long ld, int n,
 
 using namespace adm;
 
-struct ProArgs {  // GroupNorm prologue of adm_conv_fprop_gn
-    const float* coef;
-    int act;
-    float drop_p;
-    unsigned long long seed;
-    const unsigned long long* seed_dev;
-    void* a_out;
-    long long ld_a;
-};
-static int conv_fprop_impl(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h,
-                           int w, const void* wpk, int nout, int ntaps, void* out, int out_mode, long long ldc,
-                           const float* bias, const void* residual, long long ldr, float alpha, float* stats,
-                           const ProArgs* pro, void* stream);
-
 extern "C" {
-
-int adm_conv_stats_slots(int h, int w) {
-    const int s = (h * w) / 32;
-    return s < 1 ? 1 : s;
-}
 
 int adm_conv_fprop(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h, int w,
                    const void* wpk, int nout, int ntaps, void* out, int out_mode, long long ldc, const float* bias,
                    const void* residual, long long ldr, float alpha, void* stream) {
-    return adm_conv_fprop_stats(x1, c1, ld1, x2, c2, ld2, n, h, w, wpk, nout, ntaps, out, out_mode, ldc, bias, residual,
-                                ldr, alpha, nullptr, stream);
-}
-
-int adm_conv_fprop_stats(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h,
-                         int w, const void* wpk, int nout, int ntaps, void* out, int out_mode, long long ldc,
-                         const float* bias, const void* residual, long long ldr, float alpha, float* stats,
-                         void* stream) {
-    return conv_fprop_impl(x1, c1, ld1, x2, c2, ld2, n, h, w, wpk, nout, ntaps, out, out_mode, ldc, bias, residual, ldr,
-                           alpha, stats, nullptr, stream);
-}
-
-int adm_conv_gn_ok(int h, int w) { return halo_ok(9, h, w) ? 1 : 0; }
-
-int adm_conv_fprop_gn(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h, int w,
-                      const void* wpk, int nout, void* out, long long ldc, const float* bias, const void* residual,
-                      long long ldr, const float* coef, int act, float drop_p, unsigned long long seed,
-                      const unsigned long long* seed_counter, void* a_out, long long ld_a, void* stream) {
-    if (coef == nullptr || !halo_ok(9, h, w)) {
-        set_error("conv_fprop_gn: needs a coefficient table and an image that tiles into 8 x 16 pixel boxes (got %d x %d)", h, w);
-        return ADM_ERR_SHAPE;
-    }
-    if (c1 + c2 > 1024) { set_error("conv_fprop_gn: more than 1024 input channels"); return ADM_ERR_SHAPE; }
-    ProArgs pro;
-    pro.coef = coef; pro.act = act; pro.drop_p = drop_p; pro.seed = seed;
-    pro.seed_dev = drop_p > 0.f ? seed_counter : nullptr;
-    pro.a_out = a_out; pro.ld_a = ld_a;
-    return conv_fprop_impl(x1, c1, ld1, x2, c2, ld2, n, h, w, wpk, nout, 9, out, OUT_BF16, ldc, bias, residual, ldr, 1.f,
-                           nullptr, &pro, stream);
-}
-
-}  // extern "C"
-
-static int conv_fprop_impl(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h,
-                           int w, const void* wpk, int nout, int ntaps, void* out, int out_mode, long long ldc,
-                           const float* bias, const void* residual, long long ldr, float alpha, float* stats,
-                           const ProArgs* pro, void* stream) {
     if (int e = init_driver()) return e;
     if (taps_per_row(ntaps) == 0) { set_error("conv_fprop: ntaps must be 1, 9, 25 or 49"); return ADM_ERR_SHAPE; }
     if (c1 <= 0 || c1 % 8 || (x2 && (c2 <= 0 || c2 % 8))) { set_error("conv_fprop: channels must be multiples of 8"); return ADM_ERR_SHAPE; }
@@ -497,7 +374,7 @@ static int conv_fprop_impl(const void* x1, int c1, long long ld1, const void* x2
     p.k_total = p.k_iters = ntaps * p.cchunks;
     p.bn = pick_bn_cost(nout, 16, p.m_tiles, p.k_total);
     p.ksplit = 1;
-    if (!halo && stats == nullptr && pro == nullptr && out_mode != OUT_F32_ATOMIC) {
+    if (!halo && out_mode != OUT_F32_ATOMIC) {
         int bn_s = p.bn;
         const int ks = pick_splitk(nout, 16, p.m_tiles, p.k_total, &bn_s);
         if (ks > 1) { p.ksplit = ks; p.bn = bn_s; p.k_iters = (p.k_total + ks - 1) / ks; }
@@ -506,25 +383,6 @@ static int conv_fprop_impl(const void* x1, int c1, long long ld1, const void* x2
     p.M = n * h * w; p.N = nout;
     p.C = out; p.ldc = ldc; p.bias = bias; p.residual = static_cast<const __nv_bfloat16*>(residual); p.ldr = ldr;
     p.alpha = alpha; p.out_mode = out_mode;
-    if (stats != nullptr) {
-        // the epilogue's per-warp column sums assume 32 consecutive tile rows stay inside one image (or split it in two
-        // 16-pixel halves): images of 16, 64 or a multiple of 128 pixels
-        const int hw = h * w;
-        if (!(hw == 16 || hw == 64 || hw % 128 == 0) || out_mode != OUT_BF16) {
-            set_error("conv_fprop: GroupNorm statistics need H*W in {16, 64, k*128} and a bf16 output (got %d x %d)", h, w);
-            return ADM_ERR_SHAPE;
-        }
-        p.stats = stats;
-        p.stats_slots = adm_conv_stats_slots(h, w);
-    }
-    if (pro != nullptr) {
-        p.pro_coef = reinterpret_cast<const float4*>(pro->coef);
-        p.pro_act = pro->act; p.pro_c1 = c1; p.pro_c2 = x2 ? c2 : 0;
-        p.pro_drop_p = pro->drop_p; p.pro_seed = pro->seed; p.pro_seed_dev = pro->seed_dev;
-        p.pro_out = static_cast<__nv_bfloat16*>(pro->a_out); p.pro_ldo = pro->ld_a;
-        p.pro_x1 = static_cast<const __nv_bfloat16*>(x1); p.pro_ld1 = ld1;
-        p.pro_x2 = static_cast<const __nv_bfloat16*>(x2); p.pro_ld2 = ld2;
-    }
     CUtensorMap ma, ma2, mb;
     const int abw = halo ? HALO_W : p.bw, abh = halo ? HALO_H : p.bh;  // A box: the tile, or the tile + its 3x3 halo
     if (int e = nhwc_map(&ma, x1, c1, ld1, n, h, w, abw, abh, p.bni)) return e;
@@ -532,19 +390,12 @@ static int conv_fprop_impl(const void* x1, int c1, long long ld1, const void* x2
     const long long kpad = 1LL * ntaps * p.cchunks * 64;
     const long long bd[2] = {kpad, nout};
     const long long bs[1] = {kpad};
-    // CTA pairs: 256-pixel tiles, each CTA loading half of the weight rows (box BN/2) — when there are at least two
-    // pixel tiles and the output mode is a plain store.
-    const bool pair = !halo && p.ksplit == 1 && pair_enabled() && p.m_tiles >= 2 && p.bn % 16 == 0 && out_mode != OUT_F32_ATOMIC &&
-                      stats == nullptr && pro == nullptr;
-    const int bb[2] = {64, pair ? p.bn / 2 : p.bn};
+    const int bb[2] = {64, p.bn};
     if (int e = encode_map(&mb, wpk, 2, bd, bs, bb)) return e;
-    if (pair) return launch_pair(ma, ma2, mb, p, static_cast<cudaStream_t>(stream));
     if (halo) return launch_halo(ma, ma2, mb, p, static_cast<cudaStream_t>(stream));
     if (p.ksplit > 1) return launch_splitk(ma, ma2, mb, p, static_cast<cudaStream_t>(stream));
     return launch<GEMM_CONV>(ma, ma2, mb, p, static_cast<cudaStream_t>(stream));
 }
-
-extern "C" {
 
 int adm_conv_dgrad(const void* dy, int cout, long long ld_dy, int n, int h, int w, const void* wpk, int kpad,
                    int ntaps, void* dx, int n_valid, long long ldc, const void* residual, long long ldr, float alpha,

@@ -1,7 +1,7 @@
 // tcgen05 / TMEM / TMA GEMM engine shared by conv3x3 (implicit GEMM fprop + dgrad), conv1x1, wgrad, Linear and the
 // batched attention products.  Persistent warp-specialised kernels — tc_gemm_kernel<PLAIN|CONV|WGRAD> (general),
 // tc_conv_halo_kernel (3x3 fprop/dgrad with halo re-use of the pixel operand), tc_wgrad_rows_kernel (3x3 wgrad, three
-// taps per MMA), tc_conv_pair_kernel (cta_group::2 experiment) — with the same roles:
+// taps per MMA), tc_conv_splitk_kernel (cluster split-K conv) — with the same roles:
 //   warp 0      : TMA producer (one lane)        global -> 128B-swizzled smem ring
 //   warp 1      : TMEM allocator + UMMA issuer   tcgen05.mma, fp32 accumulators in TMEM (2 x 256 columns)
 //   warps 2..   : epilogue                       tcgen05.ld -> +bias, +residual, *alpha -> bf16 / fp32 / fp32 atomics
@@ -11,7 +11,6 @@
 #pragma once
 #include "ptx.cuh"
 #include "adm_internal.h"
-#include "vecmath.cuh"
 #ifdef ADM_GEMM_TIMING
 #include <stdio.h>
 #endif
@@ -26,16 +25,10 @@ constexpr int GEMM_BLOCK_K = 64;
 constexpr int GEMM_EPI_WARPS = 4;
 constexpr int EPI_HALVES = GEMM_EPI_WARPS / 4;
 constexpr int GEMM_THREADS = 64 + 32 * GEMM_EPI_WARPS;   // TMA warp + MMA warp + epilogue warps
-constexpr int PAIR_THREADS = 192;                        // the (experimental) CTA-pair kernel keeps 4 epilogue warps
 constexpr int GEMM_A_STAGE = GEMM_BLOCK_M * 128;  // 16 KB
 constexpr int GEMM_SMEM_RING = 200 * 1024;        // operand ring budget
-constexpr int GEMM_SMEM_AUX = 4096 + 8192;        // barriers + tmem ptr (first 1 KB) + per-tile bias slices (2 x 1 KB) +
-                                                  // 1 KB spare + the prologue's per-tile (A, B) table (1024 channels x 8 B)
-// halo conv with the GroupNorm prologue: + 4 transform warps.  (8 warps halve the transform time but cap the kernel at 128
-// registers per thread, which spills in the epilogue; measured in the step they are equal within noise — see
-// profiles/r03_conv_gn_prologue.txt for all the variants that were timed.)
-constexpr int GEMM_PRO_WARPS = 4;
-constexpr int GEMM_PRO_THREADS = GEMM_THREADS + 32 * GEMM_PRO_WARPS;
+constexpr int GEMM_SMEM_AUX = 4096;               // barriers + tmem ptr (first 1 KB) + per-tile bias slices (2 x 1 KB) +
+                                                  // 1 KB spare
 constexpr int GEMM_SMEM_TOTAL = GEMM_SMEM_RING + GEMM_SMEM_AUX + 1024;  // + alignment slack
 constexpr int GEMM_MAX_STAGES = 8;
 
@@ -74,36 +67,7 @@ struct GemmParams {
     int out_mode;
     const int* row_map;  // plain / wgrad tiles: GEMM row r is stored at output row row_map[r] (nullptr = identity)
     int debug;  // experiments only (ADM_GEMM_DEBUG): bit 0 = skip the MMAs, bit 1 = skip the TMA loads
-    // ---- GroupNorm statistics of the OUTPUT, emitted by the conv epilogue (SURVEY 7-6 / 8 a-8): per (sample, slot, channel)
-    // partial {sum, sum of squares} over the pixels one epilogue warp (or half-warp, 4x4 images) holds, plain stores into
-    // stats[n][slot][N][2] — no atomics, no zeroing, deterministic.  The next norm derives its group statistics from these
-    // instead of re-reading the activation (adm_gn_finalize).  nullptr = off.
-    float* stats;
-    int stats_slots;  // slots per sample: (H*W) / 32, at least 1
-    // ---- GroupNorm(+ adaptive scale/shift) + SiLU (+ dropout) PROLOGUE of the halo conv kernel (north_star: "implicit-GEMM
-    // conv3x3 ... with a GroupNorm+SiLU prologue"): the conv reads the RAW tensor; four transform warps apply
-    // y = dropout(silu(x * A[n,c] + B[n,c])) to each halo tile in shared memory, once per 64-channel chunk (not once per
-    // tap), between the TMA load and the MMAs.  pro_coef = the norm's coefficient table [n][C]{A, B, mean, rstd}.
-    const float4* pro_coef;
-    int pro_act, pro_c1, pro_c2;          // SiLU on/off; valid channels of A source 1 / 2 (C = c1 + c2)
-    float pro_drop_p;
-    unsigned long long pro_seed;
-    const unsigned long long* pro_seed_dev;
-    __nv_bfloat16* pro_out;               // optional: the activated tensor [N,H,W,C] (the wgrad operand), written once
-    long long pro_ldo;
-    const __nv_bfloat16* pro_x1;          // the raw A sources (the prologue warps read them with plain vector loads)
-    const __nv_bfloat16* pro_x2;
-    long long pro_ld1, pro_ld2;
 };
-
-// sm_100a SFU tanh; silu(v) = h * tanh(h) + h with h = v / 2
-__device__ __forceinline__ float gemm_tanh_fast(float h) {
-    float t;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(h));
-    return t;
-}
-// The dropout keep-scales are those of csrc/norm.cu (vecmath.cuh: same hash, same indexing — backward regenerates the
-// masks there).
 
 __device__ __forceinline__ void decode_pix(const GemmParams& p, int idx, int& n0, int& h0, int& w0) {
     const int per = p.tiles_w * p.tiles_h;
@@ -137,46 +101,15 @@ __device__ __forceinline__ void stage_bias(const GemmParams& p, float* sbias, in
         sbias[c] = (col_base + c < p.N) ? __ldg(p.bias + col_base + c) : 0.f;
     asm volatile("bar.sync 1, %0;" ::"n"(32 * GEMM_EPI_WARPS) : "memory");
 }
-// pair kernel: 128 epilogue threads, two columns each
-__device__ __forceinline__ void stage_bias_128(const GemmParams& p, float* sbias, int col_base, int m) {
-    if (p.bias == nullptr) return;
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        const int c = m + 128 * i;
-        if (c < p.bn) sbias[c] = (col_base + c < p.N) ? __ldg(p.bias + col_base + c) : 0.f;
-    }
-    asm volatile("bar.sync 1, 128;" ::: "memory");
-}
-
-// Column sums of 16 values per lane over the lanes of a warp in 15 (+1) shuffles: at each halving step a lane keeps the
-// half of its values selected by one lane bit and receives the partner's copy of that half.  Afterwards lane l holds in
-// v[0] the total of column (l & 15) over the 16 lanes sharing its bit 4 — or, with whole_warp, over all 32 lanes.
-__device__ __forceinline__ void warp_colsum16(float (&v)[16], int lane, bool whole_warp) {
-#pragma unroll
-    for (int step = 0; step < 4; ++step) {
-        const int off = 8 >> step;
-        const bool hi = (lane & off) != 0;
-#pragma unroll
-        for (int i = 0; i < (8 >> step); ++i) {
-            const float send = hi ? v[i] : v[i + off];
-            const float keep = hi ? v[i + off] : v[i];
-            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-        }
-    }
-    if (whole_warp) v[0] += __shfl_xor_sync(0xffffffffu, v[0], 16);
-}
 
 // Epilogue of one accumulator tile for one thread (= one output row): TMEM -> registers in groups of up to 64 columns
 // (four 32x32b.x16 loads in flight behind ONE wait, with the residual row segment prefetched behind the same wait),
 // then alpha * acc + bias + residual -> bf16 / fp32 / fp32 atomics.  c_off / r_off: element offsets of this row in the
 // output and the residual (before the column); col_shift: extra output column offset (batched GEMMs); the tile columns
 // drained are [c_begin, ncols) (multiples of 16).
-// stat_row: this lane's base into the statistics table (sample and slot resolved, column 0), or nullptr; the column sums
-// are taken over the bf16-ROUNDED outputs (what the next norm will read); rows that do not exist contribute zeros.
 __device__ __forceinline__ void epilogue_row(const GemmParams& p, uint32_t taddr, int col_base, int col_shift,
                                              long long c_off, long long r_off, bool row_ok, const float* sbias,
-                                             int c_begin, int ncols, float* stat_row = nullptr, bool stat_whole = true,
-                                             int lane = 0) {
+                                             int c_begin, int ncols) {
     for (int c0 = c_begin; c0 < ncols; c0 += 64) {
         if (col_base + c0 >= p.N) break;  // warp-uniform
         uint32_t v[4][16];
@@ -201,7 +134,7 @@ __device__ __forceinline__ void epilogue_row(const GemmParams& p, uint32_t taddr
             }
         }
         tmem_ld_wait();
-        if (!row_ok && stat_row == nullptr) continue;
+        if (!row_ok) continue;
 #pragma unroll
         for (int s = 0; s < 4; ++s) {
             if (s >= nsub) break;
@@ -234,20 +167,6 @@ __device__ __forceinline__ void epilogue_row(const GemmParams& p, uint32_t taddr
                 }
             }
             const long long off = c_off + col_shift + col;
-            if (stat_row != nullptr) {  // every lane of the warp takes part (rows that do not exist contribute zeros)
-                float s1[16], s2[16];
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                    const float r = (row_ok && col + j < p.N) ? __bfloat162float(__float2bfloat16(f[j])) : 0.f;
-                    s1[j] = r;
-                    s2[j] = r * r;
-                }
-                warp_colsum16(s1, lane, stat_whole);
-                warp_colsum16(s2, lane, stat_whole);
-                if ((stat_whole ? lane < 16 : true) && col + (lane & 15) < p.N)
-                    *reinterpret_cast<float2*>(stat_row + 2 * (col + (lane & 15))) = make_float2(s1[0], s2[0]);
-                if (!row_ok) continue;
-            }
             if (p.out_mode == OUT_BF16) {
                 __nv_bfloat16* cp = reinterpret_cast<__nv_bfloat16*>(p.C) + off;
                 if (full && ((reinterpret_cast<uintptr_t>(cp) & 15) == 0)) {
@@ -321,8 +240,6 @@ __device__ __forceinline__ void epilogue_warps(const GemmParams& p, uint8_t* sme
 
         long long row_off;  // element offset of this thread's output row (before column)
         bool row_ok;
-        float* stat_row = nullptr;
-        bool stat_whole = true;
         if (MODE == GEMM_CONV) {
             int n0, h0, w0;
             decode_pix(p, mt, n0, h0, w0);
@@ -330,22 +247,6 @@ __device__ __forceinline__ void epilogue_warps(const GemmParams& p, uint8_t* sme
             const long long pix = (static_cast<long long>(n0 + ni) * p.H + (h0 + hi)) * p.W + (w0 + wi);
             row_ok = pix < p.M;
             row_off = pix;
-            if (p.stats != nullptr) {
-                // slot of this warp's 32 rows inside its sample: tiles of one image are (tile in image) * 4 + quadrant;
-                // images smaller than a tile (8x8: 2 warps each, 4x4: half a warp each) count their own warps
-                const int rows_per_img = p.bw * p.bh;  // rows of one image inside this tile
-                int slot;
-                if (p.bni == 1) {
-                    slot = (mt % (p.tiles_w * p.tiles_h)) * 4 + quad;
-                } else {
-                    slot = (m % rows_per_img) >> 5;
-                    stat_whole = rows_per_img >= 32;
-                }
-                // samples beyond the batch (ragged last tile of packed small images) write into one scratch sample row
-                const long long nsmp = p.M / (p.H * p.W);
-                const long long smp = (n0 + ni) < nsmp ? (n0 + ni) : nsmp;
-                stat_row = p.stats + (smp * p.stats_slots + slot) * 2LL * p.N;
-            }
         } else {
             const int row = mt * 128 + m;
             row_ok = row < p.M;
@@ -360,8 +261,7 @@ __device__ __forceinline__ void epilogue_warps(const GemmParams& p, uint8_t* sme
         mbar_wait(&tfull_bar[acc], acc_phase, 4);
         tc_fence_after();
         const uint32_t taddr = tmem_base + acc * 256 + (static_cast<uint32_t>(quad * 32) << 16);
-        epilogue_row(p, taddr, col_base, col_shift, c_base, row_off * p.ldr, row_ok, sbias, c_begin, c_end, stat_row,
-                     stat_whole, lane);
+        epilogue_row(p, taddr, col_base, col_shift, c_base, row_off * p.ldr, row_ok, sbias, c_begin, c_end);
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&tempty_bar[acc]);
@@ -373,7 +273,6 @@ template <int MODE>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmA2,
                const __grid_constant__ CUtensorMap tmB, const __grid_constant__ GemmParams p) {
-    pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int stage_bytes = GEMM_A_STAGE + p.bn * 128;
@@ -409,7 +308,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
-    pdl_wait();  // everything above touched only this kernel's own state; the predecessor's results are visible from here on
 
     const int num_tiles = p.batches * p.splits * p.m_tiles * p.n_tiles;
 
@@ -613,7 +511,6 @@ __device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 tc_conv_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmA2,
                       const __grid_constant__ CUtensorMap tmB, const __grid_constant__ GemmParams p) {
-    pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int stage_bytes = GEMM_A_STAGE + p.bn * 128;
@@ -653,7 +550,6 @@ tc_conv_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
     cluster_sync_all();  // the leader's peers_bar is initialised before any remote arrive
     tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
-    pdl_wait();
 
     int n0, h0, w0;
     decode_pix(p, mt, n0, h0, w0);
@@ -773,179 +669,6 @@ tc_conv_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
     }
 }
 
-// ------------------------------------------------------------------------------------------------ CTA-pair conv kernel
-// Implicit-GEMM conv (K-major packed weights) with cta_group::2: a cluster of two CTAs computes a 256-pixel x BN tile.
-// Each CTA TMA-loads its own 128-pixel A box and HALF of the weight rows (BN/2 x 64), so per MMA k-step an SM pulls
-// 16 KB + BN*64 B through the L2 fabric instead of 16 KB + BN*128 B — the single-CTA kernel is bound by exactly that
-// traffic (profiles/r01_conv_ncu_full.txt).  Roles per CTA are those of tc_gemm_kernel; differences:
-//   * full barriers live in the leader (rank 0) and collect the TMA bytes of both CTAs;
-//   * the leader's MMA thread issues tcgen05.mma.cta_group::2 (M = 256) and its commits arrive, multicast, on the
-//     empty / tmem-full barriers of both CTAs;
-//   * both epilogues (4 warps each) release the accumulator on the leader's tmem-empty barrier (count 8).
-__global__ void __launch_bounds__(PAIR_THREADS, 1)
-tc_conv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmA2,
-                    const __grid_constant__ CUtensorMap tmB, const __grid_constant__ GemmParams p) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    const int half_bn = p.bn >> 1;
-    const int stage_bytes = GEMM_A_STAGE + half_bn * 128;
-    int num_stages = GEMM_SMEM_RING / stage_bytes;
-    if (num_stages > GEMM_MAX_STAGES) num_stages = GEMM_MAX_STAGES;
-
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + GEMM_SMEM_RING);
-    uint64_t* empty_bar = full_bar + GEMM_MAX_STAGES;
-    uint64_t* tfull_bar = empty_bar + GEMM_MAX_STAGES;
-    uint64_t* tempty_bar = tfull_bar + 2;
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tempty_bar + 2);
-
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-    const int rank = static_cast<int>(cluster_ctarank());
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmA);
-        tma_prefetch_desc(&tmA2);
-        tma_prefetch_desc(&tmB);
-        for (int i = 0; i < num_stages; ++i) {
-            mbar_init(&full_bar[i], 1);
-            mbar_init(&empty_bar[i], 1);
-        }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&tfull_bar[i], 1);
-            mbar_init(&tempty_bar[i], 8);
-        }
-        fence_barrier_init();
-        fence_proxy_async_smem();
-    }
-    if (warp == 1) tmem_alloc_pair(tmem_ptr, 512);
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();  // peer barriers are initialised before any remote arrive / TMA credit
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
-
-    const int m_pairs = (p.m_tiles + 1) >> 1;
-    const int num_tiles = m_pairs * p.n_tiles;
-    const int first = blockIdx.x >> 1, stride = gridDim.x >> 1;
-
-    if (warp == 0) {
-        // =========================================================== TMA producer (both CTAs)
-        if (lane == 0) {
-            int stage = 0;
-            uint32_t phase = 0;
-            for (int tile = first; tile < num_tiles; tile += stride) {
-                const int nt = tile % p.n_tiles;
-                const int mt = 2 * (tile / p.n_tiles) + rank;
-                int n0, h0, w0;
-                decode_pix(p, mt, n0, h0, w0);  // mt == m_tiles (odd tail): n0 is out of range -> zero-filled boxes
-                for (int ki = 0; ki < p.k_total; ++ki) {
-                    mbar_wait(&empty_bar[stage], phase ^ 1, 1);
-                    uint8_t* sa = smem + stage * stage_bytes;
-                    uint8_t* sb = sa + GEMM_A_STAGE;
-                    if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * stage_bytes);
-                    const int tap = ki / p.cchunks, kc = ki % p.cchunks;
-                    int dh = 0, dw = 0;
-                    if (p.kw == 3) { dh = tap / 3 - 1; dw = tap % 3 - 1; }
-                        else if (p.kw > 1) { dh = tap / p.kw - (p.kw >> 1); dw = tap % p.kw - (p.kw >> 1); }
-                    if (kc < p.cchunks1)
-                        tma_load_4d_pair(sa, &tmA, &full_bar[stage], kc * 64, w0 + dw, h0 + dh, n0);
-                    else
-                        tma_load_4d_pair(sa, &tmA2, &full_bar[stage], (kc - p.cchunks1) * 64, w0 + dw, h0 + dh, n0);
-                    tma_load_2d_pair(sb, &tmB, &full_bar[stage], ki * 64, nt * p.bn + rank * half_bn);
-                    if (++stage == num_stages) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // =========================================================== UMMA issuer (leader only)
-        if (lane == 0 && rank == 0) {
-            const uint32_t idesc = make_idesc_bf16(2 * GEMM_BLOCK_M, p.bn, 0, 0);
-            int stage = 0;
-            uint32_t phase = 0;
-            int acc = 0;
-            uint32_t acc_phase = 0;
-            for (int tile = first; tile < num_tiles; tile += stride) {
-                mbar_wait(&tempty_bar[acc], acc_phase ^ 1, 2);
-                tc_fence_after();
-                const uint32_t tmem_d = tmem_base + acc * 256;
-#ifdef ADM_GEMM_TIMING
-                long long t_wait = 0, t_issue = 0, t_commit = 0;
-#endif
-                for (int ki = 0; ki < p.k_total; ++ki) {
-#ifdef ADM_GEMM_TIMING
-                    const long long c0 = clock64();
-#endif
-                    mbar_wait(&full_bar[stage], phase, 3);
-                    tc_fence_after();
-#ifdef ADM_GEMM_TIMING
-                    const long long c1 = clock64();
-#endif
-                    const uint32_t sa = smem_u32(smem + stage * stage_bytes);
-                    const uint32_t sb = sa + GEMM_A_STAGE;
-#pragma unroll
-                    for (int k = 0; k < GEMM_BLOCK_K / 16; ++k) {
-                        const uint64_t da = make_smem_desc(sa + k * 32u, 16u, 1024);
-                        const uint64_t db = make_smem_desc(sb + k * 32u, 16u, 1024);
-                        umma_bf16_pair(tmem_d, da, db, idesc, (ki > 0 || k > 0) ? 1u : 0u);
-                    }
-#ifdef ADM_GEMM_TIMING
-                    const long long c2 = clock64();
-#endif
-                    umma_commit_pair(&empty_bar[stage]);
-#ifdef ADM_GEMM_TIMING
-                    const long long c3 = clock64();
-                    t_wait += c1 - c0; t_issue += c2 - c1; t_commit += c3 - c2;
-#endif
-                    if (++stage == num_stages) { stage = 0; phase ^= 1; }
-                }
-#ifdef ADM_GEMM_TIMING
-                if (blockIdx.x == 0 && tile == first)
-                    printf("[pair mma thread] k-iters %d stages %d: wait %lld issue %lld commit %lld clocks per k-iter\n",
-                           p.k_total, num_stages, t_wait / p.k_total, t_issue / p.k_total, t_commit / p.k_total);
-#endif
-                umma_commit_pair(&tfull_bar[acc]);
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-            }
-        }
-    } else {
-        // =========================================================== epilogue (4 warps per CTA, own 128 rows)
-        const int quad = warp & 3;
-        const int m = quad * 32 + lane;
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        for (int tile = first; tile < num_tiles; tile += stride) {
-            const int nt = tile % p.n_tiles;
-            const int mt = 2 * (tile / p.n_tiles) + rank;
-            int n0, h0, w0;
-            decode_pix(p, mt, n0, h0, w0);
-            const int wi = m % p.bw, hi = (m / p.bw) % p.bh, ni = m / (p.bw * p.bh);
-            const long long pix = (static_cast<long long>(n0 + ni) * p.H + (h0 + hi)) * p.W + (w0 + wi);
-            const bool row_ok = mt < p.m_tiles && pix < p.M;
-            const long long c_base = pix * p.ldc;
-            const int col_base = nt * p.bn;
-
-            float* sbias = reinterpret_cast<float*>(smem + GEMM_SMEM_RING + 1024) + acc * 256;
-            stage_bias_128(p, sbias, col_base, m);
-            mbar_wait(&tfull_bar[acc], acc_phase, 4);
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + acc * 256 + (static_cast<uint32_t>(quad * 32) << 16);
-            epilogue_row(p, taddr, col_base, 0, c_base, pix * p.ldr, row_ok, sbias, 0, p.bn);
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_leader(&tempty_bar[acc]);
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    }
-
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();  // neither CTA may free TMEM / exit while the pair's MMAs or remote arrives are in flight
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc_pair(tmem_base, 512);
-    }
-}
-
 // ------------------------------------------------------------------------------------------------ halo conv kernel
 // 3x3 implicit-GEMM conv whose pixel operand is loaded ONCE per 64-channel chunk instead of once per tap.  The pixel
 // tile is 8 (w) x 16 (h); its 10 x 18 halo (zero-filled outside the image by TMA) lands in shared memory as 180 rows of
@@ -963,11 +686,9 @@ constexpr int HALO_TX_BYTES = HALO_W * HALO_H * 128;  // 23040
 constexpr int HALO_BYTES = 23 * 1024;                 // buffer pitch, 1024-aligned
 constexpr int HALO_BUFS = 3;
 
-template <bool PRO>
-__global__ void __launch_bounds__(PRO ? GEMM_PRO_THREADS : GEMM_THREADS, 1)
+__global__ void __launch_bounds__(GEMM_THREADS, 1)
 tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmA2,
                     const __grid_constant__ CUtensorMap tmB, const __grid_constant__ GemmParams p) {
-    pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int b_bytes = p.bn * 128;
@@ -979,10 +700,9 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     uint64_t* bempty = bfull + GEMM_MAX_STAGES;
     uint64_t* tfull_bar = bempty + GEMM_MAX_STAGES;
     uint64_t* tempty_bar = tfull_bar + 2;
-    uint64_t* hfull = tempty_bar + 2;                    // halo buffer ready for the MMAs
+    uint64_t* hfull = tempty_bar + 2;  // halo buffer landed
     uint64_t* hempty = hfull + HALO_BUFS;
-    uint64_t* hraw = PRO ? hempty + HALO_BUFS : hfull;   // halo buffer landed (PRO: still to be transformed)
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(hempty + 2 * HALO_BUFS);
+    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(hempty + HALO_BUFS);
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
@@ -996,9 +716,8 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             mbar_init(&bempty[i], 1);
         }
         for (int i = 0; i < HALO_BUFS; ++i) {
-            mbar_init(&hfull[i], PRO ? GEMM_PRO_WARPS : 1);
+            mbar_init(&hfull[i], 1);
             mbar_init(&hempty[i], 1);
-            if (PRO) mbar_init(&hraw[i], 1);
         }
         for (int i = 0; i < 2; ++i) {
             mbar_init(&tfull_bar[i], 1);
@@ -1012,7 +731,6 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
-    pdl_wait();  // everything above touched only this kernel's own state; the predecessor's results are visible from here on
 
     const int num_tiles = p.m_tiles * p.n_tiles;
 
@@ -1025,17 +743,17 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 int n0, h0, w0;
                 decode_pix(p, (tile / p.n_tiles) % p.m_tiles, n0, h0, w0);
                 mbar_wait(&hempty[hs], hphase ^ 1, 5);
-                mbar_expect_tx(&hraw[hs], HALO_TX_BYTES);
+                mbar_expect_tx(&hfull[hs], HALO_TX_BYTES);
                 uint8_t* dst = smem + hs * HALO_BYTES;
                 if (kc < p.cchunks1)
-                    tma_load_4d(dst, &tmA, &hraw[hs], kc * 64, w0 - 1, h0 - 1, n0);
+                    tma_load_4d(dst, &tmA, &hfull[hs], kc * 64, w0 - 1, h0 - 1, n0);
                 else
-                    tma_load_4d(dst, &tmA2, &hraw[hs], (kc - p.cchunks1) * 64, w0 - 1, h0 - 1, n0);
+                    tma_load_4d(dst, &tmA2, &hfull[hs], (kc - p.cchunks1) * 64, w0 - 1, h0 - 1, n0);
                 if (++hs == HALO_BUFS) { hs = 0; hphase ^= 1; }
             };
             // Halo loads run AHEAD of the weight tiles by `ahead` chunk steps (a cursor over (tile, chunk) that only this
-            // thread advances): 1 step hides the TMA latency (and, with the GroupNorm prologue, the transform) under the nine
-            // MMAs of the current chunk; three buffers: loading / transforming, multiplying, draining.
+            // thread advances): 1 step hides the TMA latency under the nine MMAs of the current chunk; three buffers:
+            // loading, multiplying, draining.
             int cur_tile = blockIdx.x, cur_kc = 0;
             auto next_halo = [&]() {
                 if (cur_tile >= num_tiles) return;
@@ -1106,98 +824,8 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
         }
-    } else if (warp < 2 + GEMM_EPI_WARPS) {
+    } else {
         epilogue_warps<GEMM_CONV>(p, smem, tmem_base, tfull_bar, tempty_bar, warp, lane, num_tiles);
-    } else if (PRO) {
-        // =========================================================== GroupNorm + SiLU (+ dropout) prologue warps
-        // Thread tt owns the 16-byte unit u = tt & 7 (8 channels) of the rows r = tt >> 3, + PT / 8, ... of each 180-row halo
-        // tile.  A row is one halo pixel; rows outside the image were zero-filled by TMA and must stay zero (the conv pads
-        // the ACTIVATED tensor), channels beyond the valid count get A = B = 0 (silu(0) = 0).
-        constexpr int PT = 32 * GEMM_PRO_WARPS;
-        const int tt = threadIdx.x - GEMM_THREADS;
-        const int u = tt & 7, r0 = tt >> 3;
-        float2* sco = reinterpret_cast<float2*>(smem + GEMM_SMEM_RING + 4096);  // [cchunks * 64] (A, B) of this tile's sample
-        const int C = p.pro_c1 + p.pro_c2, V = C >> 3;
-        unsigned long long seed = p.pro_seed;
-        if (p.pro_seed_dev != nullptr) seed += *p.pro_seed_dev * 0x9E3779B97F4A7C15ull;
-        const DropCtx dc = drop_ctx(seed, p.pro_drop_p);
-        int hs = 0;
-        uint32_t hphase = 0;
-        int last_n = -1;
-        for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-            int n0, h0, w0;
-            decode_pix(p, (tile / p.n_tiles) % p.m_tiles, n0, h0, w0);
-            const bool writer = p.pro_out != nullptr && (tile % p.n_tiles) == 0;
-            if (n0 != last_n) {  // (uniform over these warps) stage this sample's coefficients, padded per 64-channel chunk
-                asm volatile("bar.sync 2, %0;" ::"n"(PT) : "memory");
-                for (int i = tt; i < p.cchunks * 64; i += PT) {
-                    const int kc = i >> 6, cc = i & 63;
-                    const bool first = kc < p.cchunks1;
-                    const int ch = first ? kc * 64 + cc : (kc - p.cchunks1) * 64 + cc;
-                    const bool ok = ch < (first ? p.pro_c1 : p.pro_c2);
-                    float2 ab = make_float2(0.f, 0.f);
-                    if (ok) {
-                        const float4 t = __ldg(p.pro_coef + 1LL * n0 * C + (first ? ch : p.pro_c1 + ch));
-                        ab = p.pro_act ? make_float2(0.5f * t.x, 0.5f * t.y) : make_float2(t.x, t.y);
-                    }
-                    sco[i] = ab;
-                }
-                asm volatile("bar.sync 2, %0;" ::"n"(PT) : "memory");
-                last_n = n0;
-            }
-            for (int kc = 0; kc < p.cchunks; ++kc) {
-                mbar_wait(&hraw[hs], hphase, 7);
-                uint8_t* buf = smem + hs * HALO_BYTES;
-                float a[8], b[8];
-#pragma unroll
-                for (int j = 0; j < 8; j += 2) {
-                    const float4 t = *reinterpret_cast<const float4*>(sco + kc * 64 + u * 8 + j);
-                    a[j] = t.x; b[j] = t.y; a[j + 1] = t.z; b[j + 1] = t.w;
-                }
-                const bool first = kc < p.cchunks1;
-                const int cbase = first ? kc * 64 + u * 8 : p.pro_c1 + (kc - p.cchunks1) * 64 + u * 8;  // channel in the concat
-                const bool ch_ok = (first ? kc * 64 + u * 8 : (kc - p.cchunks1) * 64 + u * 8) < (first ? p.pro_c1 : p.pro_c2);
-#pragma unroll 1
-                for (int r = r0; r < HALO_W * HALO_H; r += PT / 8) {
-                    const int hy = r / HALO_W, hx = r - hy * HALO_W;
-                    const int y = h0 - 1 + hy, x = w0 - 1 + hx;
-                    if (y < 0 || y >= p.H || x < 0 || x >= p.W) continue;
-                    uint4* cell = reinterpret_cast<uint4*>(buf + r * 128 + ((u ^ (r & 7)) << 4));
-                    const uint4 raw = *cell;
-                    const uint32_t w4[4] = {raw.x, raw.y, raw.z, raw.w};
-                    float v[8];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        v[2 * j] = __uint_as_float(w4[j] << 16);
-                        v[2 * j + 1] = __uint_as_float(w4[j] & 0xFFFF0000u);
-                    }
-                    const long long pix = (static_cast<long long>(n0) * p.H + y) * p.W + x;
-                    float ds[8];
-                    if (p.pro_drop_p > 0.f)
-                        dropout_scales(dc, static_cast<uint32_t>(static_cast<unsigned long long>(pix) * V + (cbase >> 3)), ds);
-                    uint32_t o[4];
-#pragma unroll
-                    for (int j = 0; j < 8; j += 2) {
-                        float y0 = fmaf(v[j], a[j], b[j]), y1 = fmaf(v[j + 1], a[j + 1], b[j + 1]);
-                        if (p.pro_act) {
-                            y0 = fmaf(y0, gemm_tanh_fast(y0), y0);
-                            y1 = fmaf(y1, gemm_tanh_fast(y1), y1);
-                        }
-                        if (p.pro_drop_p > 0.f) { y0 *= ds[j]; y1 *= ds[j + 1]; }
-                        const __nv_bfloat162 b2 = __floats2bfloat162_rn(y0, y1);
-                        o[j >> 1] = *reinterpret_cast<const uint32_t*>(&b2);
-                    }
-                    const uint4 res = make_uint4(o[0], o[1], o[2], o[3]);
-                    *cell = res;
-                    if (writer && ch_ok && hy >= 1 && hy <= HALO_H - 2 && hx >= 1 && hx <= HALO_W - 2)
-                        *reinterpret_cast<uint4*>(p.pro_out + pix * p.pro_ldo + cbase) = res;
-                }
-                fence_proxy_async_smem();  // generic-proxy writes -> visible to the tensor core
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&hfull[hs]);
-                if (++hs == HALO_BUFS) { hs = 0; hphase ^= 1; }
-            }
-        }
     }
 
     tc_fence_before();
@@ -1221,7 +849,6 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 tc_wgrad_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                      const __grid_constant__ CUtensorMap tmB2, const __grid_constant__ GemmParams p) {
-    pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int halo_w = p.bw + 2;
@@ -1259,7 +886,6 @@ tc_wgrad_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
-    pdl_wait();  // everything above touched only this kernel's own state; the predecessor's results are visible from here on
 
     // tile = (sp * m_tiles + mt) * n_tiles + nt : CTAs running together share a pixel range (split) — its dY / X boxes
     // stay L2-resident.  (A stream-K division of the (tile, k) space balanced the SMs but was 10 % slower: neighbouring

@@ -1,4 +1,4 @@
-// Shared device helpers for the memory-side kernels (GroupNorm family, conv prologue):
+// Device helpers for the memory-side kernels (GroupNorm family):
 //   * packed fp32 arithmetic (sm_100 FFMA2 / FADD2 / FMUL2: two IEEE fp32 lanes per instruction, bit-identical to the
 //     scalar ops, half the issue slots),
 //   * bf16-pair <-> fp32-pair conversions,

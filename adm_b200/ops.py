@@ -187,16 +187,9 @@ def transpose_weight_tiles(src, dst, tiles):
     return dst
 
 
-def stats_ok(h, w):
-    """Image sizes for which the conv epilogue can emit GroupNorm statistics (see adm_conv_fprop_stats)."""
-    return h * w in (16, 64) or (h * w) % 128 == 0
-
-
 def conv_fprop(x1, wpk, x2=None, bias=None, residual=None, alpha=1.0, out_dtype=BF16, out=None, nout=None,
-               keep_pad=False, stats=False):
-    """Implicit-GEMM conv (3x3 pad 1 or 1x1) on NHWC bf16.  wpk: [nout, taps, kpad] bf16.
-    stats=True: returns (out, st) where st fp32 [N + 1, slots, nout, 2] holds the per-(sample, slot, channel) partial
-    sum / sum of squares of `out`, emitted by the conv epilogue for the next GroupNorm (gn_forward_stats)."""
+               keep_pad=False):
+    """Implicit-GEMM conv (3x3 pad 1 or 1x1) on NHWC bf16.  wpk: [nout, taps, kpad] bf16."""
     _need_cuda(x1, wpk)
     p1, c1, ld1, n, h, w = _nhwc(x1)
     p2, c2, ld2 = None, 0, 0
@@ -216,50 +209,10 @@ def conv_fprop(x1, wpk, x2=None, bias=None, residual=None, alpha=1.0, out_dtype=
     if residual is not None:
         assert residual.dtype == BF16 and residual.stride(3) == 1
         ldr = residual.stride(2)
-    st = None
-    if stats:
-        slots = _lib.load().adm_conv_stats_slots(h, w)
-        st = torch.empty(n + 1, slots, nout, 2, device=x1.device, dtype=F32)
-    check(_lib.load().adm_conv_fprop_stats(p1, c1, ld1, p2, c2, ld2, n, h, w, _ptr(wpk), nout, ntaps, _ptr(out),
-                                           0 if out.dtype == BF16 else 1, ldc, _ptr(bias), _ptr(residual), ldr,
-                                           float(alpha), _ptr(st), _stream()), "conv_fprop")
-    res = out[..., :nout] if (out.shape[-1] != nout and not keep_pad) else out
-    return (res, st) if stats else res
-
-
-def conv_gn_ok(h, w):
-    """Image sizes the conv with the fused GroupNorm prologue serves (8 x 16 pixel halo tiles)."""
-    return bool(_lib.load().adm_conv_gn_ok(int(h), int(w)))
-
-
-def conv_fprop_gn(x1, wpk, coef, x2=None, bias=None, residual=None, act=True, drop_p=0.0, seed=0, seed_counter=None,
-                  want_act=True):
-    """conv3x3(dropout(silu(x * A + B))) with the GroupNorm prologue fused into the conv: reads the RAW x1 (| x2) and the
-    norm's coefficient table coef [N, C, 4].  Returns (out, a) with a = the activated tensor [N, H, W, C] (what the
-    weight-gradient kernel needs; None when want_act is False, e.g. in inference)."""
-    _need_cuda(x1, wpk, coef)
-    p1, c1, ld1, n, h, w = _nhwc(x1)
-    p2, c2, ld2 = None, 0, 0
-    if x2 is not None:
-        p2, c2, ld2, n2, h2, w2 = _nhwc(x2)
-        assert (n2, h2, w2) == (n, h, w)
-    nout, ntaps, kpad = wpk.shape
-    assert ntaps == 9 and kpad == pad64(c1) + (pad64(c2) if x2 is not None else 0), (wpk.shape, c1, c2)
-    assert coef.dtype == F32 and tuple(coef.shape) == (n, c1 + c2, 4) and coef.is_contiguous()
-    ldc = (nout + 7) // 8 * 8
-    out = torch.empty(n, h, w, ldc, device=x1.device, dtype=BF16)
-    if ldc != nout:
-        out.zero_()
-    a = torch.empty(n, h, w, c1 + c2, device=x1.device, dtype=BF16) if want_act else None
-    ldr = 0
-    if residual is not None:
-        assert residual.dtype == BF16 and residual.stride(3) == 1
-        ldr = residual.stride(2)
-    check(_lib.load().adm_conv_fprop_gn(p1, c1, ld1, p2, c2, ld2, n, h, w, _ptr(wpk), nout, _ptr(out), ldc, _ptr(bias),
-                                        _ptr(residual), ldr, _ptr(coef), int(act), float(drop_p),
-                                        int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(seed_counter), _ptr(a),
-                                        a.stride(2) if a is not None else 0, _stream()), "conv_fprop_gn")
-    return (out[..., :nout] if ldc != nout else out), a
+    check(_lib.load().adm_conv_fprop(p1, c1, ld1, p2, c2, ld2, n, h, w, _ptr(wpk), nout, ntaps, _ptr(out),
+                                     0 if out.dtype == BF16 else 1, ldc, _ptr(bias), _ptr(residual), ldr, float(alpha),
+                                     _stream()), "conv_fprop")
+    return out[..., :nout] if (out.shape[-1] != nout and not keep_pad) else out
 
 
 def conv_dgrad(dy, wpk, n_valid=None, residual=None, alpha=1.0, out=None):
@@ -404,11 +357,10 @@ def gn_apply(x1, x2, coef, act=True, drop_p=0.0, seed=0, resample=0, seed_counte
 
 
 def gn_forward(x1, x2, gamma, beta, groups, eps=1e-5, params=None, act=True, drop_p=0.0, seed=0, resample=0,
-               seed_counter=None, apply=True):
+               seed_counter=None):
     """GroupNorm statistics + apply in one call (one cluster-per-sample kernel when the batch fills the SMs).
     seed_counter: optional CUDA int64[1] step counter mixed into the dropout seed (read only when drop_p > 0).
-    apply=False: statistics only (the coefficient table for a conv with the GroupNorm prologue, conv_fprop_gn).
-    Returns (coef [N, C, 4], y or None)."""
+    Returns (coef [N, C, 4], y)."""
     _need_cuda(x1)
     n, h, w, _ = x1.shape
     p1, c1, ld1 = _src(x1)
@@ -417,32 +369,13 @@ def gn_forward(x1, x2, gamma, beta, groups, eps=1e-5, params=None, act=True, dro
     work = torch.empty(2 * n * c + n, device=x1.device, dtype=F32)
     coef = torch.empty(n, c, 4, device=x1.device, dtype=F32)
     ho, wo = (h // 2, w // 2) if resample == 1 else ((2 * h, 2 * w) if resample == 2 else (h, w))
-    out = torch.empty(n, ho, wo, c, device=x1.device, dtype=BF16) if apply else None
+    out = torch.empty(n, ho, wo, c, device=x1.device, dtype=BF16)
     ldp = params.stride(0) if params is not None else 0
     check(_lib.load().adm_gn_forward(p1, c1, ld1, p2, c2, ld2, n, h, w, groups, float(eps), _ptr(gamma), _ptr(beta),
                                      _ptr(params), ldp, _ptr(work), _ptr(coef), int(act), float(drop_p),
                                      int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(seed_counter), int(resample), _ptr(out),
-                                     out.stride(2) if apply else c, _stream()), "gn_forward")
+                                     out.stride(2), _stream()), "gn_forward")
     return coef, out
-
-
-def gn_forward_stats(x1, st1, x2, st2, gamma, beta, groups, eps=1e-5, params=None, act=True, drop_p=0.0, seed=0,
-                     resample=0, seed_counter=None):
-    """gn_forward when the producers of x1 (and x2) already emitted their statistics (conv_fprop(stats=True)): a tiny
-    finalize kernel builds the coefficient table and ONE streaming pass applies it — the activation is read once.
-    Returns (coef [N, C, 4], y)."""
-    _need_cuda(x1, st1)
-    n, h, w, _ = x1.shape
-    c1 = x1.shape[-1]
-    c2 = x2.shape[-1] if x2 is not None else 0
-    assert st1.shape[0] == n + 1 and st1.shape[2] == c1 and (x2 is None or (st2.shape[0] == n + 1 and st2.shape[2] == c2))
-    coef = torch.empty(n, c1 + c2, 4, device=x1.device, dtype=F32)
-    ldp = params.stride(0) if params is not None else 0
-    check(_lib.load().adm_gn_finalize(_ptr(st1), st1.shape[1], c1, _ptr(st2), st2.shape[1] if st2 is not None else 0, c2,
-                                      n, h * w, groups, float(eps), _ptr(gamma), _ptr(beta), _ptr(params), ldp,
-                                      _ptr(coef), _stream()), "gn_finalize")
-    y = gn_apply(x1, x2, coef, act=act, drop_p=drop_p, seed=seed, resample=resample, seed_counter=seed_counter)
-    return coef, y
 
 
 def gn_bwd(dy, x1, x2, coef, gamma, beta, groups, params=None, act=True, drop_p=0.0, seed=0, resample=0,

@@ -74,7 +74,7 @@ class ParamArena:
         fp32 flat slice, bf16 [Cin, k*k, Cout] or None)``.  The last entry is the DGRAD shadow: the same weights
         transposed with the taps mirrored (Cout a multiple of 64), re-derived from the bf16 shadow by ONE batched tile
         transpose per optimizer step, so the data gradient of a conv runs through the fprop kernels on a K-major
-        operand instead of the slower MN-major view of the fprop-packed weights (ADM_DGRAD_SHADOW=0 disables)."""
+        operand instead of the slower MN-major view of the fprop-packed weights."""
         params = order if order is not None else list(module.parameters())
         dev = params[0].device
         cl = {id(p) for p in channels_last}
@@ -88,8 +88,7 @@ class ParamArena:
         self.flat = torch.zeros(total, device=dev, dtype=torch.float32)
         self.grads = torch.zeros(total, device=dev, dtype=torch.float32)
         self.shadow = torch.zeros(total, device=dev, dtype=torch.bfloat16) if (cl and dev.type == "cuda") else None
-        want_t = self.shadow is not None and os.environ.get("ADM_DGRAD_SHADOW", "1") != "0"
-        self.shadow_t = torch.zeros(total, device=dev, dtype=torch.bfloat16) if want_t else None
+        self.shadow_t = torch.zeros(total, device=dev, dtype=torch.bfloat16) if self.shadow is not None else None
         self.t_tiles = None
         tiles = []
         self._grad_views = []
@@ -233,10 +232,10 @@ class TrainStep:
         """The qkv projections run in (q | k | v) x head x d row order (the reference interleaves (head, d, {q,k,v}),
         unet/uncond_unet.py:205).  Instead of re-packing 24 weights and biases every step, keep ONE bf16 buffer with all of
         them in executed order plus a byte-offset table, and re-derive it from the arena's bf16 shadow (weights) and fp32
-        masters (biases) with two batched row-gather launches per optimizer step (ADM_QKV_GATHER=0 disables)."""
+        masters (biases) with two batched row-gather launches per optimizer step."""
         a, eng = self.arena, self.engine
         self._qkv = None
-        if a.shadow is None or os.environ.get("ADM_QKV_GATHER", "1") == "0":
+        if a.shadow is None:
             return
         off = {id(p): o for p, o in zip(a.params, a.offsets)}
         blocks = [m for _, m, _ in eng.block_list
@@ -540,8 +539,7 @@ class TrainStep:
         else:
             self.engine.grad_hook = None
         # first backward into a zeroed arena: the grouped affine weight gradient may be stored instead of accumulated
-        self.engine.affine_grad_overwrite = (self._grads_clean and self.engine.affine_pack is not None
-                                             and os.environ.get("ADM_AFFINE_OVERWRITE", "1") != "0")
+        self.engine.affine_grad_overwrite = self._grads_clean and self.engine.affine_pack is not None
         self._grads_clean = False
         if set(kw) <= {"augment_labels"}:
             return self._direct_step(x, t, noise, kw.get("augment_labels"))

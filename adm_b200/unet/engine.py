@@ -58,22 +58,6 @@ class UNetEngine:
         # ADM_WGRAD_STREAM=0 keeps everything on one stream.
         self._side = None
         self._side_on = os.environ.get("ADM_WGRAD_STREAM", "1") != "0"
-        # ADM_GN_STATS=1: GroupNorm statistics come from the epilogue of the conv that produced the tensor
-        # (adm_conv_fprop_stats + adm_gn_finalize) instead of the norm re-reading its input.  Exact and tested, but OFF by
-        # default: measured on B200 (profiles/r03_gn_stats_epilogue_microbench.txt) the cross-lane column reduction makes
-        # the epilogue-bound convs 13-120 % slower while the norm's own statistics pass costs only ~3 us of its 24 us
-        # (its apply pass is instruction-issue bound) — the step is 1.4 ms slower with it.
-        self._gn_stats = os.environ.get("ADM_GN_STATS", "0") == "1"
-        # the data gradients fed to the GroupNorm backward kernels are consumed only there: let the kernel use them as
-        # scratch (it stores the pre-activation gradient in place between its passes).  ADM_GN_DVREUSE=0 for A/B timing.
-        self._dy_scratch = os.environ.get("ADM_GN_DVREUSE", "1") != "0"
-        # GroupNorm + SiLU (+ dropout) as a PROLOGUE of the 3x3 conv that consumes it (adm_conv_fprop_gn) wherever the image
-        # tiles into halo boxes and no resample sits between norm and conv: the norm kernel then only computes statistics.
-        # Bit-identical to the two-kernel path and tested, but OFF by default: measured on B200 it is break-even at best
-        # (profiles/r03_conv_gn_prologue.txt — the transform of a halo chunk is not fully hidden under its nine MMAs, and in
-        # training it also hashes the dropout masks and writes out the tensor the weight gradients need).
-        # ADM_CONV_GN=1: in inference (sampler) only, 2: also in training.
-        self._conv_gn = int(os.environ.get("ADM_CONV_GN", "0"))
         self._side_pending = []
         # device-resident step counter mixed into every dropout seed (fresh masks per CUDA-graph replay); owned by the
         # training step (adm_b200.train.TrainStep) and passed to the GroupNorm kernels per call
@@ -362,21 +346,7 @@ class UNetEngine:
         return self._cached(("projpad", id(blk)), [blk.proj.weight], build)
 
     # ------------------------------------------------------------------------------------------ UNetBlock
-    def _gn(self, x1, st1, x2, st2, norm, groups, **kw):
-        """GroupNorm (+ activation ...) of the fused concat (x1 | x2): from the producers' epilogue statistics when both
-        sources carry them (one finalize + one streaming pass), else statistics + apply in the cluster kernel."""
-        if st1 is not None and (x2 is None or st2 is not None):
-            return ops.gn_forward_stats(x1, st1, x2, st2, norm.weight, norm.bias, groups, norm.eps, **kw)
-        return ops.gn_forward(x1, x2, norm.weight, norm.bias, groups, norm.eps, **kw)
-
-    def _conv_stats(self, x, *args, **kw):
-        """conv_fprop that also returns the GroupNorm statistics of its output when the image size allows it."""
-        if self._gn_stats and ops.stats_ok(x.shape[1], x.shape[2]):
-            return ops.conv_fprop(x, *args, stats=True, **kw)
-        return ops.conv_fprop(x, *args, **kw), None
-
-    def block_fwd(self, blk, x1, x2, params, training, seed, save, st1=None, st2=None):
-        """Returns (block output, its epilogue statistics or None)."""
+    def block_fwd(self, blk, x1, x2, params, training, seed, save):
         c = NS(blk=blk, x1=x1, x2=x2, params=params, seed=seed)
         cin1 = x1.shape[-1]
         cin2 = x2.shape[-1] if x2 is not None else 0
@@ -384,52 +354,29 @@ class UNetEngine:
         mode = 1 if blk.down else (2 if blk.up else 0)
         c.mode = mode
         c.drop_p = float(blk.dropout) if training else 0.0
-        n_, hh, ww, _ = x1.shape
-        want_act = save is not None  # the activated tensors are only needed by the weight gradients
-        use_pro = self._conv_gn == 2 or (self._conv_gn == 1 and not want_act)
-        fuse0 = use_pro and mode == 0 and ops.conv_gn_ok(hh, ww) and not (cin1 % 8 or cin2 % 8) \
-            and (x2 is None or cin1 % 64 == 0)
-        if fuse0:  # conv0(silu(norm0(x))) in one kernel: statistics here, normalisation in the conv's prologue
-            c.sums0, _ = ops.gn_forward(x1, x2, blk.norm0.weight, blk.norm0.bias, _groups(cin), blk.norm0.eps, act=True,
-                                        apply=False)
-            # (cin1 % 64 == 0: the packed weights of the concatenated input and of the two sources are the same buffer)
-            c.h0, c.a0 = ops.conv_fprop_gn(x1, self.conv_w(blk.conv0), c.sums0, x2=x2, bias=blk.conv0.bias, act=True,
-                                           want_act=want_act)
-            st_h0 = None
-        else:
-            c.sums0, c.a0 = self._gn(x1, st1, x2, st2, blk.norm0, _groups(cin), act=True, resample=mode)
-            # after the fused concat-GroupNorm the conv sees ONE tensor a0 with cin channels
-            c.h0, st_h0 = self._conv_stats(c.a0, self.conv_w(blk.conv0), bias=blk.conv0.bias)
-        ho, wo = c.h0.shape[1], c.h0.shape[2]
-        fuse1 = use_pro and ops.conv_gn_ok(ho, wo) and cout % 8 == 0
-        if fuse1:
-            c.sums1, c.a1 = ops.gn_forward(c.h0, None, blk.norm1.weight, blk.norm1.bias, _groups(cout), blk.norm1.eps,
-                                           params=params, act=True, apply=False)
-        else:
-            c.sums1, c.a1 = self._gn(c.h0, st_h0, None, None, blk.norm1, _groups(cout), params=params, act=True,
-                                     drop_p=c.drop_p, seed=seed, seed_counter=self.seed_counter)
+        c.sums0, c.a0 = ops.gn_forward(x1, x2, blk.norm0.weight, blk.norm0.bias, _groups(cin), blk.norm0.eps, act=True,
+                                       resample=mode)
+        # after the fused concat-GroupNorm the conv sees ONE tensor a0 with cin channels
+        c.h0 = ops.conv_fprop(c.a0, self.conv_w(blk.conv0), bias=blk.conv0.bias)
+        c.sums1, c.a1 = ops.gn_forward(c.h0, None, blk.norm1.weight, blk.norm1.bias, _groups(cout), blk.norm1.eps,
+                                       params=params, act=True, drop_p=c.drop_p, seed=seed, seed_counter=self.seed_counter)
         if blk.skip is not None and blk.skip.weight is not None:
             res = ops.conv_fprop(x1, self.conv_w(blk.skip, cin1, cin2), x2=x2, bias=blk.skip.bias)
         elif mode:
             res = ops.resample(x1, mode)
         else:
             res = x1
-        if fuse1:  # conv1(dropout(silu(norm1(h0) * (1 + scale) + shift))) + residual in one kernel
-            c.h1, c.a1 = ops.conv_fprop_gn(c.h0, self.conv_w(blk.conv1), c.sums1, bias=blk.conv1.bias, residual=res,
-                                           act=True, drop_p=c.drop_p, seed=seed, seed_counter=self.seed_counter,
-                                           want_act=want_act)
-            st_out = None
-        else:
-            c.h1, st_out = self._conv_stats(c.a1, self.conv_w(blk.conv1), bias=blk.conv1.bias, residual=res)
+        c.h1 = ops.conv_fprop(c.a1, self.conv_w(blk.conv1), bias=blk.conv1.bias, residual=res)
         out = c.h1
         if blk.num_heads:
-            c.sums2, c.a2 = self._gn(c.h1, st_out, None, None, blk.norm2, _groups(cout), act=False)
+            c.sums2, c.a2 = ops.gn_forward(c.h1, None, blk.norm2.weight, blk.norm2.bias, _groups(cout), blk.norm2.eps,
+                                           act=False)
             if (cout // blk.num_heads) % 64:  # head width 72 / 96: zero-padded heads
                 wq, bq, _ = self.qkv_padded(blk)
                 c.qkv = ops.conv_fprop(c.a2, wq, bias=bq)
                 c.att, c.p = ops.attention_fwd(c.qkv, blk.num_heads, scale=(cout // blk.num_heads) ** -0.5,
                                                need_p=save is not None)
-                out, st_out = self._conv_stats(c.att, self.proj_padded(blk), bias=blk.proj.bias, residual=c.h1)
+                out = ops.conv_fprop(c.att, self.proj_padded(blk), bias=blk.proj.bias, residual=c.h1)
             else:
                 perm = self.qkv_perm(cout, blk.num_heads)
                 qp = self._qkv_pack_of(blk, perm)
@@ -442,10 +389,10 @@ class UNetEngine:
                     wq = self.conv_w(blk.qkv, perm=perm[0])
                 c.qkv = ops.conv_fprop(c.a2, wq, bias=bq)
                 c.att, c.p = ops.attention_fwd(c.qkv, blk.num_heads, need_p=save is not None)
-                out, st_out = self._conv_stats(c.att, self.conv_w(blk.proj), bias=blk.proj.bias, residual=c.h1)
+                out = ops.conv_fprop(c.att, self.conv_w(blk.proj), bias=blk.proj.bias, residual=c.h1)
         if save is not None:
             save.append(c)
-        return out, st_out
+        return out
 
     def export_dropout_masks(self, tape):
         """The dropout keep-masks (already scaled by 1/(1-p)) a training forward drew, one NCHW fp32 tensor per UNetBlock,
@@ -525,10 +472,11 @@ class UNetEngine:
         # h1 = conv1(a1) + b1 + skip(x)
         self._conv_param_grads(blk.conv1, dh1, c.a1, bias_done=h1_bias_done)
         da1 = self._dgrad(dh1, blk.conv1, self.conv_w(blk.conv1))
+        # da1 / da0 are consumed only by the GroupNorm backward: dy_scratch lets it keep the pre-activation gradient there
         dh0, _ = ops.gn_bwd(da1, c.h0, None, c.sums1, blk.norm1.weight, blk.norm1.bias, _groups(cout),
                             params=c.params, act=True, drop_p=c.drop_p, seed=c.seed, seed_counter=self.seed_counter,
                             dgamma=self._grad(blk.norm1.weight), dbeta=self._grad(blk.norm1.bias), dparams=dparams,
-                            dbias1=self._grad(blk.conv0.bias), dy_scratch=self._dy_scratch)
+                            dbias1=self._grad(blk.conv0.bias), dy_scratch=True)
         # h0 = conv0(a0) + b0
         self._conv_param_grads(blk.conv0, dh0, c.a0, bias_done=True)
         da0 = self._dgrad(dh0, blk.conv0, self.conv_w(blk.conv0))
@@ -543,7 +491,7 @@ class UNetEngine:
         return ops.gn_bwd(da0, c.x1, c.x2, c.sums0, blk.norm0.weight, blk.norm0.bias, _groups(cin),
                           act=True, resample=c.mode, dgamma=self._grad(blk.norm0.weight),
                           dbeta=self._grad(blk.norm0.bias), add=add, add_mode=add_mode, dbias1=s0, dbias1b=s1,
-                          dy_scratch=self._dy_scratch)
+                          dy_scratch=True)
 
     # ------------------------------------------------------------------------------------------ embedding MLP
     def embed_fwd(self, c_noise, aug, save):
@@ -595,8 +543,7 @@ class UNetEngine:
                                       accumulate=True)
                 ops.col_sums(dpb[:, off:off + o], self._grad(m.affine.bias))
         # [B, sum 2*Cout] x [sum 2*Cout, emb]: K = 45 k with three output tiles -> split K over the idle SMs
-        # (ADM_DEMB_SPLIT=0: A/B timing)
-        splits = 1 if os.environ.get("ADM_DEMB_SPLIT", "1") == "0" else max(1, min(40, wall.shape[0] // 1024))
+        splits = max(1, min(40, wall.shape[0] // 1024))
         demb = ops.gemm_nn(dpb, wall, splits=splits)
         _, de1b = ops.silu_bwd(e.e1, demb, want_f32=False)
         self._linear_grads(net.map_layer1, de1b, e.s0b)
@@ -651,23 +598,23 @@ class UNetEngine:
             tape.emb = emb_save[0]
             tape.dparams_all = torch.zeros_like(params_all)
 
-        def run_block(m, x1, x2, idx, st1=None, st2=None):
+        def run_block(m, x1, x2, idx):
             off = boff[id(m)]
             return self.block_fwd(m, x1, x2, params_all[:, off:off + m.affine.out_features], training,
-                                  step_seed * 4099 + idx, save, st1, st2)
+                                  step_seed * 4099 + idx, save)
 
-        x, st = xin, None
-        skips = []  # (tensor, epilogue statistics) of every encoder entry
+        x = xin
+        skips = []  # output of every encoder entry
         idx = 0
         for name, m in net.enc.items():
             if hasattr(m, "affine"):
-                x, st = run_block(m, x, None, idx, st)
+                x = run_block(m, x, None, idx)
             else:
-                x, st = self._conv_stats(x, self.conv_w(m, c1=m.in_channels), bias=m.bias)
+                x = ops.conv_fprop(x, self.conv_w(m, c1=m.in_channels), bias=m.bias)
                 if tape is not None:
                     tape.first = NS(conv=m, x=xin)
             idx += 1
-            skips.append((x, st))
+            skips.append(x)
         outs = []
         # The two decoders only share their inputs (bottleneck, skips, embedding): the second one is enqueued on the
         # side stream, forked HERE (before decoder 1 is enqueued), so their kernels interleave on the SMs — most of
@@ -686,14 +633,14 @@ class UNetEngine:
                 self._side_pending.append((x, skips, params_all))
                 ctx = torch.cuda.stream(self._side)
             with ctx:
-                h, hst = self.decouple_fwd(getattr(net, dname), x, save), None
+                h = self.decouple_fwd(getattr(net, dname), x, save)
                 sk = list(skips)
                 for name, m in dec.items():
-                    x2, st2 = sk.pop() if h.shape[-1] != m.in_channels else (None, None)
-                    h, hst = run_block(m, h, x2, idx, hst, st2)
+                    x2 = sk.pop() if h.shape[-1] != m.in_channels else None
+                    h = run_block(m, h, x2, idx)
                     idx += 1
                 o = NS(x=h, norm=norm, conv=oconv)
-                o.sums, o.a = self._gn(h, hst, None, None, norm, _groups(h.shape[-1]), act=True)
+                o.sums, o.a = ops.gn_forward(h, None, norm.weight, norm.bias, _groups(h.shape[-1]), norm.eps, act=True)
                 f = ops.conv_fprop(o.a, self.conv_w(oconv), bias=oconv.bias, out_dtype=F32, keep_pad=True)
                 if save is not None:
                     save.append(o)
@@ -750,7 +697,7 @@ class UNetEngine:
             dh, _ = ops.gn_bwd(da, o.x, None, o.sums, o.norm.weight, o.norm.bias, _groups(o.x.shape[-1]),
                                act=True, dgamma=self._grad(o.norm.weight), dbeta=self._grad(o.norm.bias),
                                dbias1=sinks[0], dbias1b=sinks[1] if len(sinks) > 1 else None,
-                               dy_scratch=self._dy_scratch)
+                               dy_scratch=True)
             self._notify(o.conv, o.norm)
             si = 0  # forward pops skips from the end, so walking the decoder backwards meets skips[0], skips[1], ...
             while not hasattr(items[pos - 1], "seq"):

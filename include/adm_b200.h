@@ -83,30 +83,6 @@ int adm_unet_output_bwd(const float* dd1, const float* dd2, const float* sigma, 
 int adm_conv_fprop(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h, int w,
                    const void* wpk, int nout, int ntaps, void* out, int out_mode, long long ldc, const float* bias,
                    const void* residual, long long ldr, float alpha, void* stream);
-/* Same, and the epilogue also emits the GroupNorm statistics of what it stores (SURVEY 8 a-8: "epilogue = ... GN-stat
- * partials for the next norm"): stats fp32 [n + 1][slots][nout][2] receives, per sample / slot / channel, the partial
- * {sum, sum of squares} over the <= 32 pixels one epilogue warp holds (slots = adm_conv_stats_slots(h, w) = h*w/32, at
- * least 1; the extra sample row is scratch for ragged tiles).  Plain stores: no atomics, no zeroing, deterministic.
- * adm_gn_finalize turns them into the coefficient table, so the following norm (unet/uncond_unet.py:128) never
- * re-reads its input for statistics.  stats == NULL is adm_conv_fprop.  Needs h*w in {16, 64, k*128}, bf16 output. */
-int adm_conv_fprop_stats(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h,
-                         int w, const void* wpk, int nout, int ntaps, void* out, int out_mode, long long ldc,
-                         const float* bias, const void* residual, long long ldr, float alpha, float* stats,
-                         void* stream);
-int adm_conv_stats_slots(int h, int w);
-/* conv3x3 with the GroupNorm(+ adaptive scale/shift) + SiLU (+ dropout) PROLOGUE fused in (north_star; UNetBlock.forward,
- * unet/uncond_unet.py:191 `conv0(silu(norm0(x)))` and :196-200 `conv1(dropout(silu(addcmul(shift, norm1(x), scale+1))))`):
- * the conv reads the RAW tensor x1 (| x2); four extra warps apply y = dropout(silu(x*A[n,c] + B[n,c])) to every halo
- * tile in shared memory, once per 64-channel chunk, between the TMA load and the tcgen05 MMAs, so the normalised tensor
- * is never read back from HBM.  coef = the norm's table [n][c1+c2]{A, B, mean, rstd} (adm_gn_stats / adm_gn_forward with
- * out == NULL); seed / seed_counter / drop_p as adm_gn_apply (the backward regenerates the same masks); a_out (optional,
- * bf16 [n][h][w][ld_a]) receives the activated tensor once — the operand adm_conv_wgrad needs in training.
- * Images must tile into 8 x 16 pixel boxes (adm_conv_gn_ok).  Output bf16.                                     */
-int adm_conv_fprop_gn(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h, int w,
-                      const void* wpk, int nout, void* out, long long ldc, const float* bias, const void* residual,
-                      long long ldr, const float* coef, int act, float drop_p, unsigned long long seed,
-                      const unsigned long long* seed_counter, void* a_out, long long ld_a, void* stream);
-int adm_conv_gn_ok(int h, int w);
 /* data gradient: dx[pix][0:n_valid] = alpha * conv^T(dy) + residual, reading the SAME packed weights through a
  * (Cin, tap, Cout) view with reversed taps; kpad = padded input channels of the forward conv.              */
 int adm_conv_dgrad(const void* dy, int cout, long long ld_dy, int n, int h, int w, const void* wpk, int kpad,
@@ -196,11 +172,6 @@ int adm_gn_stats(const void* x1, int c1, long long ld1, const void* x2, int c2, 
 /*   Pass 1: per-(sample, channel) sum / sum of squares, then the coefficient table coef[n][c] = {A, B, mean, rstd}
  *   (fp32 x4) with GN(x)[*(1+scale)+shift] = x*A + B; params = [n][ld_params] holding (scale | shift) or NULL.
  *   work: fp32 scratch of 2*n*C + n elements (zeroed by the call).                                             */
-/* The coefficient table of adm_gn_stats from statistics a producer already emitted (adm_conv_fprop_stats), for one or
- * two (fused channel concat) sources: st1 [n+1][slots1][c1][2], st2 [n+1][slots2][c2][2] or NULL.  One small kernel. */
-int adm_gn_finalize(const float* st1, int slots1, int c1, const float* st2, int slots2, int c2, int n, int hw,
-                    int groups, float eps, const float* gamma, const float* beta, const float* params,
-                    long long ld_params, float* coef, void* stream);
 /* y = act(x*A + B); act 1 = SiLU; drop_p > 0 applies Philox dropout keyed by seed; resample 0 none / 1 2x2 average /
  * 2 nearest x2.                                                                                              */
 int adm_gn_apply(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h, int w,
@@ -225,7 +196,7 @@ int adm_gn_bwd(const void* dy, long long ldy, const void* x1, int c1, long long 
  *   over dx1 is needed.
  * adm_gn_forward = gn_stats + gn_apply in one call.  When the batch fills the SMs it runs ONE kernel with a
  * thread-block cluster per sample (statistics exchanged through distributed shared memory, apply pass re-reading the
- * sample from L2); adm_gn_bwd does the same for the backward pair.  out == NULL computes the coefficient table only. */
+ * sample from L2); adm_gn_bwd does the same for the backward pair.                                            */
 int adm_gn_forward(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h, int w,
                    int groups, float eps, const float* gamma, const float* beta, const float* params,
                    long long ld_params, float* work, float* coef, int act, float drop_p, unsigned long long seed,

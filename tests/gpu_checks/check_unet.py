@@ -142,60 +142,6 @@ def groupnorm():
 
 
 @case
-def gn_stats_epilogue():
-    """GroupNorm statistics emitted by the conv epilogue (adm_conv_fprop_stats) + adm_gn_finalize + the streaming apply,
-    against F.group_norm on the conv output and against the statistics-kernel path; every tile geometry: 32x32 / 16x16
-    (halo tiles, 8 / 2 per image), 8x8 (two images per tile), 4x4 (eight per tile, half-warp segments, ragged batch),
-    1x1 convs with a residual, a fused channel concat of two producers."""
-    import torch
-    import torch.nn.functional as F
-    from adm_b200 import ops
-    torch.manual_seed(11)
-    ok = True
-    for (n, hw, cin, cout, k, with_res) in [(4, 32, 64, 192, 3, False), (6, 16, 128, 384, 3, True), (5, 8, 64, 192, 3, False),
-                                            (13, 4, 128, 384, 3, True), (16, 16, 192, 96, 1, True), (3, 8, 128, 72, 1, False),
-                                            (130, 4, 64, 64, 3, False)]:
-        x = (torch.randn(n, hw, hw, cin, device="cuda")).bfloat16()
-        wt = (torch.randn(cout, cin, k, k, device="cuda") / (k * cin ** 0.5))
-        bias = 0.1 * torch.randn(cout, device="cuda")
-        res = torch.randn(n, hw, hw, cout, device="cuda").bfloat16() if with_res else None
-        wpk = ops.pack_conv_weight(wt)
-        y0 = ops.conv_fprop(x, wpk, bias=bias, residual=res)
-        y, st = ops.conv_fprop(x, wpk, bias=bias, residual=res, stats=True)
-        # y0 may come from the cluster split-K kernel (another fp32 summation order): equal up to the bf16 rounding
-        ok &= _report(f"stats-epilogue output vs plain n{n} {hw}x{hw} {cin}->{cout} k{k}", y, y0, 4e-3)
-        ok &= tuple(st.shape) == (n + 1, max(1, hw * hw // 32), cout, 2)
-        ref = y.float()
-        tot = st[:n].sum(1)  # [n, cout, 2]
-        ok &= _report(f"epilogue sum   n{n} {hw}x{hw} {cin}->{cout} k{k}", tot[..., 0], ref.sum((1, 2)), 2e-5)
-        ok &= _report(f"epilogue sumsq n{n} {hw}x{hw} {cin}->{cout} k{k}", tot[..., 1], (ref * ref).sum((1, 2)), 2e-5)
-        g = min(32, cout // 4)
-        gamma = 1 + 0.1 * torch.randn(cout, device="cuda")
-        beta = 0.1 * torch.randn(cout, device="cuda")
-        params = 0.3 * torch.randn(n, 2 * cout, device="cuda")
-        coef_s, ys = ops.gn_forward_stats(y, st, None, None, gamma, beta, g, 1e-5, params=params, act=True)
-        coef_k, yk = ops.gn_forward(y, None, gamma, beta, g, 1e-5, params=params, act=True)
-        ok &= _report("  coef from epilogue stats vs stats kernel", coef_s, coef_k, 1e-4)
-        ok &= _report("  y from epilogue stats vs stats kernel", ys, yk, 4e-3)
-        v = F.group_norm(ref.permute(0, 3, 1, 2), g, gamma, beta, 1e-5)
-        v = F.silu(v * (1 + params[:, :cout, None, None]) + params[:, cout:, None, None])
-        ok &= _report("  y vs F.group_norm", ys, v.permute(0, 2, 3, 1), 6e-3)
-    # fused concat of two producers with different channel counts (group 21 of cat(384, 192) straddles the sources)
-    n, hw = 4, 16
-    xa = torch.randn(n, hw, hw, 64, device="cuda").bfloat16()
-    wa = ops.pack_conv_weight(torch.randn(384, 64, 3, 3, device="cuda") / 24)
-    wb = ops.pack_conv_weight(torch.randn(192, 64, 1, 1, device="cuda") / 8)
-    ya, sa = ops.conv_fprop(xa, wa, stats=True)
-    yb, sb = ops.conv_fprop(xa, wb, stats=True)
-    gamma = 1 + 0.1 * torch.randn(576, device="cuda")
-    beta = 0.1 * torch.randn(576, device="cuda")
-    coef_s, ys = ops.gn_forward_stats(ya, sa, yb, sb, gamma, beta, 32, 1e-5, act=True)
-    v = F.silu(F.group_norm(torch.cat([ya, yb], -1).float().permute(0, 3, 1, 2), 32, gamma, beta, 1e-5))
-    ok &= _report("concat (384 | 192) from two producers vs F.group_norm", ys, v.permute(0, 2, 3, 1), 6e-3)
-    return ok
-
-
-@case
 def conv_splitk():
     """Cluster split-K conv (tc_conv_splitk_kernel): fprop and dgrad at the under-filled 4x4 / 8x8 levels, with the split
     the cost model picks and with forced (tile width, split) pairs, against fp32 torch convolutions of the same bf16 data."""
@@ -231,59 +177,6 @@ def conv_splitk():
         os.environ.pop("ADM_SPLITK_FORCE", None)
         if old is not None:
             os.environ["ADM_SPLITK_FORCE"] = old
-    return ok
-
-
-@case
-def conv_gn_prologue():
-    """adm_conv_fprop_gn (GroupNorm + adaptive scale/shift + SiLU + dropout applied to the halo tiles in shared memory inside
-    the conv) against the two-kernel path gn_apply -> conv_fprop: the activated tensor it writes out and the conv result
-    must be BIT-identical (same formula, same rounding, same MMA order); plus fp32 torch as the outer reference."""
-    import torch
-    import torch.nn.functional as F
-    from adm_b200 import ops
-    torch.manual_seed(12)
-    ok = True
-    for (n, h, w, c1, c2, cout, drop, with_res, act) in [(4, 16, 16, 128, 0, 192, 0.0, False, True),
-                                                         (3, 32, 32, 64, 0, 64, 0.1, True, True),
-                                                         (5, 16, 16, 128, 64, 384, 0.0, False, True),
-                                                         (2, 32, 16, 192, 192, 96, 0.1, True, True),
-                                                         (6, 16, 8, 96, 0, 192, 0.0, False, True),
-                                                         (130, 16, 16, 64, 0, 64, 0.1, False, False)]:
-        c = c1 + c2
-        x1 = (torch.randn(n, h, w, c1, device="cuda") * 1.3 + 0.2).bfloat16()
-        x2 = (torch.randn(n, h, w, c2, device="cuda") * 0.8 - 0.1).bfloat16() if c2 else None
-        wt = torch.randn(cout, c, 3, 3, device="cuda") / (3 * c ** 0.5)
-        bias = 0.1 * torch.randn(cout, device="cuda")
-        res = torch.randn(n, h, w, cout, device="cuda").bfloat16() if with_res else None
-        gamma = 1 + 0.1 * torch.randn(c, device="cuda")
-        beta = 0.1 * torch.randn(c, device="cuda")
-        params = 0.3 * torch.randn(n, 2 * c, device="cuda")
-        g = min(32, c // 4)
-        wpk = ops.pack_conv_weight(wt, c1, c2) if c2 else ops.pack_conv_weight(wt)
-        coef, _ = ops.gn_forward(x1, x2, gamma, beta, g, 1e-5, params=params, act=act, apply=False)
-        a_ref = ops.gn_apply(x1, x2, coef, act=act, drop_p=drop, seed=99)
-        wpk1 = ops.pack_conv_weight(wt)  # single concatenated source
-        y_ref = ops.conv_fprop(a_ref, wpk1, bias=bias, residual=res)
-        y, a = ops.conv_fprop_gn(x1, wpk, coef, x2=x2, bias=bias, residual=res, act=act, drop_p=drop, seed=99)
-        tag = f"n{n} {h}x{w} {c1}+{c2}->{cout} drop{drop} act{int(act)}"
-        eq_a = bool(torch.equal(a, a_ref))
-        print(f"  {tag}: activated tensor bit-equal {eq_a}", flush=True)
-        ok &= eq_a
-        # y_ref may come from the cluster split-K kernel (another fp32 summation order): equal up to the bf16 rounding
-        ok &= _report(f"conv output vs unfused {tag}", y, y_ref, 4e-3)
-        y2, none = ops.conv_fprop_gn(x1, wpk, coef, x2=x2, bias=bias, residual=res, act=act, drop_p=drop, seed=99,
-                                     want_act=False)
-        ok &= none is None and bool(torch.equal(y2, y))
-        if drop == 0.0:
-            xc = torch.cat([x1, x2], -1) if c2 else x1
-            v = F.group_norm(xc.float().permute(0, 3, 1, 2), g, gamma, beta, 1e-5)
-            v = v * (1 + params[:, :c, None, None]) + params[:, c:, None, None]
-            v = F.silu(v) if act else v
-            yr = F.conv2d(v, wt, bias, padding=1)
-            if res is not None:
-                yr = yr + res.float().permute(0, 3, 1, 2)
-            ok &= _report(f"  {tag} vs fp32 torch", y, yr.permute(0, 2, 3, 1), 1.5e-2)
     return ok
 
 

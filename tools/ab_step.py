@@ -1,7 +1,7 @@
 """A/B timing of the captured CIFAR training step under different environment switches, one subprocess per variant
 (the switches are read once per process), interleaved over several rounds so box drift hits every variant equally.
 
-    python tools/ab_step.py "ADM_DGRAD_SHADOW=0" "ADM_DGRAD_SHADOW=1" [--rounds 2] [--steps 30] [--sample]
+    python tools/ab_step.py "ADM_WGRAD_STREAM=0" "ADM_WGRAD_STREAM=1" [--rounds 2] [--steps 30] [--sample]
 """
 import os
 import subprocess

@@ -1,5 +1,5 @@
 """Discriminating micro-benchmarks for the conv / GEMM engine: plain K-major GEMM vs implicit-GEMM conv of the same
-FLOPs, L2-resident vs rotating (cold) operands.  Toggle the CTA-pair path with ADM_GEMM_PAIR=0/1 (read at first use)."""
+FLOPs, L2-resident vs rotating (cold) operands."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -7,7 +7,6 @@ from adm_b200 import ops
 from tools.bench_convs_lib import timeit
 
 N = 128
-print("ADM_GEMM_PAIR =", os.environ.get("ADM_GEMM_PAIR", "(default 1)"))
 for cin, cout, res in [(384, 384, 16), (192, 192, 32), (768, 384, 16), (384, 384, 8), (256, 256, 16), (128, 128, 32)]:
     flops = 2.0 * N * res * res * cin * cout * 9
     w = ops.pack_conv_weight(torch.randn(cout, cin, 3, 3, device="cuda") / 60)

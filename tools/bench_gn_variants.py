@@ -53,8 +53,6 @@ def main():
         for act, dp_ in ((False, 0.0), (True, 0.0), (True, 0.1)):
             t = graph_time(lambda i: ops.gn_apply(xs[i], None, coef, act=act, drop_p=dp_, seed=i), nbuf)
             row.append(f"apply act={int(act)} drop={dp_}: {t:5.1f} us ({mb / t:.2f})")
-        t = graph_time(lambda i: ops.gn_forward(xs[i], None, gamma, beta, g, 1e-5, params=params, act=True, apply=False), nbuf)
-        row.append(f"cluster stats-only {t:5.1f}")
         t = graph_time(lambda i: ops.gn_forward(xs[i], None, gamma, beta, g, 1e-5, params=params, act=True, drop_p=0.0), nbuf)
         row.append(f"cluster fwd nodrop {t:5.1f}")
         t = graph_time(lambda i: ops.gn_forward(xs[i], None, gamma, beta, g, 1e-5, params=params, act=True, drop_p=0.1, seed=i), nbuf)
@@ -64,15 +62,6 @@ def main():
             t = graph_time(lambda i: ops.gn_bwd(dys[i], xs[i], None, cf, gamma, beta, g, params=params, act=True, drop_p=0.1,
                                                 seed=i, dgamma=dg, dbeta=db, dparams=dp, dy_scratch=scratch), nbuf)
             row.append(f"cluster bwd drop scratch={int(scratch)} {t:5.1f}")
-        if ops.conv_gn_ok(hw, hw) and c <= 384:
-            wpk = ops.pack_conv_weight(torch.randn(c, c, 3, 3, device=dev) / (3 * c ** 0.5))
-            bias = torch.zeros(c, device=dev)
-            t = graph_time(lambda i: ops.conv_fprop(xs[i], wpk, bias=bias), nbuf)
-            row.append(f"| conv {c}->{c} plain {t:5.1f}")
-            t = graph_time(lambda i: ops.conv_fprop_gn(xs[i], wpk, cf, bias=bias, act=True, want_act=False), nbuf)
-            row.append(f"+prologue {t:5.1f}")
-            t = graph_time(lambda i: ops.conv_fprop_gn(xs[i], wpk, cf, bias=bias, act=True, drop_p=0.1, seed=i, want_act=True), nbuf)
-            row.append(f"+prologue+drop+write-a {t:5.1f}")
         print("  ".join(row), flush=True)
 
 

@@ -2,7 +2,7 @@
 k-iteration of the first tile of CTA 0.  Needs a library built with -DADM_GEMM_TIMING:
 
     make -C adm_b200/csrc -B NVCCFLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC --expt-relaxed-constexpr -DADM_GEMM_TIMING"
-    ADM_GEMM_PAIR=0 python tools/gemm_thread_timing.py      # single-CTA kernel;  ADM_GEMM_PAIR=1: cta_group::2 kernel
+    python tools/gemm_thread_timing.py
     ADM_GEMM_DEBUG=1|2|3: skip the MMAs / the TMA loads / both (plain tc_gemm_kernel only)
 
 Round-1 result (conv3x3 384->384 @16x16 x128): wait 204 + issue 291 + commit 55 = 550 clocks per k-iteration; with the
