@@ -31,6 +31,17 @@ static inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block
     }
     return cudaLaunchKernelEx(&cfg, kern, args...);
 }
+
+// Raises Kern's dynamic shared-memory limit to `bytes` on the first successful call.  The flag is keyed on the kernel
+// itself, not on its signature: the GEMM engine's kernels all share one parameter list.
+template <auto Kern>
+static inline cudaError_t set_smem_limit_once(int bytes) {
+    static bool done = false;
+    if (done) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    done = e == cudaSuccess;
+    return e;
+}
 #endif
 
 #define ADM_CHECK_LAUNCH(name)                                              \

@@ -15,8 +15,6 @@
 #include "adm_internal.h"
 #include <cuda_bf16.h>
 #include <stdint.h>
-#include <stdlib.h>
-#include <string.h>
 #include <cooperative_groups.h>
 
 #include "vecmath.cuh"
@@ -1245,21 +1243,12 @@ static int grid_for(long long work, int threads, int n_batch) {
 
 
 // Cluster size for the one-cluster-per-sample kernels: the smallest K in {1,2,4,8} with n*K CTAs covering >= 60 % of
-// the SMs; 0 when even K = 8 cannot (small batches use the multi-block kernels).  ADM_GN_PATH=general|fused overrides.
+// the SMs; 0 when even K = 8 cannot (small batches use the multi-block kernels).
 static int gn_cluster_size(int n) {
-    static int forced = -1;
-    if (forced < 0) {
-        const char* e = getenv("ADM_GN_PATH");
-        forced = e == nullptr ? 0 : (strcmp(e, "general") == 0 ? 1 : (strcmp(e, "fused") == 0 ? 2 : 0));
-    }
-    if (forced == 1) return 0;
     const int want = (num_sms() * 6 + 9) / 10;
     int k = 1;
     while (k < 8 && n * k < want) k *= 2;
-    static int mult = -1;  // experiments: ADM_GN_KMULT=2|4 splits every sample over that many more CTAs
-    if (mult < 0) { const char* e = getenv("ADM_GN_KMULT"); mult = e ? atoi(e) : 1; if (mult < 1) mult = 1; }
-    if (n * k >= want) for (int m = mult; m > 1 && k < 8; m >>= 1) k *= 2;
-    return (n * k >= want || forced == 2) ? k : 0;
+    return n * k >= want ? k : 0;
 }
 
 static int gn_fused_threads(int V, int hw, int k) {
@@ -1270,28 +1259,9 @@ static int gn_fused_threads(int V, int hw, int k) {
     return tpv * V;
 }
 
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_cluster(void (*kern)(KArgs...), int grid, int block, size_t smem, int k, cudaStream_t s,
-                                  Args... args) {
-    static bool attr_set = false;  // per kernel instantiation
-    if (!attr_set) {
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        attr_set = true;
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(block);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = k;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kern, args...);
-}
+// Dynamic shared-memory limit of the two cluster kernels: covers their largest launch (gn_bwd_fused_kernel at C = 2048
+// with 512 threads, 184 KB).
+constexpr int GNF_SMEM_LIMIT = 200 * 1024;
 
 }  // namespace adm
 
@@ -1375,10 +1345,12 @@ int adm_gn_forward(const void* x1, int c1, long long ld1, const void* x2, int c2
     const int V = C / 8;
     const int threads = gn_fused_threads(V, h * w, k);
     const size_t smem = sizeof(float) * (6 * C + 16 * threads);  // ring (4 x 16 B per thread) aliases the scratch
-    cudaError_t e = launch_cluster(gn_fwd_fused_kernel, n * k, threads, smem, k, static_cast<cudaStream_t>(stream),
-                                   static_cast<const bf16*>(x1), c1, ld1, static_cast<const bf16*>(x2), c2, ld2, h, w,
-                                   groups, eps, gamma, beta, params, ld_params, reinterpret_cast<float4*>(coef), act,
-                                   drop_p, seed, resample, static_cast<bf16*>(out), ldo, g_seed_dev);
+    cudaError_t e = set_smem_limit_once<gn_fwd_fused_kernel>(GNF_SMEM_LIMIT);
+    if (e == cudaSuccess)
+        e = launch_k(gn_fwd_fused_kernel, dim3(n * k), dim3(threads), smem, static_cast<cudaStream_t>(stream), k,
+                     static_cast<const bf16*>(x1), c1, ld1, static_cast<const bf16*>(x2), c2, ld2, h, w, groups, eps, gamma,
+                     beta, params, ld_params, reinterpret_cast<float4*>(coef), act, drop_p, seed, resample,
+                     static_cast<bf16*>(out), ldo, g_seed_dev);
     if (e != cudaSuccess) {
         set_error("gn_forward launch: %s", cudaGetErrorString(e));
         return ADM_ERR_CUDA;
@@ -1408,11 +1380,13 @@ int adm_gn_bwd(const void* dy, long long ldy, const void* x1, int c1, long long 
     if (kc > 0) {
         const int threads = gn_fused_threads(C / 8, h * w, kc);
         const size_t smem = sizeof(float) * (7 * C + 16 * threads) + 16 * GNF_STAGES * 3 * threads;
-        cudaError_t e = launch_cluster(
-            gn_bwd_fused_kernel, n * kc, threads, smem, kc, s, dyp, ldy, x1p, c1, ld1, x2p, c2, ld2, h, w, groups,
-            reinterpret_cast<const float4*>(coef), gamma, beta, params, ld_params, act, drop_p, seed, resample, dgamma,
-            dbeta, dparams, ld_dparams, static_cast<const bf16*>(add), ldadd, add_mode, static_cast<bf16*>(dx1), ldx1,
-            static_cast<bf16*>(dx2), ldx2, dbias1, dbias1b, g_seed_dev, dy_scratch);
+        cudaError_t e = set_smem_limit_once<gn_bwd_fused_kernel>(GNF_SMEM_LIMIT);
+        if (e == cudaSuccess)
+            e = launch_k(gn_bwd_fused_kernel, dim3(n * kc), dim3(threads), smem, s, kc, dyp, ldy, x1p, c1, ld1, x2p, c2, ld2,
+                         h, w, groups, reinterpret_cast<const float4*>(coef), gamma, beta, params, ld_params, act, drop_p,
+                         seed, resample, dgamma, dbeta, dparams, ld_dparams, static_cast<const bf16*>(add), ldadd, add_mode,
+                         static_cast<bf16*>(dx1), ldx1, static_cast<bf16*>(dx2), ldx2, dbias1, dbias1b, g_seed_dev,
+                         dy_scratch);
         if (e != cudaSuccess) {
             set_error("gn_bwd (fused) launch: %s", cudaGetErrorString(e));
             return ADM_ERR_CUDA;

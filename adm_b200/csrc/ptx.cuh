@@ -28,16 +28,6 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 }
 __device__ __forceinline__ uint32_t mbar_try_wait(uint64_t* bar, uint32_t parity) {
     uint32_t ok;
-#ifdef ADM_MBAR_TEST_WAIT
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok;
-#endif
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"

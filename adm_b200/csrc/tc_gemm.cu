@@ -81,90 +81,24 @@ static int encode_map(CUtensorMap* m, const void* ptr, int rank, const long long
     return 0;
 }
 
-template <int MODE>
-static int launch(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const GemmParams& p,
-                  cudaStream_t stream) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(tc_gemm_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             GEMM_SMEM_TOTAL);
-        if (e != cudaSuccess) {
-            set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            return ADM_ERR_CUDA;
-        }
-        attr_set = true;
-    }
+// Launches a GEMM-engine kernel over the tiles of p: GEMM_THREADS threads and GEMM_SMEM_TOTAL bytes of shared memory
+// per CTA.  Without a cluster the kernel is persistent: min(tiles, SMs) CTAs stride over the tiles.  With one (the
+// split-K conv) every tile gets its own cluster of `cluster` CTAs.
+template <auto Kern>
+static int launch_gemm(const char* name, int cluster, const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b,
+                       const GemmParams& p, cudaStream_t stream) {
     const long long tiles = 1LL * p.batches * p.splits * p.m_tiles * p.n_tiles;
     if (tiles <= 0 || tiles > INT_MAX) {
-        set_error("gemm: bad tile count %lld", tiles);
+        set_error("%s: bad tile count %lld", name, tiles);
         return ADM_ERR_SHAPE;
     }
-    const int grid = static_cast<int>(tiles < num_sms() ? tiles : num_sms());
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("ADM_GEMM_DEBUG"); dbg = e ? atoi(e) : 0; }
-    GemmParams pd = p;
-    pd.debug = dbg;
-    cudaError_t e = launch_k(tc_gemm_kernel<MODE>, dim3(grid), dim3(GEMM_THREADS), GEMM_SMEM_TOTAL, stream, 0, a, a2, b, pd);
+    const long long grid = cluster > 0 ? tiles * cluster : (tiles < num_sms() ? tiles : num_sms());
+    cudaError_t e = set_smem_limit_once<Kern>(GEMM_SMEM_TOTAL);
+    if (e == cudaSuccess)
+        e = launch_k(Kern, dim3(static_cast<unsigned>(grid)), dim3(GEMM_THREADS), GEMM_SMEM_TOTAL, stream, cluster, a, a2, b, p);
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess) {
-        set_error("tc_gemm launch: %s", cudaGetErrorString(e));
-        return ADM_ERR_CUDA;
-    }
-    count_launch();
-    return 0;
-}
-
-// Halo conv launch (tc_conv_halo_kernel): plain persistent grid.
-static int launch_halo(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const GemmParams& p,
-                       cudaStream_t stream) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(tc_conv_halo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             GEMM_SMEM_TOTAL);
-        if (e != cudaSuccess) {
-            set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            return ADM_ERR_CUDA;
-        }
-        attr_set = true;
-    }
-    const long long tiles = 1LL * p.m_tiles * p.n_tiles;
-    if (tiles <= 0 || tiles > INT_MAX) {
-        set_error("conv: bad tile count %lld", tiles);
-        return ADM_ERR_SHAPE;
-    }
-    const int grid = static_cast<int>(tiles < num_sms() ? tiles : num_sms());
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("ADM_GEMM_DEBUG"); dbg = e ? atoi(e) : 0; }
-    GemmParams pd = p;
-    pd.debug = dbg;
-    cudaError_t e = launch_k(tc_conv_halo_kernel, dim3(grid), dim3(GEMM_THREADS), GEMM_SMEM_TOTAL, stream, 0, a, a2, b, pd);
-    if (e == cudaSuccess) e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        set_error("tc_conv_halo launch: %s", cudaGetErrorString(e));
-        return ADM_ERR_CUDA;
-    }
-    count_launch();
-    return 0;
-}
-
-// Cluster split-K conv launch (tc_conv_splitk_kernel): one tile per CTA, clusters of p.ksplit CTAs along K.
-static int launch_splitk(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const GemmParams& p,
-                         cudaStream_t stream) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(tc_conv_splitk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             GEMM_SMEM_TOTAL);
-        if (e != cudaSuccess) {
-            set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            return ADM_ERR_CUDA;
-        }
-        attr_set = true;
-    }
-    const int grid = p.m_tiles * p.n_tiles * p.ksplit;
-    cudaError_t e = launch_k(tc_conv_splitk_kernel, dim3(grid), dim3(GEMM_THREADS), GEMM_SMEM_TOTAL, stream, p.ksplit, a, a2, b, p);
-    if (e == cudaSuccess) e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        set_error("tc_conv_splitk launch: %s", cudaGetErrorString(e));
+        set_error("%s launch: %s", name, cudaGetErrorString(e));
         return ADM_ERR_CUDA;
     }
     count_launch();
@@ -173,13 +107,11 @@ static int launch_splitk(const CUtensorMap& a, const CUtensorMap& a2, const CUte
 
 // Under-filled convs (few pixel tiles, long K): pick (N tile, K split) minimising the critical path
 // ceil(k_total / ks) x (128 + bn) operand rows + reduction, subject to tiles x ks <= SMs.  Returns ks (1 = plain kernel).
-// ADM_CONV_SPLITK=0 disables (A/B timing).
 static int pick_splitk(int n, int multiple, int m_tiles, int k_total, int* bn_out) {
-    static int on = -1;
-    if (on < 0) { const char* e = getenv("ADM_CONV_SPLITK"); on = (e != nullptr && e[0] == '0') ? 0 : 1; }
-    if (!on) return 1;
     const int n_pad = (n + multiple - 1) / multiple * multiple;
-    if (const char* f = getenv("ADM_SPLITK_FORCE")) {  // tests: "bn,ks" forces a tile width and split (read per call)
+    // Test hook, read per call: ADM_SPLITK_FORCE="bn,ks" forces a tile width and split when they fit the problem, so the
+    // tests can cover (bn, ks) pairs of the split-K kernel that the cost model below does not pick.
+    if (const char* f = getenv("ADM_SPLITK_FORCE")) {
         int fb = 0, fk = 0;
         if (sscanf(f, "%d,%d", &fb, &fk) == 2 && fb >= multiple && fb % multiple == 0 && n_pad % fb == 0 && fk >= 1 && fk <= 8 &&
             m_tiles * (n_pad / fb) * fk <= num_sms() && (fk - 1) * ((k_total + fk - 1) / fk) < k_total) {
@@ -205,44 +137,6 @@ static int pick_splitk(int n, int multiple, int m_tiles, int k_total, int* bn_ou
     return best_ks;
 }
 
-static int launch_wgrad_rows(const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& b2, const GemmParams& p,
-                             cudaStream_t stream) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(tc_wgrad_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             GEMM_SMEM_TOTAL);
-        if (e != cudaSuccess) {
-            set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            return ADM_ERR_CUDA;
-        }
-        attr_set = true;
-    }
-    const long long tiles = 1LL * p.splits * p.m_tiles * p.n_tiles;
-    if (tiles <= 0 || tiles > INT_MAX) {
-        set_error("wgrad: bad tile count %lld", tiles);
-        return ADM_ERR_SHAPE;
-    }
-    const int grid = static_cast<int>(tiles < num_sms() ? tiles : num_sms());
-    cudaError_t e = launch_k(tc_wgrad_rows_kernel, dim3(grid), dim3(GEMM_THREADS), GEMM_SMEM_TOTAL, stream, 0, a, b, b2, p);
-    if (e == cudaSuccess) e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        set_error("tc_wgrad_rows launch: %s", cudaGetErrorString(e));
-        return ADM_ERR_CUDA;
-    }
-    count_launch();
-    return 0;
-}
-
-// ADM_WGRAD_ROWS=0 falls back to the per-tap wgrad tiles (experiments / A-B timing).
-static bool wgrad_rows_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("ADM_WGRAD_ROWS");
-        v = (e != nullptr && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
 // split K (pixels) for the wgrad kernels: the split that minimises waves x (k-iterations per tile + epilogue cost) on
 // the persistent grid — fewer, fuller waves beat "more tiles" (wave quantisation), fewer splits mean fewer atomics.
 static void pick_wgrad_split(GemmParams* p, int base_tiles, int epi) {
@@ -256,24 +150,12 @@ static void pick_wgrad_split(GemmParams* p, int base_tiles, int epi) {
         const long long cost = waves * (k_per + epi);
         if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_s = s_eff; }
     }
-    if (const char* e = getenv("ADM_WGRAD_SPLITS")) {  // experiments: force the split count
-        const int s = atoi(e);
-        if (s >= 1 && s <= p->k_total) best_s = s;
-    }
     p->k_iters = (p->k_total + best_s - 1) / best_s;
     p->splits = (p->k_total + p->k_iters - 1) / p->k_iters;
 }
 
 // The halo kernel serves 3x3 convs whose images tile into 8 x 16 pixel boxes (the 32x32 and 16x16 levels).
-// ADM_CONV_HALO=0 falls back to the per-tap loads (experiments / A-B timing).
-static bool halo_ok(int ntaps, int h, int w) {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("ADM_CONV_HALO");
-        v = (e != nullptr && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1 && ntaps == 9 && w % 8 == 0 && h % 16 == 0;
-}
+static bool halo_ok(int ntaps, int h, int w) { return ntaps == 9 && w % 8 == 0 && h % 16 == 0; }
 
 // Largest multiple of 16 that is <= cap and divides ceil16(n); falls back to the smallest cover.
 static int pick_bn(int n, int cap, int multiple) {
@@ -289,10 +171,6 @@ static int pick_bn(int n, int cap, int multiple) {
 // when there are too few pixel tiles to fill the SMs (4x4 / 8x8 levels), where narrower tiles cut the critical path.
 static int pick_bn_cost(int n, int multiple, int m_tiles, int k_total) {
     const int n_pad = (n + multiple - 1) / multiple * multiple;
-    if (const char* e = getenv("ADM_BN")) {  // experiments: force the N tile when it is legal for this problem
-        const int bn = atoi(e);
-        if (bn >= multiple && bn <= 256 && bn % multiple == 0 && n_pad % bn == 0) return bn;
-    }
     const int sms = num_sms();
     long long best = -1;
     int best_bn = multiple;
@@ -392,9 +270,10 @@ int adm_conv_fprop(const void* x1, int c1, long long ld1, const void* x2, int c2
     const long long bs[1] = {kpad};
     const int bb[2] = {64, p.bn};
     if (int e = encode_map(&mb, wpk, 2, bd, bs, bb)) return e;
-    if (halo) return launch_halo(ma, ma2, mb, p, static_cast<cudaStream_t>(stream));
-    if (p.ksplit > 1) return launch_splitk(ma, ma2, mb, p, static_cast<cudaStream_t>(stream));
-    return launch<GEMM_CONV>(ma, ma2, mb, p, static_cast<cudaStream_t>(stream));
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (halo) return launch_gemm<tc_conv_halo_kernel>("tc_conv_halo", 0, ma, ma2, mb, p, s);
+    if (p.ksplit > 1) return launch_gemm<tc_conv_splitk_kernel>("tc_conv_splitk", p.ksplit, ma, ma2, mb, p, s);
+    return launch_gemm<tc_gemm_kernel<GEMM_CONV>>("tc_gemm", 0, ma, ma2, mb, p, s);
 }
 
 int adm_conv_dgrad(const void* dy, int cout, long long ld_dy, int n, int h, int w, const void* wpk, int kpad,
@@ -432,9 +311,10 @@ int adm_conv_dgrad(const void* dy, int cout, long long ld_dy, int n, int h, int 
     const long long bs[2] = {kpad, 1LL * kpad * ntaps};
     const int bb[3] = {64, 1, 64};
     if (int e = encode_map(&mb, wpk, 3, bd, bs, bb)) return e;
-    if (halo) return launch_halo(ma, ma, mb, p, static_cast<cudaStream_t>(stream));
-    if (p.ksplit > 1) return launch_splitk(ma, ma, mb, p, static_cast<cudaStream_t>(stream));
-    return launch<GEMM_CONV>(ma, ma, mb, p, static_cast<cudaStream_t>(stream));
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (halo) return launch_gemm<tc_conv_halo_kernel>("tc_conv_halo", 0, ma, ma, mb, p, s);
+    if (p.ksplit > 1) return launch_gemm<tc_conv_splitk_kernel>("tc_conv_splitk", p.ksplit, ma, ma, mb, p, s);
+    return launch_gemm<tc_gemm_kernel<GEMM_CONV>>("tc_gemm", 0, ma, ma, mb, p, s);
 }
 
 int adm_conv_wgrad(const void* dy, int cout, long long ld_dy, const void* x1, int c1, long long ld1, const void* x2,
@@ -458,7 +338,7 @@ int adm_conv_wgrad_mapped(const void* dy, int cout, long long ld_dy, const void*
     p.k_total = p.tiles_w * p.tiles_h * ((n + p.bni - 1) / p.bni);
     const int kpad = pad64(c1) + (x2 ? pad64(c2) : 0);
     p.M = cout; p.N = kpad;
-    if (ntaps == 9 && wgrad_rows_enabled() && p.bni == 1 && (p.bw == 8 || p.bw % 16 == 0)) {
+    if (ntaps == 9 && p.bni == 1 && (p.bw == 8 || p.bw % 16 == 0)) {
         // tap-row kernel: M chunks = (dy, 64-channel dY chunk), N = the three dx taps of one 64-channel X chunk
         p.co_chunks = pad64(cout) / 64;
         p.m_tiles = (3 * p.co_chunks + 1) / 2;
@@ -474,7 +354,7 @@ int adm_conv_wgrad_mapped(const void* dy, int cout, long long ld_dy, const void*
         if (int e = nhwc_map(&ma, dy, cout, ld_dy, n, h, w, p.bw, p.bh, 1)) return e;
         if (int e = nhwc_map(&mb, x1, c1, ld1, n, h, w, p.bw + 2, p.bh, 1)) return e;
         if (x2) { if (int e = nhwc_map(&mb2, x2, c2, ld2, n, h, w, p.bw + 2, p.bh, 1)) return e; } else mb2 = mb;
-        return launch_wgrad_rows(ma, mb, mb2, p, static_cast<cudaStream_t>(stream));
+        return launch_gemm<tc_wgrad_rows_kernel>("tc_wgrad_rows", 0, ma, mb, mb2, p, static_cast<cudaStream_t>(stream));
     }
     p.m_tiles = (cout + 127) / 128;
     p.bn = x2 ? pick_bn(pad64(c1), 256, 64) : pick_bn(kpad, 256, 64);
@@ -492,7 +372,7 @@ int adm_conv_wgrad_mapped(const void* dy, int cout, long long ld_dy, const void*
     if (int e = nhwc_map(&ma, dy, cout, ld_dy, n, h, w, p.bw, p.bh, p.bni)) return e;
     if (int e = nhwc_map(&mb, x1, c1, ld1, n, h, w, p.bw, p.bh, p.bni)) return e;
     if (x2) { if (int e = nhwc_map(&mb2, x2, c2, ld2, n, h, w, p.bw, p.bh, p.bni)) return e; } else mb2 = mb;
-    return launch<GEMM_WGRAD>(ma, mb2, mb, p, static_cast<cudaStream_t>(stream));
+    return launch_gemm<tc_gemm_kernel<GEMM_WGRAD>>("tc_gemm", 0, ma, mb2, mb, p, static_cast<cudaStream_t>(stream));
 }
 
 int adm_device_error(void) {
@@ -535,7 +415,7 @@ int adm_gemm_batched(const adm_gemm_desc* d, void* stream) {
         const int box[3] = {64, d->b.mn_major ? 64 : p.bn, 1};
         if (int e = encode_map(&mb, d->b.ptr, 3, dims, str, box)) return e;
     }
-    return launch<GEMM_PLAIN>(ma, ma, mb, p, static_cast<cudaStream_t>(stream));
+    return launch_gemm<tc_gemm_kernel<GEMM_PLAIN>>("tc_gemm", 0, ma, ma, mb, p, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

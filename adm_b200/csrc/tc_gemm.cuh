@@ -11,9 +11,6 @@
 #pragma once
 #include "ptx.cuh"
 #include "adm_internal.h"
-#ifdef ADM_GEMM_TIMING
-#include <stdio.h>
-#endif
 
 namespace adm {
 
@@ -66,7 +63,6 @@ struct GemmParams {
     float alpha;
     int out_mode;
     const int* row_map;  // plain / wgrad tiles: GEMM row r is stored at output row row_map[r] (nullptr = identity)
-    int debug;  // experiments only (ADM_GEMM_DEBUG): bit 0 = skip the MMAs, bit 1 = skip the TMA loads
 };
 
 __device__ __forceinline__ void decode_pix(const GemmParams& p, int idx, int& n0, int& h0, int& w0) {
@@ -335,11 +331,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     mbar_wait(&empty_bar[stage], phase ^ 1, 1);
                     uint8_t* sa = smem + stage * stage_bytes;
                     uint8_t* sb = sa + GEMM_A_STAGE;
-                    if (p.debug & 2) {
-                        mbar_arrive(&full_bar[stage]);
-                        if (++stage == num_stages) { stage = 0; phase ^= 1; }
-                        continue;
-                    }
                     mbar_expect_tx(&full_bar[stage], stage_bytes);
                     if (MODE == GEMM_CONV) {
                         int dh = 0, dw = 0;
@@ -419,39 +410,17 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 mbar_wait(&tempty_bar[acc], acc_phase ^ 1, 2);
                 tc_fence_after();
                 const uint32_t tmem_d = tmem_base + acc * 256;
-#ifdef ADM_GEMM_TIMING
-                long long t_wait = 0, t_issue = 0, t_commit = 0;
-#endif
                 for (int ki = k_begin; ki < k_end; ++ki) {
-#ifdef ADM_GEMM_TIMING
-                    const long long c0 = clock64();
-#endif
                     mbar_wait(&full_bar[stage], phase, 3);
                     tc_fence_after();
-#ifdef ADM_GEMM_TIMING
-                    const long long c1 = clock64();
-#endif
                     const uint32_t sa16 = (smem_u32(smem + stage * stage_bytes) & 0x3FFFFu) >> 4;
                     const uint64_t da = da0 + sa16, db = db0 + (sa16 + (GEMM_A_STAGE >> 4));
 #pragma unroll
                     for (int k = 0; k < GEMM_BLOCK_K / 16; ++k)
-                        if (!(p.debug & 1))
-                            umma_bf16(tmem_d, da + k * a_kstep, db + k * b_kstep, idesc, (ki > k_begin || k > 0) ? 1u : 0u);
-#ifdef ADM_GEMM_TIMING
-                    const long long c2 = clock64();
-#endif
+                        umma_bf16(tmem_d, da + k * a_kstep, db + k * b_kstep, idesc, (ki > k_begin || k > 0) ? 1u : 0u);
                     umma_commit(&empty_bar[stage]);
-#ifdef ADM_GEMM_TIMING
-                    const long long c3 = clock64();
-                    t_wait += c1 - c0; t_issue += c2 - c1; t_commit += c3 - c2;
-#endif
                     if (++stage == num_stages) { stage = 0; phase ^= 1; }
                 }
-#ifdef ADM_GEMM_TIMING
-                if (blockIdx.x == 0 && tile == blockIdx.x)
-                    printf("[mma thread] k-iters %d: wait %lld issue %lld commit %lld clocks per k-iter\n", k_end - k_begin,
-                           t_wait / (k_end - k_begin), t_issue / (k_end - k_begin), t_commit / (k_end - k_begin));
-#endif
                 umma_commit(&tfull_bar[acc]);
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
@@ -769,11 +738,6 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                     for (int tap = 0; tap < 9; ++tap) {
                         mbar_wait(&bempty[bs], bphase ^ 1, 1);
                         uint8_t* sb = b_ring + bs * b_bytes;
-                        if (p.debug & 2) {  // ADM_GEMM_DEBUG=2 (timing experiment, results are garbage): no weight traffic
-                            mbar_arrive(&bfull[bs]);
-                            if (++bs == nb) { bs = 0; bphase ^= 1; }
-                            continue;
-                        }
                         mbar_expect_tx(&bfull[bs], b_bytes);
                         if (!p.b_mn) {
                             tma_load_2d(sb, &tmB, &bfull[bs], (tap * p.cchunks + kc) * 64, nt * p.bn);

@@ -18,7 +18,6 @@ ddm_const.py:179-180) raise.
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 import torch.nn.functional as F
@@ -66,7 +65,7 @@ class AugmentPipe:
         self.aniso_rotate_prob, self.translate_frac_std = float(aniso_rotate_prob), float(translate_frac_std)
         # CUDA batches run flips + warp as ONE kernel (adm_augment_warp); fused = False keeps the torch-op sequence below
         # (the same arithmetic, ~40 launches), which is also what runs on CPU tensors
-        self.fused = os.environ.get("ADM_AUG_FUSED", "1") != "0"  # 0: A/B timing of the torch-op sequence
+        self.fused = True
 
     # ------------------------------------------------------------------------------------------ random parameters
     def draw(self, n, h, w, device):

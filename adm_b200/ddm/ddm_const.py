@@ -18,7 +18,6 @@ Deviations from the reference, all documented in DESIGN.md:
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 import torch.nn as nn
@@ -441,7 +440,7 @@ class LatentDiffusion(DDPM):
         """ddm_const.py:868-888: x' = x + (t'-t) * (C + eps / (sqrt(t) + sqrt(t'))) == x0 + C t' + sqrt(t') eps with
         x0 = x - C t - sqrt(t) eps and no clamp — K3 with do_clip = 0.  On CUDA the whole N-step loop (N UNet forwards,
         conditional or not, + N fused updates) is captured once per (shape, N, condition shape) into a CUDA graph and
-        replayed with the start noise and the condition copied into its static inputs (``ADM_SAMPLE_GRAPH=0``: eager)."""
+        replayed with the start noise and the condition copied into its static inputs (``use_graph=False``: eager)."""
         device = self.eps.device
         ts = self.t_steps()
         if x_T is None:
@@ -449,7 +448,7 @@ class LatentDiffusion(DDPM):
         x_T = x_T.to(device=device, dtype=torch.float64)
         if use_graph is None:
             use_graph = (x_T.is_cuda and not torch.cuda.is_current_stream_capturing()
-                         and os.environ.get("ADM_SAMPLE_GRAPH", "1") != "0" and not self.__dict__.get("_latent_graph_off"))
+                         and not self.__dict__.get("_latent_graph_off"))
         was_training = self.model.training
         self.model.eval()
         try:

@@ -9,7 +9,6 @@ ranks of per-rank gradients, reduced once per optimizer step (not per micro-batc
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 import torch.distributed as dist
@@ -194,9 +193,8 @@ class TrainStep:
                             for _ in range(4)]
         self._hyper_events = [None] * 4
         self._ring_i = 0
-        # gradient buckets in completion order (ADM_BUCKET_MB overrides the size: A/B timing of the data-parallel step)
+        # gradient buckets in completion order
         n = self.arena.numel
-        bucket_mb = int(os.environ.get("ADM_BUCKET_MB", bucket_mb))
         per = max(1, bucket_mb * (1 << 20) // 4)
         self.buckets = [(s, min(n, s + per)) for s in range(0, n, per)]
         self.comm_stream = torch.cuda.Stream(device=dev) if (self.world > 1 and dev.type == "cuda") else None

@@ -19,7 +19,6 @@ There is no CPU fallback: the kernels raise on non-CUDA tensors.
 from __future__ import annotations
 
 import math
-import os
 from functools import partial
 
 import torch
@@ -177,7 +176,8 @@ class BasicAttetnionLayer(nn.Module):
         as one fused pass (``AF.relation_tail``): the 1x1 ``out_conv`` commutes with the bilinear resize (per-pixel
         linear map, resize weights sum to one), so it runs on the pooled tokens and the resize + residual GroupNorm is a
         single read of x2 / conv and a single bf16 write with the sum in fp32 registers.  The window-pooled cross
-        attention itself (a few hundred tokens) stays torch ops.  ``ADM_REL_FUSED=0`` keeps the unfused path."""
+        attention itself (a few hundred tokens) stays torch ops.  With ``_REL_FUSED = False`` every layer runs the unfused
+        tail (fp32 residual add + GroupNorm, bilinear resize, full-resolution out_conv) as torch ops."""
         b, _, _, c1 = x1.shape
         _, h2, w2, c2 = x2.shape
         gn = self.gn
@@ -189,15 +189,12 @@ class BasicAttetnionLayer(nn.Module):
         y = _conv1x1(torch.cat([up.to(torch.bfloat16), x2], dim=-1), self.concat_conv)
         if fused:
             shortcut = None
-        elif os.environ.get("ADM_REL_GN", "torch") == "torch":
+        else:
             # fp32 GroupNorm on the channels-last view: the residual stream of the relation layer stays fp32 end to end, as
-            # under the reference's fp32 arithmetic (with the bf16 kernel here one Downsample weight gradient of the golden
-            # check drops from cosine 0.9995 to 0.9983)
+            # under the reference's fp32 arithmetic (with the bf16 GroupNorm kernel one Downsample weight gradient of the
+            # golden check drops from cosine 0.9995 to 0.9983)
             pre = x2r + y.float()
             shortcut = F.group_norm(_nchw(pre), gn.num_groups, gn.weight, gn.bias, gn.eps).permute(0, 2, 3, 1)
-        else:
-            pre = x2r + y.float()
-            shortcut = AF.group_norm_act(pre.to(torch.bfloat16), gn.weight, gn.bias, gn.num_groups, gn.eps, act=False)
         pooled = _window_pool(x1, self.window_size1, self.avgpool_q)  # [b, hq, wq, c]
         hq, wq = pooled.shape[1:3]
         q = (pooled + self.pos_enc(pooled).to(pooled.dtype)).reshape(b, -1, c2)
@@ -220,7 +217,7 @@ class BasicAttetnionLayer(nn.Module):
         return shortcut.float() + _conv1x1(pooled, self.out_conv).float()  # fp32 (rounded once, by RelationNet.forward)
 
 
-_REL_FUSED = os.environ.get("ADM_REL_FUSED", "1") != "0"
+_REL_FUSED = True
 
 
 def _window_pool(x, window, pool):

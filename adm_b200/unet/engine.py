@@ -16,7 +16,6 @@ role of autograd's AccumulateGrad for its own parameters.
 from __future__ import annotations
 
 import contextlib
-import os
 from types import SimpleNamespace as NS
 
 import torch
@@ -55,9 +54,7 @@ class UNetEngine:
         # Weight / bias gradients of the convs run on a side stream, concurrently with the data-gradient chain: a wgrad
         # only feeds the optimizer, and every GEMM is a persistent kernel whose last partial wave leaves SMs idle (and
         # the 4x4 / 8x8 levels never fill 148 SMs) — the other stream's CTAs take those SMs.  Joined at every _notify.
-        # ADM_WGRAD_STREAM=0 keeps everything on one stream.
         self._side = None
-        self._side_on = os.environ.get("ADM_WGRAD_STREAM", "1") != "0"
         self._side_pending = []
         # device-resident step counter mixed into every dropout seed (fresh masks per CUDA-graph replay); owned by the
         # training step (adm_b200.train.TrainStep) and passed to the GroupNorm kernels per call
@@ -245,7 +242,7 @@ class UNetEngine:
             bias = None
         else:
             bias = conv.bias
-        if self._side_on and dy.is_cuda:
+        if dy.is_cuda:
             with torch.cuda.stream(self._fork_side(dy, x1, x2, dy_cols)):
                 self._conv_weight_grad(conv, dy, x1, x2, perm)
                 if bias is not None:
@@ -620,7 +617,7 @@ class UNetEngine:
         # side stream, forked HERE (before decoder 1 is enqueued), so their kernels interleave on the SMs — most of
         # them leave a partial last wave, the 4x4 / 8x8 levels never fill the GPU.  Host order (and the tape) unchanged.
         fork = None
-        if self._side_on and x.is_cuda:
+        if x.is_cuda:
             if self._side is None:
                 self._side = torch.cuda.Stream()
             fork = torch.cuda.Event()

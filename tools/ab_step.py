@@ -1,7 +1,8 @@
-"""A/B timing of the captured CIFAR training step under different environment switches, one subprocess per variant
-(the switches are read once per process), interleaved over several rounds so box drift hits every variant equally.
+"""A/B timing of the captured CIFAR training step under different environments, one subprocess per variant, interleaved
+over several rounds so box drift hits every variant equally.  Two builds of the library are compared through
+ADM_B200_LIB (the Python package is this tree's in both; "" is the in-tree build):
 
-    python tools/ab_step.py "ADM_WGRAD_STREAM=0" "ADM_WGRAD_STREAM=1" [--rounds 2] [--steps 30] [--sample]
+    python tools/ab_step.py "ADM_B200_LIB=/path/to/other/adm_b200/libadm_b200.so" "" [--rounds 2] [--steps 30] [--sample]
 """
 import os
 import subprocess
