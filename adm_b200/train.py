@@ -5,6 +5,9 @@ Mirrors the step body of the reference Trainer (/root/reference/train_uncond_dpm
 ``clip_grad_norm_(1.0)`` (:292), AdamW(lr, weight_decay=1e-4) (:179-180), warm-up + polynomial LambdaLR (:169-182).
 Semantics we define explicitly (the reference's DDP wiring is accidental, SURVEY §2): gradients are the MEAN over
 ranks of per-rank gradients, reduced once per optimizer step (not per micro-batch).
+
+``AutogradDataParallel`` gives the same semantics to a model that trains through torch autograd and a torch optimizer
+(the conditional UNet of scripts/train_cond_ldm.py): one flat gradient arena, one all-reduce per optimizer step.
 """
 from __future__ import annotations
 
@@ -155,6 +158,102 @@ class ParamArena:
     def zero_grad(self):
         self.grads.zero_()
 
+    def broadcast(self, src=0, group=None, extra=()):
+        """Rank `src`'s parameter arena, then each tensor of `extra` (in place), to every rank of `group`."""
+        for t in (self.flat, *extra):
+            dist.broadcast(t, src=src, group=group)
+
+
+class AutogradDataParallel:
+    """Data parallelism for a model that trains through torch autograd and a torch optimizer (the conditional UNet),
+    where TrainStep's engine-driven reduction does not apply.
+
+    The trainable parameters are re-homed into a ParamArena, so every ``.grad`` is a view of ONE flat fp32 buffer that
+    autograd accumulates into.  The step is: ``zero_grad()``, forward + backward of every micro-batch, ``all_reduce()``
+    once after the last one (one collective over the whole buffer), ``clip_mean_()``, optimizer step.  The gradient is
+    the mean over ranks (DESIGN.md §1); the 1/world factor is folded into the clipping pass.  Gradients must be zeroed
+    through ``zero_grad()``: setting ``.grad`` to None would detach it from the buffer."""
+
+    def __init__(self, module, params, process_group=None):
+        """module: the whole model (its parameters outside `params` and its buffers are replicated too);
+        params: the trainable parameters."""
+        self.module, self.pg = module, process_group
+        self.world = dist.get_world_size(process_group) if (dist.is_available() and dist.is_initialized()) else 1
+        self.arena = ParamArena(module, order=list(params))
+        self.sync()
+
+    @torch.no_grad()
+    def sync(self, src=0):
+        """Rank `src`'s weights to every rank: the trainable arena, the frozen parameters and every buffer.  Called at
+        construction (replicas may start from different seeds) and after a checkpoint load on rank `src`."""
+        if self.world == 1:
+            return
+        homed = {id(p) for p in self.arena.params}
+        rest = [t.data for t in (*self.module.parameters(), *self.module.buffers()) if id(t) not in homed]
+        self.arena.broadcast(src, self.pg, rest)
+
+    def broadcast_object(self, obj, src=0):
+        """A picklable value of rank `src` on every rank."""
+        if self.world == 1:
+            return obj
+        box = [obj]
+        dist.broadcast_object_list(box, src=src, group=self.pg)
+        return box[0]
+
+    @torch.no_grad()
+    def sync_optimizer(self, opt, src=0):
+        """Rank `src`'s torch.optim state to every rank: the hyperparameters of each parameter group except the
+        learning rate (the trainer sets that every step) and the per-parameter state, allocated with rank `src`'s
+        shapes, dtypes and devices on the ranks that have none (a fresh optimizer before its first step)."""
+        if self.world == 1:
+            return
+        params = [p for g in opt.param_groups for p in g["params"]]
+        meta = None
+        if dist.get_rank(self.pg) == src:
+            groups = [{k: v for k, v in g.items() if k not in ("params", "lr")} for g in opt.param_groups]
+            state = []
+            for p in params:
+                st = opt.state.get(p, {})
+                state.append(({k: (tuple(v.shape), v.dtype, v.device == p.device) for k, v in st.items()
+                               if torch.is_tensor(v)},
+                              {k: v for k, v in st.items() if not torch.is_tensor(v)}))
+            meta = (groups, state)
+        groups, state = self.broadcast_object(meta, src)
+        for g, hyper in zip(opt.param_groups, groups):
+            g.update(hyper)
+        for p, (tensors, values) in zip(params, state):
+            if not tensors and not values:
+                continue
+            st = opt.state[p]
+            st.update(values)
+            for k, (shape, dtype, on_param) in tensors.items():
+                t = st.get(k)
+                if not torch.is_tensor(t) or tuple(t.shape) != shape or t.dtype != dtype:
+                    t = st[k] = torch.empty(shape, dtype=dtype, device=p.device if on_param else "cpu")
+                if t.device == p.device:
+                    dist.broadcast(t, src=src, group=self.pg)
+                else:  # a host scalar (torch keeps a non-capturable step count there): through the parameter's device
+                    buf = t.to(p.device)
+                    dist.broadcast(buf, src=src, group=self.pg)
+                    t.copy_(buf)
+
+    def zero_grad(self):
+        self.arena.zero_grad()
+
+    def all_reduce(self):
+        """Sum the gradient buffer over the ranks: one collective, stream-ordered after the backward that filled it."""
+        if self.world > 1:
+            dist.all_reduce(self.arena.grads, op=dist.ReduceOp.SUM, group=self.pg)
+
+    def clip_mean_(self, max_norm):
+        """Summed gradients -> their mean over the ranks, clipped to `max_norm` the way
+        ``torch.nn.utils.clip_grad_norm_`` clips it, in one pass over the buffer and without a host synchronisation
+        (it can be captured in a CUDA graph).  Returns the norm of the mean gradient before clipping."""
+        g = self.arena.grads
+        norm = torch.linalg.vector_norm(g) / self.world
+        g.mul_(torch.clamp(max_norm / (norm + 1e-6), max=1.0) / self.world)
+        return norm
+
 
 def lr_lambda(step, train_num_steps, lr, min_lr, warmup=5000):
     """train_uncond_dpm.py:169-177: linear warm-up to 1 over `warmup` steps, then (1 - iter/total)^0.96 with a floor."""
@@ -280,10 +379,7 @@ class TrainStep:
         exist) are broadcast to every rank — what accelerate / DDP do for the reference at wrap time
         (train_uncond_dpm.py:197-198).  Called at construction and after a checkpoint load."""
         if self.world > 1:
-            dist.broadcast(self.arena.flat, src=src, group=self.pg)
-            if moments:
-                dist.broadcast(self.m, src=src, group=self.pg)
-                dist.broadcast(self.v, src=src, group=self.pg)
+            self.arena.broadcast(src, self.pg, (self.m, self.v) if moments else ())
         self.refresh()
 
     # ------------------------------------------------------------------------------------------ gradient reduction
