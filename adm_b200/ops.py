@@ -473,6 +473,9 @@ def softmax_fwd(s):
     return p
 
 
+SOFTMAX_BWD_MAX_LEN = 1024  # one warp per row, 32 values per lane (adm_softmax_bwd)
+
+
 def softmax_bwd(p, dp, scale):
     rows, length = p.numel() // p.shape[-1], p.shape[-1]
     ds = torch.empty(p.shape, device=p.device, dtype=BF16)
@@ -500,24 +503,34 @@ def _attn_workspace(n, hw, heads, backward, device):
     return torch.empty(nbytes, device=device, dtype=torch.uint8), nbytes
 
 
-def attention_fwd(qkv, heads, scale=None, need_p=True, fused=None):
+def attention_fwd(qkv, heads, scale=None, need_p=True, fused=None, out=None, lse=None, work=None):
     """qkv: [N, H, W, 3C] bf16 laid out as (q | k | v), each [heads, d].  Returns (a [N,H,W,C], aux) where aux is what
     attention_bwd needs besides qkv and a: the per-row log-sum-exp [N, heads, HW] fp32 for the fused kernel (d == 64, HW in
     {16, 64, 256}: ONE kernel, probabilities only ever in TMEM), or the normalised probabilities [N*heads, HW, HW] bf16
     for the unfused path.  aux is None when need_p is False.
-    scale defaults to 1/sqrt(d) (d = C / heads as stored, which may include zero padding of the head dim)."""
+    scale defaults to 1/sqrt(d) (d = C / heads as stored, which may include zero padding of the head dim).
+    out / lse: contiguous tensors to write a / the log-sum-exp into (allocated when None); work: a uint8 scratch buffer
+    for the blocked kernels (HW > 256), at least adm_attn_long_workspace bytes."""
     n, h, w, c3 = qkv.shape
     c, hw = c3 // 3, h * w
     d = c // heads
     scale = 1.0 / d ** 0.5 if scale is None else float(scale)
     assert qkv.is_contiguous()
+    if out is None:
+        out = torch.empty(n, h, w, c, device=qkv.device, dtype=BF16)
+    assert out.is_contiguous() and out.dtype == BF16 and tuple(out.shape) == (n, h, w, c)
+    a = out
     if fused is None:
         fused = attention_fused_ok(d, hw)
     if fused:
-        a = torch.empty(n, h, w, c, device=qkv.device, dtype=BF16)
-        lse = torch.empty(n, heads, hw, device=qkv.device, dtype=F32) if need_p else None
+        if lse is None and need_p:
+            lse = torch.empty(n, heads, hw, device=qkv.device, dtype=F32)
+        assert lse is None or (lse.is_contiguous() and lse.dtype == F32 and tuple(lse.shape) == (n, heads, hw))
         if hw > 256:
-            work, nbytes = _attn_workspace(n, hw, heads, False, qkv.device)
+            if work is None:
+                work, nbytes = _attn_workspace(n, hw, heads, False, qkv.device)
+            else:
+                nbytes = work.numel() * work.element_size()
             check(_lib.load().adm_attn_fwd_long(_ptr(qkv), n, hw, heads, scale, _ptr(a), _ptr(lse), _ptr(work), nbytes,
                                                 _stream()), "attn_fwd_long")
             return a, lse
@@ -531,7 +544,6 @@ def attention_fwd(qkv, heads, scale=None, need_p=True, fused=None):
           _operand(qkv, 0, qk_dims, qk_str, c0=0, c0_lo=d, bhi=1),
           _operand(qkv, 0, qk_dims, qk_str, c0=c, c0_lo=d, bhi=1), "attn QK^T")
     p = softmax_fwd(s)
-    a = torch.empty(n, h, w, c, device=qkv.device, dtype=BF16)
     _gemm(dict(m=hw, n=d, k=hw, batches=n * heads, bdiv=heads, splits=1, c=a.data_ptr(), out_mode=0, ldc=c,
                c_bhi=hw * c, c_blo=0, c_col_lo=d, alpha=1.0),
           _operand(p, 0, (hw, hw, n * heads), (hw, hw * hw), bhi=heads, blo=1),
@@ -539,28 +551,38 @@ def attention_fwd(qkv, heads, scale=None, need_p=True, fused=None):
     return a, p
 
 
-def attention_bwd(da, qkv, aux, heads, scale=None, fused=None, a=None):
+def attention_bwd(da, qkv, aux, heads, scale=None, fused=None, a=None, out=None, work=None):
     """Returns dqkv [N,H,W,3C] bf16.  Fused (aux = log-sum-exp, `a` = the forward output): ONE kernel recomputes the
-    probabilities and produces dQ, dK, dV.  Unfused (aux = the saved probabilities): five batched GEMMs + softmax_bwd."""
+    probabilities and produces dQ, dK, dV.  Unfused (aux = the saved probabilities): five batched GEMMs + softmax_bwd.
+    out: a contiguous tensor to write dqkv into (allocated when None); work: as in attention_fwd."""
     n, h, w, c3 = qkv.shape
     c, hw = c3 // 3, h * w
     d = c // heads
     scale = 1.0 / d ** 0.5 if scale is None else float(scale)
     assert da.is_contiguous() and qkv.is_contiguous()
-    dqkv = torch.empty_like(qkv)
+    if out is None:
+        out = torch.empty_like(qkv)
+    assert out.is_contiguous() and out.dtype == BF16 and out.shape == qkv.shape
+    dqkv = out
     if fused is None:
         fused = attention_fused_ok(d, hw)
     if fused:
         assert a is not None and a.is_contiguous() and aux is not None and aux.dtype == F32, \
             "fused attention backward needs the forward output and its log-sum-exp"
         if hw > 256:
-            work, nbytes = _attn_workspace(n, hw, heads, True, qkv.device)
+            if work is None:
+                work, nbytes = _attn_workspace(n, hw, heads, True, qkv.device)
+            else:
+                nbytes = work.numel() * work.element_size()
             check(_lib.load().adm_attn_bwd_long(_ptr(da), _ptr(qkv), _ptr(a), _ptr(aux), n, hw, heads, scale, _ptr(dqkv),
                                                 _ptr(work), nbytes, _stream()), "attn_bwd_long")
             return dqkv
         check(_lib.load().adm_attn_bwd_fused(_ptr(da), _ptr(qkv), _ptr(a), _ptr(aux), n, hw, heads, scale, _ptr(dqkv),
                                              _stream()), "attn_bwd_fused")
         return dqkv
+    if hw > SOFTMAX_BWD_MAX_LEN:  # before the first GEMM: a rejected shape launches nothing and leaves dqkv untouched
+        raise _lib.AdmError(f"attention_bwd: the unfused backward takes rows of at most {SOFTMAX_BWD_MAX_LEN} keys "
+                            f"(got {hw})")
     p = aux
     qk_dims, qk_str = (c3, hw, n), (c3, c3 * hw)
     a_dims, a_str = (c, hw, n), (c, c * hw)
