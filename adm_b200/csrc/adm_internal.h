@@ -1,6 +1,7 @@
 // Internal helpers shared by the .cu translation units of libadm_b200.so.
 #pragma once
 #include <stdarg.h>
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include "../../include/adm_b200.h"
 
@@ -9,6 +10,10 @@ void set_error(const char* fmt, ...);
 const char* get_error();
 int num_sms();
 void count_launch();
+// bf16 tensor map, 128B swizzle, zero OOB fill.  dims/box innermost first; strides in ELEMENTS for dims 1..rank-1.
+// Returns 0, or ADM_ERR_SHAPE / ADM_ERR_CUDA with the error set.
+int encode_map(CUtensorMap* m, const void* ptr, int rank, const long long* dims, const long long* strides,
+               const int* box);
 
 #ifdef __CUDACC__
 // <<<>>> replacement for the hot kernels: optional thread-block cluster.

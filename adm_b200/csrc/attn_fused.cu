@@ -644,33 +644,12 @@ __global__ void __launch_bounds__(256) attn_reduce_kernel(const __nv_bfloat16* _
 
 using namespace adm;
 
-#include <cudaTypedefs.h>
-
-static PFN_cuTensorMapEncodeTiled af_encode = nullptr;
-
 // (channel, pixel, sample) view of a [B, N, ld] bf16 tensor; box = 64 channels x box_pix pixels x box_smp samples
 static int af_map(CUtensorMap* m, const void* ptr, long long ld, int n_pix, int batch, int box_pix, int box_smp) {
-    if (af_encode == nullptr) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess || fn == nullptr) {
-            set_error("cuTensorMapEncodeTiled unavailable");
-            return ADM_ERR_CUDA;
-        }
-        af_encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled>(fn);
-    }
-    cuuint64_t gd[3] = {static_cast<cuuint64_t>(ld), static_cast<cuuint64_t>(n_pix), static_cast<cuuint64_t>(batch)};
-    cuuint64_t gs[2] = {static_cast<cuuint64_t>(ld) * 2, static_cast<cuuint64_t>(ld) * n_pix * 2};
-    cuuint32_t bx[3] = {64, static_cast<cuuint32_t>(box_pix), static_cast<cuuint32_t>(box_smp)};
-    cuuint32_t es[3] = {1, 1, 1};
-    CUresult r = af_encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), gd, gs, bx, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_error("attention: cuTensorMapEncodeTiled failed with CUresult %d", static_cast<int>(r));
-        return ADM_ERR_CUDA;
-    }
-    return 0;
+    const long long dims[3] = {ld, n_pix, batch};
+    const long long strides[2] = {ld, ld * n_pix};
+    const int box[3] = {64, box_pix, box_smp};
+    return encode_map(m, ptr, 3, dims, strides, box);
 }
 
 static int af_setup(const char* what, AttnParams* p, int batch, int n_pix, int heads, float scale) {
@@ -705,10 +684,9 @@ extern "C" int adm_attn_fwd_fused(const void* qkv, int batch, int n_pix, int hea
     p.out = static_cast<__nv_bfloat16*>(out); p.lse = lse; p.o_in = nullptr;
     CUtensorMap mq;
     if (int e = af_map(&mq, qkv, 3LL * p.c, n_pix, batch, n_pix, p.pack)) return e;
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AT_SMEM_TOTAL);
-        attr_set = true;
+    if (const cudaError_t e = set_smem_limit_once<attn_fwd_kernel>(AT_SMEM_TOTAL)) {
+        set_error("attn_fwd_fused launch: %s", cudaGetErrorString(e));
+        return ADM_ERR_CUDA;
     }
     const int grid = p.units < num_sms() ? p.units : num_sms();
     launch_k(attn_fwd_kernel, dim3(grid), dim3(AT_THREADS), AT_SMEM_TOTAL, static_cast<cudaStream_t>(stream), 0, mq, p);
@@ -732,10 +710,9 @@ extern "C" int adm_attn_bwd_fused(const void* da, const void* qkv, const void* o
     CUtensorMap mq, mdo;
     if (int e = af_map(&mq, qkv, 3LL * p.c, n_pix, batch, n_pix, p.pack)) return e;
     if (int e = af_map(&mdo, da, p.c, n_pix, batch, n_pix, p.pack)) return e;
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaFuncSetAttribute(attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AT_SMEM_TOTAL);
-        attr_set = true;
+    if (const cudaError_t e = set_smem_limit_once<attn_bwd_kernel>(AT_SMEM_TOTAL)) {
+        set_error("attn_bwd_fused launch: %s", cudaGetErrorString(e));
+        return ADM_ERR_CUDA;
     }
     const int grid = p.units < num_sms() ? p.units : num_sms();
     launch_k(attn_bwd_kernel, dim3(grid), dim3(AT_THREADS), AT_SMEM_TOTAL, static_cast<cudaStream_t>(stream), 0, mq, mdo, p);
@@ -789,7 +766,10 @@ extern "C" int adm_attn_fwd_long(const void* qkv, int batch, int n_pix, int head
     p.o_in = nullptr;
     CUtensorMap mq;
     if (int e = af_map(&mq, qkv, 3LL * p.c, n_pix, batch, 256, 1)) return e;
-    cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AT_SMEM_TOTAL);
+    if (const cudaError_t e = set_smem_limit_once<attn_fwd_kernel>(AT_SMEM_TOTAL)) {
+        set_error("attn_fwd_long launch: %s", cudaGetErrorString(e));
+        return ADM_ERR_CUDA;
+    }
     const int grid = p.units < num_sms() ? p.units : num_sms();
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     launch_k(attn_fwd_kernel, dim3(grid), dim3(AT_THREADS), AT_SMEM_TOTAL, st, 0, mq, p);
@@ -822,7 +802,10 @@ extern "C" int adm_attn_bwd_long(const void* da, const void* qkv, const void* ou
     CUtensorMap mq, mdo;
     if (int e = af_map(&mq, qkv, 3LL * p.c, n_pix, batch, 256, 1)) return e;
     if (int e = af_map(&mdo, da, p.c, n_pix, batch, 256, 1)) return e;
-    cudaFuncSetAttribute(attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AT_SMEM_TOTAL);
+    if (const cudaError_t e = set_smem_limit_once<attn_bwd_kernel>(AT_SMEM_TOTAL)) {
+        set_error("attn_bwd_long launch: %s", cudaGetErrorString(e));
+        return ADM_ERR_CUDA;
+    }
     const int grid = p.units < num_sms() ? p.units : num_sms();
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     launch_k(attn_bwd_kernel, dim3(grid), dim3(AT_THREADS), AT_SMEM_TOTAL, st, 0, mq, mdo, p);

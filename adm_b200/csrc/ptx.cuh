@@ -37,17 +37,50 @@ __device__ __forceinline__ uint32_t mbar_try_wait(uint64_t* bar, uint32_t parity
         : "memory");
     return ok;
 }
-// Bounded wait: a pipeline bug must never hang the GPU box.  ~4 s at 2 GHz, then flag + trap.
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, int code) {
-    if (mbar_try_wait(bar, parity)) return;
+__device__ __forceinline__ uint32_t mbar_try_wait_cluster(uint64_t* bar, uint32_t parity) {  // acquire at cluster scope
+    uint32_t ok;
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
+        "selp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(ok)
+        : "r"(smem_u32(bar)), "r"(parity)
+        : "memory");
+    return ok;
+}
+// Bounded wait: a pipeline bug must never hang the GPU box.  ~4 s at 2 GHz, then flag + trap.  `code` names the wait
+// site in g_device_error.
+template <typename TryWait>
+__device__ __forceinline__ void bounded_wait(TryWait try_wait, int code) {
+    if (try_wait()) return;
     const long long t0 = clock64();
-    while (!mbar_try_wait(bar, parity)) {
+    while (!try_wait()) {
         if (clock64() - t0 > 8000000000LL) {
             g_device_error = code;
             __threadfence_system();
             asm volatile("trap;");
         }
     }
+}
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, int code) {
+    bounded_wait([=] { return mbar_try_wait(bar, parity); }, code);
+}
+__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity, int code) {
+    bounded_wait([=] { return mbar_try_wait_cluster(bar, parity); }, code);
+}
+// Distributed shared memory: the address of this CTA's shared variable `saddr` in the cluster CTA `rank`.
+__device__ __forceinline__ uint32_t mapa_shared(uint32_t saddr, uint32_t rank) {
+    uint32_t r;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
+    return r;
+}
+__device__ __forceinline__ float4 ld_dsmem_f4(uint32_t caddr) {
+    float4 v;
+    asm volatile("ld.shared::cluster.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(caddr));
+    return v;
+}
+__device__ __forceinline__ void mbar_arrive_remote(uint32_t caddr) {  // release at cluster scope
+    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(caddr) : "memory");
 }
 __device__ __forceinline__ void fence_barrier_init() {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");

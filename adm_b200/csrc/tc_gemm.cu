@@ -45,9 +45,9 @@ static int init_driver() {
     return 0;
 }
 
-// bf16 tensor map, 128B swizzle, zero OOB fill.  dims/box innermost first; strides in ELEMENTS for dims 1..rank-1.
-static int encode_map(CUtensorMap* m, const void* ptr, int rank, const long long* dims, const long long* strides,
-                      const int* box) {
+int encode_map(CUtensorMap* m, const void* ptr, int rank, const long long* dims, const long long* strides,
+               const int* box) {
+    if (int e = init_driver()) return e;
     cuuint64_t gd[5];
     cuuint64_t gs[4];
     cuuint32_t bx[5];
@@ -235,7 +235,6 @@ extern "C" {
 int adm_conv_fprop(const void* x1, int c1, long long ld1, const void* x2, int c2, long long ld2, int n, int h, int w,
                    const void* wpk, int nout, int ntaps, void* out, int out_mode, long long ldc, const float* bias,
                    const void* residual, long long ldr, float alpha, void* stream) {
-    if (int e = init_driver()) return e;
     if (taps_per_row(ntaps) == 0) { set_error("conv_fprop: ntaps must be 1, 9, 25 or 49"); return ADM_ERR_SHAPE; }
     if (c1 <= 0 || c1 % 8 || (x2 && (c2 <= 0 || c2 % 8))) { set_error("conv_fprop: channels must be multiples of 8"); return ADM_ERR_SHAPE; }
     GemmParams p;
@@ -279,7 +278,6 @@ int adm_conv_fprop(const void* x1, int c1, long long ld1, const void* x2, int c2
 int adm_conv_dgrad(const void* dy, int cout, long long ld_dy, int n, int h, int w, const void* wpk, int kpad,
                    int ntaps, void* dx, int n_valid, long long ldc, const void* residual, long long ldr, float alpha,
                    void* stream) {
-    if (int e = init_driver()) return e;
     if (taps_per_row(ntaps) == 0) { set_error("conv_dgrad: ntaps must be 1, 9, 25 or 49"); return ADM_ERR_SHAPE; }
     if (kpad % 64) { set_error("conv_dgrad: kpad must be a multiple of 64"); return ADM_ERR_SHAPE; }
     GemmParams p;
@@ -325,7 +323,6 @@ int adm_conv_wgrad(const void* dy, int cout, long long ld_dy, const void* x1, in
 int adm_conv_wgrad_mapped(const void* dy, int cout, long long ld_dy, const void* x1, int c1, long long ld1,
                           const void* x2, int c2, long long ld2, int n, int h, int w, int ntaps, const int* row_map,
                           float* dw, void* stream) {
-    if (int e = init_driver()) return e;
     if (row_map != nullptr && ntaps != 1) { set_error("conv_wgrad: a row map is supported for 1x1 convs only"); return ADM_ERR_SHAPE; }
     if (taps_per_row(ntaps) == 0) { set_error("conv_wgrad: ntaps must be 1, 9, 25 or 49"); return ADM_ERR_SHAPE; }
     GemmParams p;
@@ -382,7 +379,6 @@ int adm_device_error(void) {
 }
 
 int adm_gemm_batched(const adm_gemm_desc* d, void* stream) {
-    if (int e = init_driver()) return e;
     GemmParams p;
     init_params(&p);
     p.M = d->m; p.N = d->n;

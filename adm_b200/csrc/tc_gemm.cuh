@@ -4,9 +4,8 @@
 // taps per MMA), tc_conv_splitk_kernel (cluster split-K conv) — with the same roles:
 //   warp 0      : TMA producer (one lane)        global -> 128B-swizzled smem ring
 //   warp 1      : TMEM allocator + UMMA issuer   tcgen05.mma, fp32 accumulators in TMEM (2 x 256 columns)
-//   warps 2..   : epilogue                       tcgen05.ld -> +bias, +residual, *alpha -> bf16 / fp32 / fp32 atomics
-//                 (warp w drains TMEM lane quadrant w % 4; with GEMM_EPI_WARPS = 8 the two warps of a quadrant split
-//                 the tile's columns)
+//   warps 2..5  : epilogue                       tcgen05.ld -> +bias, +residual, *alpha -> bf16 / fp32 / fp32 atomics
+//                 (warp w drains TMEM lane quadrant w % 4)
 // Tile = 128 (M) x BN (N, runtime, multiple of 16, <= 256) x 64 (K per stage, bf16 = one 128 B swizzle row).
 #pragma once
 #include "ptx.cuh"
@@ -16,11 +15,10 @@ namespace adm {
 
 constexpr int GEMM_BLOCK_M = 128;
 constexpr int GEMM_BLOCK_K = 64;
-// Epilogue warps: 4 (one per TMEM lane quadrant) or 8 (two per quadrant, each draining half of the tile's columns).
-// Measured on B200 (tools/gemm_accounting.py): 8 warps change nothing on the short-K 1x1 convs — they wait for operand
-// bytes, not for the epilogue — and cost ~8 % on the small 8x8 / 4x4 tiles, so 4 it is.
+// Epilogue warps: one per TMEM lane quadrant.  Eight (two per quadrant, each draining half of the tile's columns) were
+// tried and removed: measured on B200 (tools/gemm_accounting.py) they changed nothing on the short-K 1x1 convs — they
+// wait for operand bytes, not for the epilogue — and cost ~8 % on the small 8x8 / 4x4 tiles.
 constexpr int GEMM_EPI_WARPS = 4;
-constexpr int EPI_HALVES = GEMM_EPI_WARPS / 4;
 constexpr int GEMM_THREADS = 64 + 32 * GEMM_EPI_WARPS;   // TMA warp + MMA warp + epilogue warps
 constexpr int GEMM_A_STAGE = GEMM_BLOCK_M * 128;  // 16 KB
 constexpr int GEMM_SMEM_RING = 200 * 1024;        // operand ring budget
@@ -88,6 +86,96 @@ struct PixWalker {
     }
 };
 
+// Coordinates of a tile of the persistent tile space: tile = ((plane * m_tiles + mt) * n_tiles + nt), plane = bt * splits
+// + sp (see GemmParams).
+struct TileCoord {
+    int nt, mt, sp, bt;
+    __device__ __forceinline__ TileCoord(const GemmParams& p, int tile) {
+        nt = tile % p.n_tiles;
+        int r = tile / p.n_tiles;
+        mt = r % p.m_tiles;
+        r /= p.m_tiles;
+        sp = r % p.splits;
+        bt = r / p.splits;
+    }
+    __device__ __forceinline__ int b_hi(const GemmParams& p) const { return bt / p.bdiv; }
+    __device__ __forceinline__ int b_lo(const GemmParams& p) const { return bt % p.bdiv; }
+    // The plane alone, in one division: the issuers need nothing but the split.
+    static __device__ __forceinline__ int plane(const GemmParams& p, int tile) { return tile / (p.n_tiles * p.m_tiles); }
+};
+
+// Pixel shift (dh, dw) of conv tap `tap` (row-major over the kw x kw kernel, 'same' padding).
+__device__ __forceinline__ void tap_shift(const GemmParams& p, int tap, int& dh, int& dw) {
+    dh = 0;
+    dw = 0;
+    if (p.kw == 3) { dh = tap / 3 - 1; dw = tap % 3 - 1; }
+    else if (p.kw > 1) { dh = tap / p.kw - (p.kw >> 1); dw = tap % p.kw - (p.kw >> 1); }
+}
+
+// Shared memory and TMEM every kernel of the engine starts from: the 1024-aligned operand ring (GEMM_SMEM_RING bytes),
+// then the barriers, the TMEM address and the kernel's own barriers.
+struct GemmPipeline {
+    uint8_t* smem;
+    int num_stages;        // stages of the stage ring
+    uint64_t* full_bar;    // [GEMM_MAX_STAGES] stage landed (TMA transaction bytes)
+    uint64_t* empty_bar;   // [GEMM_MAX_STAGES] stage consumed (UMMA commit)
+    uint64_t* tfull_bar;   // [2] accumulator complete (UMMA commit)
+    uint64_t* tempty_bar;  // [2] accumulator drained (one arrive per epilogue warp)
+    uint64_t* own_bar;     // the kernel's own barriers
+    uint32_t tmem_base;
+};
+
+// Sets a kernel up: thread 0 prefetches the three tensor maps and initialises as many stage_bytes stages as ring_bytes
+// hold (at most GEMM_MAX_STAGES), `naccs` accumulator barrier pairs and, through init_own(own_bar), the kernel's own
+// barriers; warp 1 allocates `tmem_cols` TMEM columns.
+template <typename InitOwn>
+__device__ __forceinline__ GemmPipeline pipeline_setup(uint8_t* smem_raw, const CUtensorMap* m0, const CUtensorMap* m1,
+                                                       const CUtensorMap* m2, int ring_bytes, int stage_bytes, int naccs,
+                                                       uint32_t tmem_cols, InitOwn init_own) {
+    GemmPipeline pl;
+    pl.smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+    pl.num_stages = min(ring_bytes / stage_bytes, GEMM_MAX_STAGES);
+    pl.full_bar = reinterpret_cast<uint64_t*>(pl.smem + GEMM_SMEM_RING);
+    pl.empty_bar = pl.full_bar + GEMM_MAX_STAGES;
+    pl.tfull_bar = pl.empty_bar + GEMM_MAX_STAGES;
+    pl.tempty_bar = pl.tfull_bar + 2;
+    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(pl.tempty_bar + 2);
+    pl.own_bar = pl.tempty_bar + 3;
+
+    if (threadIdx.x == 0) {
+        tma_prefetch_desc(m0);
+        tma_prefetch_desc(m1);
+        tma_prefetch_desc(m2);
+        for (int i = 0; i < pl.num_stages; ++i) {
+            mbar_init(&pl.full_bar[i], 1);
+            mbar_init(&pl.empty_bar[i], 1);
+        }
+        for (int i = 0; i < naccs; ++i) {
+            mbar_init(&pl.tfull_bar[i], 1);
+            mbar_init(&pl.tempty_bar[i], GEMM_EPI_WARPS);
+        }
+        init_own(pl.own_bar);
+        fence_barrier_init();
+        fence_proxy_async_smem();
+    }
+    if ((threadIdx.x >> 5) == 1) tmem_alloc(tmem_ptr, tmem_cols);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    pl.tmem_base = *tmem_ptr;
+    return pl;
+}
+
+// All roles are done: warp 1 frees the TMEM columns pipeline_setup allocated.
+__device__ __forceinline__ void pipeline_teardown(const GemmPipeline& pl, uint32_t tmem_cols) {
+    tc_fence_before();
+    __syncthreads();
+    if ((threadIdx.x >> 5) == 1) {
+        tc_fence_after();
+        tmem_dealloc(pl.tmem_base, tmem_cols);
+    }
+}
+
 // The epilogue warps stage the tile's bias slice (bn <= 256 floats, zero beyond N) in shared memory BEFORE waiting for the
 // accumulator: per-chunk __ldg of the bias missed L1 behind the streaming stores and cost ~30 us on the epilogue-bound
 // 1x1 convs.  `t` = epilogue thread index; named barrier 1 covers exactly the epilogue threads.
@@ -102,11 +190,11 @@ __device__ __forceinline__ void stage_bias(const GemmParams& p, float* sbias, in
 // (four 32x32b.x16 loads in flight behind ONE wait, with the residual row segment prefetched behind the same wait),
 // then alpha * acc + bias + residual -> bf16 / fp32 / fp32 atomics.  c_off / r_off: element offsets of this row in the
 // output and the residual (before the column); col_shift: extra output column offset (batched GEMMs); the tile columns
-// drained are [c_begin, ncols) (multiples of 16).
+// drained are [0, ncols) (a multiple of 16).
 __device__ __forceinline__ void epilogue_row(const GemmParams& p, uint32_t taddr, int col_base, int col_shift,
                                              long long c_off, long long r_off, bool row_ok, const float* sbias,
-                                             int c_begin, int ncols) {
-    for (int c0 = c_begin; c0 < ncols; c0 += 64) {
+                                             int ncols) {
+    for (int c0 = 0; c0 < ncols; c0 += 64) {
         if (col_base + c0 >= p.N) break;  // warp-uniform
         uint32_t v[4][16];
         uint4 rr[4][2];
@@ -216,52 +304,100 @@ __device__ __forceinline__ void epilogue_row(const GemmParams& p, uint32_t taddr
 // The epilogue warps' persistent loop (4 warps, one TMEM lane quadrant each): per tile, stage the bias slice, wait for
 // the accumulator, drain it through epilogue_row, release it.  Shared by tc_gemm_kernel and tc_conv_halo_kernel.
 template <int MODE>
-__device__ __forceinline__ void epilogue_warps(const GemmParams& p, uint8_t* smem, uint32_t tmem_base,
-                                               uint64_t* tfull_bar, uint64_t* tempty_bar, int warp, int lane,
+__device__ __forceinline__ void epilogue_warps(const GemmParams& p, const GemmPipeline& pl, int warp, int lane,
                                                int num_tiles) {
     const int quad = warp & 3;
-    const int half = (warp - 2) >> 2;   // which half of the tile's columns this warp drains
-    const int m = quad * 32 + lane;     // row inside the tile
-    const int c_split = EPI_HALVES == 2 ? (((p.bn >> 1) + 15) & ~15) : p.bn;
-    const int c_begin = half ? c_split : 0, c_end = half ? p.bn : c_split;
+    const int m = quad * 32 + lane;  // row inside the tile
     int acc = 0;
     uint32_t acc_phase = 0;
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const int nt = tile % p.n_tiles;
-        int r = tile / p.n_tiles;
-        const int mt = r % p.m_tiles;
-        r /= p.m_tiles;
-        const int bt = r / p.splits;
-        const int b_hi = bt / p.bdiv, b_lo = bt % p.bdiv;
+        const TileCoord tc(p, tile);
+        const int b_hi = tc.b_hi(p), b_lo = tc.b_lo(p);
 
         long long row_off;  // element offset of this thread's output row (before column)
         bool row_ok;
         if (MODE == GEMM_CONV) {
             int n0, h0, w0;
-            decode_pix(p, mt, n0, h0, w0);
+            decode_pix(p, tc.mt, n0, h0, w0);
             const int wi = m % p.bw, hi = (m / p.bw) % p.bh, ni = m / (p.bw * p.bh);
             const long long pix = (static_cast<long long>(n0 + ni) * p.H + (h0 + hi)) * p.W + (w0 + wi);
             row_ok = pix < p.M;
             row_off = pix;
         } else {
-            const int row = mt * 128 + m;
+            const int row = tc.mt * 128 + m;
             row_ok = row < p.M;
             row_off = (p.row_map != nullptr && row_ok) ? __ldg(p.row_map + row) : row;
         }
         const long long c_base = b_hi * p.c_bhi + b_lo * p.c_blo + row_off * p.ldc;
-        const int col_base = nt * p.bn;           // column inside [0, N)
+        const int col_base = tc.nt * p.bn;        // column inside [0, N)
         const int col_shift = b_lo * p.c_col_lo;  // extra offset in the output row
 
-        float* sbias = reinterpret_cast<float*>(smem + GEMM_SMEM_RING + 1024) + acc * 256;
+        float* sbias = reinterpret_cast<float*>(pl.smem + GEMM_SMEM_RING + 1024) + acc * 256;
         stage_bias(p, sbias, col_base, (warp - 2) * 32 + lane);
-        mbar_wait(&tfull_bar[acc], acc_phase, 4);
+        mbar_wait(&pl.tfull_bar[acc], acc_phase, 4);
         tc_fence_after();
-        const uint32_t taddr = tmem_base + acc * 256 + (static_cast<uint32_t>(quad * 32) << 16);
-        epilogue_row(p, taddr, col_base, col_shift, c_base, row_off * p.ldr, row_ok, sbias, c_begin, c_end);
+        const uint32_t taddr = pl.tmem_base + acc * 256 + (static_cast<uint32_t>(quad * 32) << 16);
+        epilogue_row(p, taddr, col_base, col_shift, c_base, row_off * p.ldr, row_ok, sbias, p.bn);
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty_bar[acc]);
+        if (lane == 0) mbar_arrive(&pl.tempty_bar[acc]);
         if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+    }
+}
+
+// One stage of the implicit-GEMM conv, k-iteration ki = tap * cchunks + kc: the pixel box at tap `tap`'s shift, channel
+// chunk kc (past cchunks1 from A source 2: the fused channel concat), and the weight tile.
+__device__ __forceinline__ void load_conv_stage(const GemmParams& p, const CUtensorMap* tmA, const CUtensorMap* tmA2,
+                                                const CUtensorMap* tmB, uint8_t* sa, uint64_t* bar, int ki, int tap,
+                                                int kc, int nt, int n0, int h0, int w0) {
+    uint8_t* sb = sa + GEMM_A_STAGE;
+    int dh, dw;
+    tap_shift(p, tap, dh, dw);
+    if (kc < p.cchunks1)
+        tma_load_4d(sa, tmA, bar, kc * 64, w0 + dw, h0 + dh, n0);
+    else
+        tma_load_4d(sa, tmA2, bar, (kc - p.cchunks1) * 64, w0 + dw, h0 + dh, n0);
+    if (!p.b_mn) {
+        // weights [Nout][ntaps * Kpad], K-major
+        tma_load_2d(sb, tmB, bar, ki * 64, nt * p.bn);
+    } else {
+        // dgrad on the fprop-packed weights viewed as (N_gemm = Cin, taps, K_gemm = Cout): the spatial flip is the tap
+        // reversal, the transpose is the MN-major operand mode.
+        for (int c = 0; c * 64 < p.bn; ++c)
+            tma_load_3d(sb + c * 8192, tmB, bar, nt * p.bn + c * 64, p.ntaps - 1 - tap, kc * 64);
+    }
+}
+
+// UMMA descriptors of a 128 x bn x 64 ring stage (A at the stage start, B GEMM_A_STAGE bytes behind it).  Built once, out
+// of the issue loop: this thread's instruction stream is the critical path of the main loop.
+struct StageDescs {
+    uint32_t idesc;
+    uint32_t a_kstep, b_kstep;  // 16-deep k-step strides, in 16 B units
+    uint64_t da0, db0;
+    __device__ __forceinline__ StageDescs(int bn, int a_mn, int b_mn)
+        : idesc(make_idesc_bf16(GEMM_BLOCK_M, bn, a_mn, b_mn)),
+          a_kstep((a_mn ? 2048u : 32u) >> 4),
+          b_kstep((b_mn ? 2048u : 32u) >> 4),
+          da0(make_smem_desc(0, a_mn ? 8192u : 16u, 1024)),
+          db0(make_smem_desc(0, b_mn ? 8192u : 16u, 1024)) {}
+};
+
+// Issues k-iterations [k_begin, k_end) of one tile into the accumulator at tmem_d: per ring stage, wait for it to land,
+// four UMMA k-steps, release it.  `code` names the full-barrier wait site.
+__device__ __forceinline__ void issue_k_range(const GemmPipeline& pl, const StageDescs& d, int stage_bytes, int& stage,
+                                              uint32_t& phase, uint32_t tmem_d, int k_begin, int k_end, int code) {
+    for (int ki = k_begin; ki < k_end; ++ki) {
+        mbar_wait(&pl.full_bar[stage], phase, code);
+        tc_fence_after();
+        // In a non-leader CTA of a cluster the shared-window address carries bits above the 14-bit descriptor field:
+        // unmasked they spill into the leading-byte-offset field (which only MN-major multi-chunk B reads).
+        const uint32_t sa16 = (smem_u32(pl.smem + stage * stage_bytes) & 0x3FFFFu) >> 4;
+        const uint64_t da = d.da0 + sa16, db = d.db0 + (sa16 + (GEMM_A_STAGE >> 4));
+#pragma unroll
+        for (int k = 0; k < GEMM_BLOCK_K / 16; ++k)
+            umma_bf16(tmem_d, da + k * d.a_kstep, db + k * d.b_kstep, d.idesc, (ki > k_begin || k > 0) ? 1u : 0u);
+        umma_commit(&pl.empty_bar[stage]);
+        if (++stage == pl.num_stages) { stage = 0; phase ^= 1; }
     }
 }
 
@@ -270,41 +406,13 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmA2,
                const __grid_constant__ CUtensorMap tmB, const __grid_constant__ GemmParams p) {
     extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int stage_bytes = GEMM_A_STAGE + p.bn * 128;
-    int num_stages = GEMM_SMEM_RING / stage_bytes;
-    if (num_stages > GEMM_MAX_STAGES) num_stages = GEMM_MAX_STAGES;
-
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + GEMM_SMEM_RING);
-    uint64_t* empty_bar = full_bar + GEMM_MAX_STAGES;
-    uint64_t* tfull_bar = empty_bar + GEMM_MAX_STAGES;
-    uint64_t* tempty_bar = tfull_bar + 2;
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tempty_bar + 2);
-
+    const GemmPipeline pl = pipeline_setup(smem_raw, &tmA, &tmA2, &tmB, GEMM_SMEM_RING, stage_bytes, 2, 512,
+                                           [](uint64_t*) {});
+    uint8_t* smem = pl.smem;
+    uint64_t* full_bar = pl.full_bar;
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmA);
-        tma_prefetch_desc(&tmA2);
-        tma_prefetch_desc(&tmB);
-        for (int i = 0; i < num_stages; ++i) {
-            mbar_init(&full_bar[i], 1);
-            mbar_init(&empty_bar[i], 1);
-        }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&tfull_bar[i], 1);
-            mbar_init(&tempty_bar[i], GEMM_EPI_WARPS);
-        }
-        fence_barrier_init();
-        fence_proxy_async_smem();
-    }
-    if (warp == 1) tmem_alloc(tmem_ptr, 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
-
     const int num_tiles = p.batches * p.splits * p.m_tiles * p.n_tiles;
 
     if (warp == 0) {
@@ -313,51 +421,30 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             int stage = 0;
             uint32_t phase = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-                const int nt = tile % p.n_tiles;
-                int r = tile / p.n_tiles;
-                const int mt = r % p.m_tiles;
-                r /= p.m_tiles;
-                const int sp = r % p.splits;
-                const int bt = r / p.splits;
-                const int k_begin = sp * p.k_iters;
+                const TileCoord tc(p, tile);
+                const int nt = tc.nt, mt = tc.mt, bt = tc.bt;
+                const int k_begin = tc.sp * p.k_iters;
                 const int k_end = min(p.k_total, k_begin + p.k_iters);
                 int n0 = 0, h0 = 0, w0 = 0;
                 if (MODE == GEMM_CONV) decode_pix(p, mt, n0, h0, w0);
-                const int b_hi = bt / p.bdiv, b_lo = bt % p.bdiv;
+                const int b_hi = tc.b_hi(p), b_lo = tc.b_lo(p);
                 int tap = 0, kc = 0;  // conv: ki = tap * cchunks + kc, walked without divisions
                 if (MODE == GEMM_CONV) { tap = k_begin / p.cchunks; kc = k_begin % p.cchunks; }
                 PixWalker px(p, MODE == GEMM_WGRAD ? k_begin : 0);
                 for (int ki = k_begin; ki < k_end; ++ki) {
-                    mbar_wait(&empty_bar[stage], phase ^ 1, 1);
+                    mbar_wait(&pl.empty_bar[stage], phase ^ 1, 1);
                     uint8_t* sa = smem + stage * stage_bytes;
                     uint8_t* sb = sa + GEMM_A_STAGE;
                     mbar_expect_tx(&full_bar[stage], stage_bytes);
                     if (MODE == GEMM_CONV) {
-                        int dh = 0, dw = 0;
-                        if (p.kw == 3) { dh = tap / 3 - 1; dw = tap % 3 - 1; }
-                        else if (p.kw > 1) { dh = tap / p.kw - (p.kw >> 1); dw = tap % p.kw - (p.kw >> 1); }
-                        if (kc < p.cchunks1)
-                            tma_load_4d(sa, &tmA, &full_bar[stage], kc * 64, w0 + dw, h0 + dh, n0);
-                        else
-                            tma_load_4d(sa, &tmA2, &full_bar[stage], (kc - p.cchunks1) * 64, w0 + dw, h0 + dh, n0);
-                        if (!p.b_mn) {
-                            // weights [Nout][ntaps * Kpad], K-major
-                            tma_load_2d(sb, &tmB, &full_bar[stage], ki * 64, nt * p.bn);
-                        } else {
-                            // dgrad on the fprop-packed weights viewed as (N_gemm = Cin, taps, K_gemm = Cout): the
-                            // spatial flip is the tap reversal, the transpose is the MN-major operand mode.
-                            for (int c = 0; c * 64 < p.bn; ++c)
-                                tma_load_3d(sb + c * 8192, &tmB, &full_bar[stage], nt * p.bn + c * 64,
-                                            p.ntaps - 1 - tap, kc * 64);
-                        }
+                        load_conv_stage(p, &tmA, &tmA2, &tmB, sa, &full_bar[stage], ki, tap, kc, nt, n0, h0, w0);
                         if (++kc == p.cchunks) { kc = 0; ++tap; }
                     } else if (MODE == GEMM_WGRAD) {
                         // K runs over pixel blocks of 64; bt = tap.  A = dY (MN-major), B = shifted X (MN-major).
                         n0 = px.n0; h0 = px.h0; w0 = px.w0;
                         px.advance(p);
-                        int dh = 0, dw = 0;
-                        if (p.kw == 3) { dh = bt / 3 - 1; dw = bt % 3 - 1; }
-                        else if (p.kw > 1) { dh = bt / p.kw - (p.kw >> 1); dw = bt % p.kw - (p.kw >> 1); }
+                        int dh, dw;
+                        tap_shift(p, bt, dh, dw);
                         tma_load_4d(sa, &tmA, &full_bar[stage], mt * 128, w0, h0, n0);
                         tma_load_4d(sa + 8192, &tmA, &full_bar[stage], mt * 128 + 64, w0, h0, n0);
                         // fused channel concat on the X side: columns >= n_split come from the second source
@@ -386,56 +473,33 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                                             b1 + ki * 64, b2);
                         }
                     }
-                    if (++stage == num_stages) { stage = 0; phase ^= 1; }
+                    if (++stage == pl.num_stages) { stage = 0; phase ^= 1; }
                 }
             }
         }
     } else if (warp == 1) {
         // =========================================================== UMMA issuer
         if (lane == 0) {
-            const uint32_t idesc = make_idesc_bf16(GEMM_BLOCK_M, p.bn, p.a_mn, p.b_mn);
-            const uint32_t a_lbo = p.a_mn ? 8192u : 16u, b_lbo = p.b_mn ? 8192u : 16u;
-            // descriptor constants and k-step strides (in 16 B units) are hoisted: this thread's instruction stream is
-            // the critical path of the main loop
-            const uint32_t a_kstep = (p.a_mn ? 2048u : 32u) >> 4, b_kstep = (p.b_mn ? 2048u : 32u) >> 4;
-            const uint64_t da0 = make_smem_desc(0, a_lbo, 1024), db0 = make_smem_desc(0, b_lbo, 1024);
+            const StageDescs d(p.bn, p.a_mn, p.b_mn);
             int stage = 0;
             uint32_t phase = 0;
             int acc = 0;
             uint32_t acc_phase = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-                const int sp = (tile / (p.n_tiles * p.m_tiles)) % p.splits;
-                const int k_begin = sp * p.k_iters;
+                const int k_begin = TileCoord::plane(p, tile) % p.splits * p.k_iters;
                 const int k_end = min(p.k_total, k_begin + p.k_iters);
-                mbar_wait(&tempty_bar[acc], acc_phase ^ 1, 2);
+                mbar_wait(&pl.tempty_bar[acc], acc_phase ^ 1, 2);
                 tc_fence_after();
-                const uint32_t tmem_d = tmem_base + acc * 256;
-                for (int ki = k_begin; ki < k_end; ++ki) {
-                    mbar_wait(&full_bar[stage], phase, 3);
-                    tc_fence_after();
-                    const uint32_t sa16 = (smem_u32(smem + stage * stage_bytes) & 0x3FFFFu) >> 4;
-                    const uint64_t da = da0 + sa16, db = db0 + (sa16 + (GEMM_A_STAGE >> 4));
-#pragma unroll
-                    for (int k = 0; k < GEMM_BLOCK_K / 16; ++k)
-                        umma_bf16(tmem_d, da + k * a_kstep, db + k * b_kstep, idesc, (ki > k_begin || k > 0) ? 1u : 0u);
-                    umma_commit(&empty_bar[stage]);
-                    if (++stage == num_stages) { stage = 0; phase ^= 1; }
-                }
-                umma_commit(&tfull_bar[acc]);
+                issue_k_range(pl, d, stage_bytes, stage, phase, pl.tmem_base + acc * 256, k_begin, k_end, 3);
+                umma_commit(&pl.tfull_bar[acc]);
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
         }
     } else {
         // =========================================================== epilogue (4 warps, one TMEM lane quadrant each)
-        epilogue_warps<MODE>(p, smem, tmem_base, tfull_bar, tempty_bar, warp, lane, num_tiles);
+        epilogue_warps<MODE>(p, pl, warp, lane, num_tiles);
     }
-
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 512);
-    }
+    pipeline_teardown(pl, 512);
 }
 
 // ------------------------------------------------------------------------------------------------ cluster split-K conv
@@ -445,52 +509,19 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 // TMEM accumulator; the non-leaders then park their fp32 partial tiles in their (now idle) operand ring, signal the leader's
 // mbarrier across the cluster, and the leader adds them through distributed shared memory (ld.shared::cluster) into its
 // accumulator before the ordinary epilogue.  One tile per CTA (grid = tiles x ksplit); roles as in tc_gemm_kernel.
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t saddr, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ float4 ld_dsmem_f4(uint32_t caddr) {
-    float4 v;
-    asm volatile("ld.shared::cluster.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(caddr));
-    return v;
-}
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t caddr) {  // release at cluster scope
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(caddr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity, int code) {  // acquire at cluster scope
-    const long long t0 = clock64();
-    uint32_t ok = 0;
-    while (!ok) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-        if (!ok && clock64() - t0 > 8000000000LL) {
-            g_device_error = code;
-            __threadfence_system();
-            asm volatile("trap;");
-        }
-    }
-}
-
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 tc_conv_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmA2,
                       const __grid_constant__ CUtensorMap tmB, const __grid_constant__ GemmParams p) {
     extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int stage_bytes = GEMM_A_STAGE + p.bn * 128;
-    int num_stages = GEMM_SMEM_RING / stage_bytes;
-    if (num_stages > GEMM_MAX_STAGES) num_stages = GEMM_MAX_STAGES;
-
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + GEMM_SMEM_RING);
-    uint64_t* empty_bar = full_bar + GEMM_MAX_STAGES;
-    uint64_t* tfull_bar = empty_bar + GEMM_MAX_STAGES;
-    uint64_t* peers_bar = tfull_bar + 1;  // leader: the non-leaders' partial tiles are parked
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(peers_bar + 1);
+    // one accumulator; the leader's own barrier counts the non-leaders' parked partial tiles
+    const GemmPipeline pl = pipeline_setup(smem_raw, &tmA, &tmA2, &tmB, GEMM_SMEM_RING, stage_bytes, 1, 256,
+                                           [&](uint64_t* own) { mbar_init(own, (p.ksplit - 1) * GEMM_EPI_WARPS); });
+    cluster_sync_all();  // the leader's peers_bar is initialised before any remote arrive
+    uint8_t* smem = pl.smem;
+    uint64_t* full_bar = pl.full_bar;
+    uint64_t* peers_bar = pl.own_bar;
+    const uint32_t tmem_base = pl.tmem_base;
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
@@ -499,26 +530,6 @@ tc_conv_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
     const int nt = tile % p.n_tiles, mt = tile / p.n_tiles;
     const int k_begin = rank * p.k_iters;
     const int k_end = min(p.k_total, k_begin + p.k_iters);
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmA);
-        tma_prefetch_desc(&tmA2);
-        tma_prefetch_desc(&tmB);
-        for (int i = 0; i < num_stages; ++i) {
-            mbar_init(&full_bar[i], 1);
-            mbar_init(&empty_bar[i], 1);
-        }
-        mbar_init(tfull_bar, 1);
-        mbar_init(peers_bar, (p.ksplit - 1) * GEMM_EPI_WARPS);
-        fence_barrier_init();
-        fence_proxy_async_smem();
-    }
-    if (warp == 1) tmem_alloc(tmem_ptr, 256);
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();  // the leader's peers_bar is initialised before any remote arrive
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
 
     int n0, h0, w0;
     decode_pix(p, mt, n0, h0, w0);
@@ -529,50 +540,21 @@ tc_conv_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
             uint32_t phase = 0;
             int tap = k_begin / p.cchunks, kc = k_begin % p.cchunks;
             for (int ki = k_begin; ki < k_end; ++ki) {
-                mbar_wait(&empty_bar[stage], phase ^ 1, 41);
+                mbar_wait(&pl.empty_bar[stage], phase ^ 1, 41);
                 uint8_t* sa = smem + stage * stage_bytes;
-                uint8_t* sb = sa + GEMM_A_STAGE;
                 mbar_expect_tx(&full_bar[stage], stage_bytes);
-                int dh = 0, dw = 0;
-                if (p.kw == 3) { dh = tap / 3 - 1; dw = tap % 3 - 1; }
-                        else if (p.kw > 1) { dh = tap / p.kw - (p.kw >> 1); dw = tap % p.kw - (p.kw >> 1); }
-                if (kc < p.cchunks1)
-                    tma_load_4d(sa, &tmA, &full_bar[stage], kc * 64, w0 + dw, h0 + dh, n0);
-                else
-                    tma_load_4d(sa, &tmA2, &full_bar[stage], (kc - p.cchunks1) * 64, w0 + dw, h0 + dh, n0);
-                if (!p.b_mn) {
-                    tma_load_2d(sb, &tmB, &full_bar[stage], ki * 64, nt * p.bn);
-                } else {
-                    for (int c = 0; c * 64 < p.bn; ++c)
-                        tma_load_3d(sb + c * 8192, &tmB, &full_bar[stage], nt * p.bn + c * 64, p.ntaps - 1 - tap, kc * 64);
-                }
+                load_conv_stage(p, &tmA, &tmA2, &tmB, sa, &full_bar[stage], ki, tap, kc, nt, n0, h0, w0);
                 if (++kc == p.cchunks) { kc = 0; ++tap; }
-                if (++stage == num_stages) { stage = 0; phase ^= 1; }
+                if (++stage == pl.num_stages) { stage = 0; phase ^= 1; }
             }
         }
     } else if (warp == 1) {
         // =========================================================== UMMA issuer
         if (lane == 0) {
-            const uint32_t idesc = make_idesc_bf16(GEMM_BLOCK_M, p.bn, 0, p.b_mn);
-            const uint32_t b_lbo = p.b_mn ? 8192u : 16u;
-            const uint32_t b_kstep = (p.b_mn ? 2048u : 32u) >> 4;
-            const uint64_t da0 = make_smem_desc(0, 16u, 1024), db0 = make_smem_desc(0, b_lbo, 1024);
             int stage = 0;
             uint32_t phase = 0;
-            for (int ki = k_begin; ki < k_end; ++ki) {
-                mbar_wait(&full_bar[stage], phase, 43);
-                tc_fence_after();
-                // In a non-leader CTA of a cluster the shared-window address carries bits above the 14-bit descriptor field:
-                // unmasked they spill into the leading-byte-offset field (which only MN-major multi-chunk B reads).
-                const uint32_t sa16 = (smem_u32(smem + stage * stage_bytes) & 0x3FFFFu) >> 4;
-                const uint64_t da = da0 + sa16, db = db0 + (sa16 + (GEMM_A_STAGE >> 4));
-#pragma unroll
-                for (int k = 0; k < GEMM_BLOCK_K / 16; ++k)
-                    umma_bf16(tmem_base, da + 2 * k, db + k * b_kstep, idesc, (ki > k_begin || k > 0) ? 1u : 0u);
-                umma_commit(&empty_bar[stage]);
-                if (++stage == num_stages) { stage = 0; phase ^= 1; }
-            }
-            umma_commit(tfull_bar);
+            issue_k_range(pl, StageDescs(p.bn, 0, p.b_mn), stage_bytes, stage, phase, tmem_base, k_begin, k_end, 43);
+            umma_commit(pl.tfull_bar);
         }
     } else {
         // =========================================================== epilogue (4 warps, one TMEM lane quadrant each)
@@ -584,7 +566,7 @@ tc_conv_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
         const int col_base = nt * p.bn;
         float* sbias = reinterpret_cast<float*>(smem + GEMM_SMEM_RING + 1024);
         if (rank == 0) stage_bias(p, sbias, col_base, (warp - 2) * 32 + lane);
-        mbar_wait(tfull_bar, 0, 44);  // this CTA's K range is in its accumulator; its operand ring is idle from here on
+        mbar_wait(pl.tfull_bar, 0, 44);  // this CTA's K range is in its accumulator; its operand ring is idle from here on
         tc_fence_after();
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
         float4* park = reinterpret_cast<float4*>(smem);  // [bn / 4][128 rows] float4: lanes write consecutive 16 B
@@ -625,17 +607,11 @@ tc_conv_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
                 }
                 tmem_st_wait();
             }
-            epilogue_row(p, taddr, col_base, 0, pix * p.ldc, pix * p.ldr, row_ok, sbias, 0, p.bn);
+            epilogue_row(p, taddr, col_base, 0, pix * p.ldc, pix * p.ldr, row_ok, sbias, p.bn);
         }
     }
-
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();  // no CTA exits (or frees TMEM) while the leader may still read its shared memory
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 256);
-    }
+    pipeline_teardown(pl, 256);
+    cluster_sync_all();  // no CTA exits while the leader may still read its parked partial tile
 }
 
 // ------------------------------------------------------------------------------------------------ halo conv kernel
@@ -659,48 +635,24 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
 tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmA2,
                     const __grid_constant__ CUtensorMap tmB, const __grid_constant__ GemmParams p) {
     extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int b_bytes = p.bn * 128;
-    int nb = (GEMM_SMEM_RING - HALO_BUFS * HALO_BYTES) / b_bytes;
-    if (nb > GEMM_MAX_STAGES) nb = GEMM_MAX_STAGES;
+    // the stage ring is the weight ring, behind the halo buffers; the kernel's own barriers are the halo ring's
+    const auto init_halo_ring = [](uint64_t* own) {
+        for (int i = 0; i < 2 * HALO_BUFS; ++i) mbar_init(&own[i], 1);
+    };
+    const GemmPipeline pl = pipeline_setup(smem_raw, &tmA, &tmA2, &tmB, GEMM_SMEM_RING - HALO_BUFS * HALO_BYTES, b_bytes,
+                                           2, 512, init_halo_ring);
+    uint8_t* smem = pl.smem;
     uint8_t* b_ring = smem + HALO_BUFS * HALO_BYTES;
-
-    uint64_t* bfull = reinterpret_cast<uint64_t*>(smem + GEMM_SMEM_RING);
-    uint64_t* bempty = bfull + GEMM_MAX_STAGES;
-    uint64_t* tfull_bar = bempty + GEMM_MAX_STAGES;
-    uint64_t* tempty_bar = tfull_bar + 2;
-    uint64_t* hfull = tempty_bar + 2;  // halo buffer landed
+    const int nb = pl.num_stages;
+    uint64_t* bfull = pl.full_bar;
+    uint64_t* bempty = pl.empty_bar;
+    uint64_t* hfull = pl.own_bar;  // halo buffer landed
     uint64_t* hempty = hfull + HALO_BUFS;
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(hempty + HALO_BUFS);
+    const uint32_t tmem_base = pl.tmem_base;
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmA);
-        tma_prefetch_desc(&tmA2);
-        tma_prefetch_desc(&tmB);
-        for (int i = 0; i < nb; ++i) {
-            mbar_init(&bfull[i], 1);
-            mbar_init(&bempty[i], 1);
-        }
-        for (int i = 0; i < HALO_BUFS; ++i) {
-            mbar_init(&hfull[i], 1);
-            mbar_init(&hempty[i], 1);
-        }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&tfull_bar[i], 1);
-            mbar_init(&tempty_bar[i], GEMM_EPI_WARPS);
-        }
-        fence_barrier_init();
-        fence_proxy_async_smem();
-    }
-    if (warp == 1) tmem_alloc(tmem_ptr, 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
-
     const int num_tiles = p.m_tiles * p.n_tiles;
 
     if (warp == 0) {
@@ -720,21 +672,21 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                     tma_load_4d(dst, &tmA2, &hfull[hs], (kc - p.cchunks1) * 64, w0 - 1, h0 - 1, n0);
                 if (++hs == HALO_BUFS) { hs = 0; hphase ^= 1; }
             };
-            // Halo loads run AHEAD of the weight tiles by `ahead` chunk steps (a cursor over (tile, chunk) that only this
-            // thread advances): 1 step hides the TMA latency under the nine MMAs of the current chunk; three buffers:
-            // loading, multiplying, draining.
+            // Halo loads run one chunk step AHEAD of the weight tiles (a cursor over (tile, chunk) that only this thread
+            // advances): one step hides the TMA latency under the nine MMAs of the current chunk; three buffers:
+            // loading, multiplying, draining.  (Two steps make this thread wait for the buffer still being multiplied
+            // before it issues weights.)
             int cur_tile = blockIdx.x, cur_kc = 0;
             auto next_halo = [&]() {
                 if (cur_tile >= num_tiles) return;
                 load_halo(cur_tile, cur_kc);
                 if (++cur_kc == p.cchunks) { cur_kc = 0; cur_tile += gridDim.x; }
             };
-            const int ahead = 1;  // (2 makes this thread wait for the buffer still being multiplied before it issues weights)
-            for (int i = 0; i < ahead; ++i) next_halo();
+            next_halo();
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
                 const int nt = tile % p.n_tiles;
                 for (int kc = 0; kc < p.cchunks; ++kc) {
-                    next_halo();  // the halo `ahead` steps from now goes out before this step's nine weight tiles
+                    next_halo();  // the next step's halo goes out before this step's nine weight tiles
                     for (int tap = 0; tap < 9; ++tap) {
                         mbar_wait(&bempty[bs], bphase ^ 1, 1);
                         uint8_t* sb = b_ring + bs * b_bytes;
@@ -762,7 +714,7 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             int acc = 0;
             uint32_t acc_phase = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-                mbar_wait(&tempty_bar[acc], acc_phase ^ 1, 2);
+                mbar_wait(&pl.tempty_bar[acc], acc_phase ^ 1, 2);
                 tc_fence_after();
                 const uint32_t tmem_d = tmem_base + acc * 256;
                 for (int kc = 0; kc < p.cchunks; ++kc) {
@@ -784,20 +736,15 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                     umma_commit(&hempty[hs]);
                     if (++hs == HALO_BUFS) { hs = 0; hphase ^= 1; }
                 }
-                umma_commit(&tfull_bar[acc]);
+                umma_commit(&pl.tfull_bar[acc]);
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
         }
     } else {
-        epilogue_warps<GEMM_CONV>(p, smem, tmem_base, tfull_bar, tempty_bar, warp, lane, num_tiles);
+        epilogue_warps<GEMM_CONV>(p, pl, warp, lane, num_tiles);
     }
 
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 512);
-    }
+    pipeline_teardown(pl, 512);
 }
 
 // ------------------------------------------------------------------------------------------------ tap-row wgrad kernel
@@ -809,47 +756,19 @@ tc_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 //     (zero outside the image): Cout = 192 gives 9 M chunks = 4.5 tiles instead of 9 x 2 half-empty ones.
 // Per k-iteration (64 pixels) an SM ingests 16 KB + ~9 KB for 128 x 192 x 64 MACs, against 16 KB + 24 KB per tap before.
 // K = pixels (split across CTAs, fp32 atomics into the gradient arena), roles as in tc_gemm_kernel.
-// K = pixels (split across CTAs, fp32 atomics into the gradient arena), roles as in tc_gemm_kernel.
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 tc_wgrad_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                      const __grid_constant__ CUtensorMap tmB2, const __grid_constant__ GemmParams p) {
     extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int halo_w = p.bw + 2;
     const int b_tx = p.bh * halo_w * 128;
     const int stage_bytes = GEMM_A_STAGE + ((b_tx + 1023) & ~1023);
-    int num_stages = GEMM_SMEM_RING / stage_bytes;
-    if (num_stages > GEMM_MAX_STAGES) num_stages = GEMM_MAX_STAGES;
-
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + GEMM_SMEM_RING);
-    uint64_t* empty_bar = full_bar + GEMM_MAX_STAGES;
-    uint64_t* tfull_bar = empty_bar + GEMM_MAX_STAGES;
-    uint64_t* tempty_bar = tfull_bar + 2;
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tempty_bar + 2);
-
+    const GemmPipeline pl = pipeline_setup(smem_raw, &tmA, &tmB, &tmB2, GEMM_SMEM_RING, stage_bytes, 2, 512,
+                                           [](uint64_t*) {});
+    uint8_t* smem = pl.smem;
+    uint64_t* full_bar = pl.full_bar;
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmA);
-        tma_prefetch_desc(&tmB);
-        tma_prefetch_desc(&tmB2);
-        for (int i = 0; i < num_stages; ++i) {
-            mbar_init(&full_bar[i], 1);
-            mbar_init(&empty_bar[i], 1);
-        }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&tfull_bar[i], 1);
-            mbar_init(&tempty_bar[i], GEMM_EPI_WARPS);
-        }
-        fence_barrier_init();
-        fence_proxy_async_smem();
-    }
-    if (warp == 1) tmem_alloc(tmem_ptr, 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
 
     // tile = (sp * m_tiles + mt) * n_tiles + nt : CTAs running together share a pixel range (split) — its dY / X boxes
     // stay L2-resident.  (A stream-K division of the (tile, k) space balanced the SMs but was 10 % slower: neighbouring
@@ -863,28 +782,26 @@ tc_wgrad_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
             int stage = 0;
             uint32_t phase = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-                const int nt = tile % p.n_tiles;
-                const int mt = (tile / p.n_tiles) % p.m_tiles;
-                const int sp = tile / (p.n_tiles * p.m_tiles);
-                const int k_begin = sp * p.k_iters;
+                const TileCoord tc(p, tile);
+                const int k_begin = tc.sp * p.k_iters;
                 const int k_end = min(p.k_total, k_begin + p.k_iters);
-                const int mc0 = 2 * mt, mc1 = min(2 * mt + 1, m_chunks - 1);  // an odd tail repeats a chunk (masked)
+                const int mc0 = 2 * tc.mt, mc1 = min(2 * tc.mt + 1, m_chunks - 1);  // an odd tail repeats a chunk (masked)
                 const int dy0 = mc0 / p.co_chunks, cc0 = mc0 % p.co_chunks;
                 const int dy1 = mc1 / p.co_chunks, cc1 = mc1 % p.co_chunks;
-                const bool src2 = nt >= p.cchunks1;
+                const bool src2 = tc.nt >= p.cchunks1;
                 const CUtensorMap* mb = src2 ? &tmB2 : &tmB;
-                const int nc = (src2 ? nt - p.cchunks1 : nt) * 64;
+                const int nc = (src2 ? tc.nt - p.cchunks1 : tc.nt) * 64;
                 PixWalker px(p, k_begin);
                 for (int ki = k_begin; ki < k_end; ++ki) {
                     const int n0 = px.n0, h0 = px.h0, w0 = px.w0;
                     px.advance(p);
-                    mbar_wait(&empty_bar[stage], phase ^ 1, 1);
+                    mbar_wait(&pl.empty_bar[stage], phase ^ 1, 1);
                     uint8_t* sa = smem + stage * stage_bytes;
                     mbar_expect_tx(&full_bar[stage], GEMM_A_STAGE + b_tx);
                     tma_load_4d(sa, &tmA, &full_bar[stage], cc0 * 64, w0, h0 + 1 - dy0, n0);
                     tma_load_4d(sa + 8192, &tmA, &full_bar[stage], cc1 * 64, w0, h0 + 1 - dy1, n0);
                     tma_load_4d(sa + GEMM_A_STAGE, mb, &full_bar[stage], nc, w0 - 1, h0, n0);
-                    if (++stage == num_stages) { stage = 0; phase ^= 1; }
+                    if (++stage == pl.num_stages) { stage = 0; phase ^= 1; }
                 }
             }
         }
@@ -910,12 +827,11 @@ tc_wgrad_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
             int acc = 0;
             uint32_t acc_phase = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-                const int sp = tile / (p.n_tiles * p.m_tiles);
-                const int k_begin = sp * p.k_iters;
+                const int k_begin = TileCoord::plane(p, tile) * p.k_iters;  // no batches: the plane is the split
                 const int k_end = min(p.k_total, k_begin + p.k_iters);
-                mbar_wait(&tempty_bar[acc], acc_phase ^ 1, 2);
+                mbar_wait(&pl.tempty_bar[acc], acc_phase ^ 1, 2);
                 tc_fence_after();
-                const uint32_t tmem_d = tmem_base + acc * 256;
+                const uint32_t tmem_d = pl.tmem_base + acc * 256;
                 for (int ki = k_begin; ki < k_end; ++ki) {
                     mbar_wait(&full_bar[stage], phase, 3);
                     tc_fence_after();
@@ -924,50 +840,38 @@ tc_wgrad_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                     for (int k = 0; k < GEMM_BLOCK_K / 16; ++k)
                         umma_bf16(tmem_d, da0 + (sa16 + a_off[k]), db0 + (sa16 + b_off[k]), idesc,
                                   (ki > k_begin || k > 0) ? 1u : 0u);
-                    umma_commit(&empty_bar[stage]);
-                    if (++stage == num_stages) { stage = 0; phase ^= 1; }
+                    umma_commit(&pl.empty_bar[stage]);
+                    if (++stage == pl.num_stages) { stage = 0; phase ^= 1; }
                 }
-                umma_commit(&tfull_bar[acc]);
+                umma_commit(&pl.tfull_bar[acc]);
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
         }
     } else {
         // =========================================================== epilogue: rows = (dy, co), three 64-column taps
         const int quad = warp & 3;
-        const int half = (warp - 2) >> 2;
         const int m = quad * 32 + lane;
         int acc = 0;
         uint32_t acc_phase = 0;
         for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-            const int nt = tile % p.n_tiles;
-            const int mt = (tile / p.n_tiles) % p.m_tiles;
-            const int mc = 2 * mt + (m >> 6);
+            const TileCoord tc(p, tile);
+            const int mc = 2 * tc.mt + (m >> 6);
             const int dy = mc / p.co_chunks, co = (mc % p.co_chunks) * 64 + (m & 63);
             const bool row_ok = mc < m_chunks && co < p.M;
             const long long c_base = static_cast<long long>(co) * p.ldc;
-            mbar_wait(&tfull_bar[acc], acc_phase, 4);
+            mbar_wait(&pl.tfull_bar[acc], acc_phase, 4);
             tc_fence_after();
-            const uint32_t taddr = tmem_base + acc * 256 + (static_cast<uint32_t>(quad * 32) << 16);
-            // 3 taps x 64 columns (with two warps per quadrant: 96 columns each, taps {0, 1 lower half} / {1 upper, 2})
+            const uint32_t taddr = pl.tmem_base + acc * 256 + (static_cast<uint32_t>(quad * 32) << 16);
 #pragma unroll 1
-            for (int i = 0; i < (EPI_HALVES == 2 ? 2 : 3); ++i) {
-                const int dx = half + i;
-                const int cb = (half == 1 && i == 0) ? 32 : 0, ce = (EPI_HALVES == 2 && half == 0 && i == 1) ? 32 : 64;
-                epilogue_row(p, taddr + dx * 64, nt * 64, (dy * 3 + dx) * p.c_col_lo, c_base, 0, row_ok, nullptr, cb, ce);
-            }
+            for (int dx = 0; dx < 3; ++dx)
+                epilogue_row(p, taddr + dx * 64, tc.nt * 64, (dy * 3 + dx) * p.c_col_lo, c_base, 0, row_ok, nullptr, 64);
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty_bar[acc]);
+            if (lane == 0) mbar_arrive(&pl.tempty_bar[acc]);
             if (++acc == 2) { acc = 0; acc_phase ^= 1; }
         }
     }
-
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 512);
-    }
+    pipeline_teardown(pl, 512);
 }
 
 }  // namespace adm
