@@ -1370,6 +1370,11 @@ int adm_gn_bwd(const void* dy, long long ldy, const void* x1, int c1, long long 
     const int C = c1 + c2;
     ADM_REQUIRE(c1 > 0 && c1 % 8 == 0 && c2 % 8 == 0 && C % groups == 0, "gn_bwd: bad channels / groups");
     ADM_REQUIRE(C <= 2048, "gn_bwd: C too large");
+    // a half-resolution dy (or add) covers an H x W input only when both are even: pixel (H - 1, .) of an odd H would
+    // read row H / 2 of dy, which belongs to the next sample (past the tensor for the last one)
+    ADM_REQUIRE((resample == 0 || (resample == 1 && h % 2 == 0 && w % 2 == 0) || resample == 2) &&
+                    (add == nullptr || add_mode == 0 || (add_mode == 1 && h % 2 == 0 && w % 2 == 0) || add_mode == 2),
+                "gn_bwd: bad resample / add_mode");
     ADM_REQUIRE((dbias1 == nullptr || dx1 != nullptr) && (dbias1b == nullptr || dbias1 != nullptr),
                 "gn_bwd: dbias1 needs dx1 (and dbias1b needs dbias1)");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
